@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR                   # also writes the last timed step's fields to DIR/fields.npy
 
 Workload (BASELINE.json configs[1]): `mcedm edm_sampler Heun sampling, n_samples=1024 of 128x128 SWE
 fields` — stochastic Heun, 50 steps (99 U-Net evaluations per field), observed-state mask blending,
@@ -35,6 +36,7 @@ sys.path.insert(0, ROOT)
 
 FLOPS_PER_EVAL = 18.797e9          # per sample per U-Net forward (BASELINE.md §2)
 EVALS_PER_FIELD = 99
+DUMP_ROWS = 128                    # 128 fp64 fields of 2 x 128 x 128 = 32 MiB per dump
 
 
 _STDOUT = sys.stdout
@@ -58,7 +60,15 @@ def parse():
     ap.add_argument("--train-batch", type=int, default=32, help="training samples per GPU per step (config 3: 256 / 8)")
     ap.add_argument("--train-steps", type=int, default=20)
     ap.add_argument("--no-train", action="store_true", help="skip the training-throughput measurement")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the fields the last timed step returned as DIR/fields.npy "
+                         f"(float64; at most {DUMP_ROWS} rows, a fixed seeded sample of them when there are more)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm only")
+    return args
 
 
 def peaks():
@@ -278,16 +288,25 @@ def run_b200(args):
         return float(ms)
 
     for _ in range(args.warmup):
-        xs = one_step(False)
-    assert xs.shape == (rows_total, 1, 128, 128, 2) and xs.dtype == torch.float64
+        one_step(False)
     checks = multi_gpu_checks(pl, cfg, dev, rank, world) if world > 1 else None
     clocks = ClockSampler(local)
     if rank == 0:
         clocks.start()
     launches0 = L.LAUNCHES[0]
-    ms = timed(lambda: one_step(False), args.steps)
+    last = []
+
+    def timed_step():
+        last.clear()                                  # the previous step's output is freed before the next one runs
+        last.append(one_step(False))
+
+    ms = timed(timed_step, args.steps)
     launches = L.LAUNCHES[0] - launches0
     clk = clocks.stop() if rank == 0 else None
+    xs = last[0]
+    assert xs.shape == (rows_total, 1, 128, 128, 2) and xs.dtype == torch.float64
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, xs)          # before the e2e steps below reuse the sampler's buffers
     one_step(True)
     ms_e2e = timed(lambda: one_step(True), args.steps)
     L.check_watchdog()
@@ -419,6 +438,21 @@ def run_b200(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, xs):
+    """Writes the fp64 fields `xs` [rows, 1, 128, 128, 2] of one sampling step as out_dir/fields.npy: every row when there
+    are at most DUMP_ROWS, else DUMP_ROWS rows drawn by a fixed seed and kept in ascending order, so that two builds run
+    with the same arguments write the same rows and can be compared element for element."""
+    import numpy as np
+    import torch
+
+    n = xs.shape[0]
+    rows = torch.arange(n)
+    if n > DUMP_ROWS:
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "fields.npy"), xs[rows.to(xs.device)].cpu().numpy())
 
 
 def multi_gpu_checks(pl, cfg, dev, rank, world):

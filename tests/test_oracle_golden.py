@@ -1,10 +1,22 @@
 """CPU: the oracle (oracle/edm_oracle.py) against fixtures produced by the unmodified reference."""
+import pytest
 import torch
 
 from common import NoiseFeed, fixture_state, golden, hparams, stress_unet
 from mcedm_b200 import data as D
 from mcedm_b200.utils import rel_l2, state_hash
 from oracle import edm_oracle as O
+
+
+@pytest.fixture(autouse=True)
+def fixture_thread_count():
+    """torch's CPU reductions split their work by thread count, so the fp32 result depends on it: the fixtures were
+    written with 8 threads, and the same count reproduces them bit for bit on any host (16 threads move a 4-step
+    trajectory by 1.3e-6)."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(n)
 
 
 def _sd_cfg(config="config_adm_edm_mcedm_res32"):
