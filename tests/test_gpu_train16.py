@@ -58,10 +58,21 @@ def from_flat(L, f, B, H, W):
     (2, 64, 64, 0, 1, True, 0, True, True, True),
     (33, 16, 16, 0, 1, False, None, False, True, True)])       # 16 pixels per CTA
 def test_gn_bwd16_matches_autograd(L, dev, fmt, add16, B, H, W, rs, act, use_ss, add0_mode, use_add1, x_flat, dy_flat):
+    check_gn_bwd16(L, dev, fmt, add16, B, H, W, rs, act, use_ss, add0_mode, use_add1, x_flat, dy_flat)
+
+
+def check_gn_bwd16(L, dev, fmt, add16, B, H, W, rs, act, use_ss, add0_mode, use_add1, x_flat, dy_flat, spread=False):
+    """mcedm_gn_bwd16 on seeded inputs, launched twice, against fp64 autograd of the same GroupNorm(+scale/shift, +SiLU,
+    +resample) expression.  After each launch the watchdog word is clear (a timed-out wait for the sample's coefficients
+    records 0xdead7000 and then carries on with stale ones) and every ticket word is back at zero.  `spread`: x and dy
+    get a per-sample scale and x a per-sample offset, so that one sample's coefficients are far from its neighbours'."""
     lib = L.lib()
     dt = torch.float16 if fmt else torch.bfloat16
     g = torch.Generator().manual_seed(H * 7 + rs + fmt)
-    x = (torch.randn(B, H, W, 64, generator=g) * 2 + 0.5).to(dev).to(dt)          # the RAW stored activation
+    x = torch.randn(B, H, W, 64, generator=g) * 2 + 0.5
+    if spread:
+        x = x * (torch.rand(B, 1, 1, 1, generator=g) * 1.5 + 0.25) + (torch.rand(B, 1, 1, 1, generator=g) * 4 - 2)
+    x = x.to(dev).to(dt)                                  # the RAW stored activation
     gamma, beta = torch.randn(64, generator=g).to(dev), torch.randn(64, generator=g).to(dev)
     ss = (torch.randn(B, 128, generator=g) * 0.3).to(dev)
     xf = x.float().contiguous()
@@ -72,7 +83,10 @@ def test_gn_bwd16_matches_autograd(L, dev, fmt, add16, B, H, W, rs, act, use_ss,
     L.check(lib.mcedm_gn_coef(L.ptr(st), H * W // 128, L.ptr(gamma), L.ptr(beta), L.ptr(ss) if use_ss else None, 128, 64,
                               1e-5, B, H, W, L.ptr(coef), L.ptr(mr), L.stream_ptr()))
     Ho, Wo = (2 * H, 2 * W) if rs == 1 else (H // 2, W // 2) if rs == 2 else (H, W)
-    dy = torch.randn(B, Ho, Wo, 64, generator=g).to(dev).to(dt)
+    dy = torch.randn(B, Ho, Wo, 64, generator=g)
+    if spread:
+        dy = dy * (torch.rand(B, 1, 1, 1, generator=g) * 3.75 + 0.25)
+    dy = dy.to(dev).to(dt)
     xl = flat_geom(L, H, W) if x_flat else (0, 0)
     dyl = flat_geom(L, Ho, Wo) if dy_flat else (0, 0)
     x_buf = to_flat(L, x) if x_flat else x.contiguous()
@@ -108,7 +122,8 @@ def test_gn_bwd16_matches_autograd(L, dev, fmt, add16, B, H, W, rs, act, use_ss,
                                    L.ptr(red), L.ptr(kcoef), L.ptr(ticket), L.ptr(dgb), L.ptr(dss) if use_ss else None,
                                    128, L.ptr(add0_buf), add0_mode or 0, a0l[0], a0l[1], L.ptr(add1_buf), add16,
                                    L.ptr(dx), L.ptr(dx16), L.ptr(dxd), L.ptr(cs), L.stream_ptr()), "gn_bwd16")
-    assert int(ticket.abs().sum()) == 0
+        L.check_watchdog()
+        assert int(ticket.abs().sum()) == 0
     xd = x.double().permute(0, 3, 1, 2).requires_grad_(True)
     gd, bd, sd = gamma.double().requires_grad_(True), beta.double().requires_grad_(True), ss.double().requires_grad_(True)
     y = F.group_norm(xd, 16, gd, bd, 1e-5)
