@@ -401,6 +401,28 @@ MCEDM_API int mcedm_edm_euler_guided(const double* x_hat, const float* D, const 
 MCEDM_API int mcedm_edm_correct_guided(const double* x_hat, const double* x_e, const float* D2, const float* gdx,
                                        const double* d_cur, const float* mask, double t_hat, double t_next,
                                        long long total, double* x_next, void* stream);
+/* Classifier-free guidance: the network runs once on 2B rows, rows [0, B) with cond and rows [B, 2B) with the all-zero
+ * condition, both on the same x_in; F (2*total elements) = [F_c | F_u].  The kernels below read
+ *   F_w = (1+w)*F_c - w*F_u   (fp32; (1+w) and w rounded to fp32 in the call, two rounded products, one rounded
+ *                              difference, no FMA)
+ * where their siblings above read F, with otherwise the same arithmetic.  w must be finite.
+ * churn_cfg: as edm_churn, writing x_in to both halves (2*total elements);
+ * euler_cfg / correct_cfg: as edm_euler / edm_correct with F_w; euler_cfg writes x_in to both halves;
+ * denoised_cfg: as edm_denoised with F_w (the PDE-guided sampler then runs edm_euler_guided / _correct_guided on D);
+ * precond_out_cfg: as edm_precond_out with F_w (B rows), also writing F_w to F_w_out. */
+MCEDM_API int mcedm_edm_churn_cfg(const double* x_cur, const double* eps, const float* mask, double coef, float c_in,
+                                  long long total, double* x_hat, float* x_in, void* stream);
+MCEDM_API int mcedm_edm_euler_cfg(const double* x_hat, const float* F, const float* mask, double t_hat, double t_next,
+                                  float c_skip, float c_out, float c_in_next, double w, long long total, double* d_cur,
+                                  double* x_next, float* x_in, float* D_out, void* stream);
+MCEDM_API int mcedm_edm_correct_cfg(const double* x_hat, const double* x_e, const float* F2, const double* d_cur,
+                                    const float* mask, double t_hat, double t_next, float c_skip, float c_out, double w,
+                                    long long total, double* x_next, float* D_out, void* stream);
+MCEDM_API int mcedm_edm_denoised_cfg(const double* x, const float* F, float c_skip, float c_out, double w,
+                                     long long total, float* D, void* stream);
+MCEDM_API int mcedm_edm_precond_out_cfg(const float* x, const float* F, const float* c_skip, const float* c_out,
+                                        int coef_stride, double w, int B, long long chw, float* D, float* F_w_out,
+                                        void* stream);
 /* RePaint-style conditioning of PlDdim.sample_edm (models/ddim.py:959-1051; mask == 1 means KNOWN):
  * x0 = double((hu*sqrt_a + noise*sqrt_1ma)*mask + noise*(1-mask)) * t0                          (:987-993) */
 MCEDM_API int mcedm_edm_vp_init(const float* hu, const float* noise, const float* mask, float sqrt_a, float sqrt_1ma,

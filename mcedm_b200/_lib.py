@@ -84,6 +84,11 @@ _PROTOTYPES = {
     "mcedm_edm_denoised": [_vp, _vp, _f, _f, C.c_longlong, _vp, _vp],
     "mcedm_edm_euler_guided": [_vp, _vp, _vp, _vp, _d, _d, _f, C.c_longlong, _vp, _vp, _vp, _vp],
     "mcedm_edm_correct_guided": [_vp, _vp, _vp, _vp, _vp, _vp, _d, _d, C.c_longlong, _vp, _vp],
+    "mcedm_edm_churn_cfg": [_vp, _vp, _vp, _d, _f, C.c_longlong, _vp, _vp, _vp],
+    "mcedm_edm_euler_cfg": [_vp, _vp, _vp, _d, _d, _f, _f, _f, _d, C.c_longlong, _vp, _vp, _vp, _vp, _vp],
+    "mcedm_edm_correct_cfg": [_vp, _vp, _vp, _vp, _vp, _d, _d, _f, _f, _d, C.c_longlong, _vp, _vp, _vp],
+    "mcedm_edm_denoised_cfg": [_vp, _vp, _f, _f, _d, C.c_longlong, _vp, _vp],
+    "mcedm_edm_precond_out_cfg": [_vp, _vp, _vp, _vp, _i, _d, _i, C.c_longlong, _vp, _vp, _vp],
     "mcedm_edm_vp_init": [_vp, _vp, _vp, _f, _f, _d, C.c_longlong, _vp, _vp],
     "mcedm_edm_repaint_blend": [_vp, _vp, _vp, _f, _f, C.c_longlong, _vp, _vp],
     "mcedm_ddim_init": [_vp, _vp, _vp, _f, _f, C.c_longlong, _vp, _vp],

@@ -14,6 +14,10 @@ Same EDM mathematics as `PlMcedm`, so the class reuses its kernel path unchanged
     the denoised field is materialised after each network evaluation, the residual gradient is one stencil launch, and
     the Euler / correction kernels subtract `(5*dx)/t_hat` (ddim.py:1571, :1590).  No host synchronisation: the
     reference's `has_nan ... .item()` test is dead code (SweFvLoss.forward already zeroes NaNs, pde_loss.py:241).
+  * classifier-free guidance (`sparams.w`, |w| >= 1e-3): each evaluation is one network batch of 2B rows, the second
+    half with the all-zero condition that the training step's condition drop (`cond_p`) feeds, and the sampler uses
+    D_w = c_skip*x + c_out*((1+w)*F_c - w*F_u) (mcedm.guidance_weight); with `guide_dx` the PDE-guidance gradient is
+    taken of D_w.
 What is NOT mirrored: `dx_cond`, self-conditioning, `node_type`, `select_by_pde`, the Darcy residual *gradient*, the
 training-time PDE loss term, and the DDIM sampler (`sample`, `sample_with_repeat` raise, as in the reference).
 """
@@ -22,7 +26,7 @@ from __future__ import annotations
 import torch
 from einops import rearrange
 
-from .mcedm import PlMcedm
+from .mcedm import PlMcedm, guidance_weight
 from .nn_misc import CorrelationLoss
 
 
@@ -170,9 +174,7 @@ class PlCondEdm(PlMcedm):
     @torch.no_grad()
     def sample_edm(self, h, u_noise, sparams, return_last=True, guide_dx=False):   # ddim.py:1532-1601
         """h: condition b h w c; u_noise: the caller's N(0,1) draw b h w c. Returns xs [b, t, h, w, c] float64."""
-        w = sparams.w
-        if not (w is None or abs(w) < 0.001):
-            raise NotImplementedError("classifier-free guidance (w != 0) is not supported")
+        w = guidance_weight(sparams.w, h)
         if not u_noise.is_cuda:
             from . import _lib as L
 
@@ -181,7 +183,7 @@ class PlCondEdm(PlMcedm):
         noise = rearrange(u_noise, "b h w c -> b c h w").contiguous()
         guide_fn = (lambda c, D: self.get_dx_pde(c, D, calc_prob=True)) if guide_dx else None
         return self._sample_core(noise, cond, torch.ones_like(noise, dtype=torch.float32), sparams, return_last,
-                                 guide_fn=guide_fn)
+                                 guide_fn=guide_fn, w=w)
 
     # ---------------------------------------------------------------- evaluation steps
     def validation_step(self, val_batch, batch_idx):                  # ddim.py:1154-1217

@@ -13,6 +13,8 @@
 #include "runtime.cuh"
 #include "../../include/mcedm_b200.h"
 
+#include <cmath>
+
 namespace mcedm {
 
 // x0 = known*(1-m) [fp32 product, as torch computes it on fp32 tensors]  +  (double(noise)*t0) * m
@@ -31,7 +33,22 @@ __global__ void edm_init_kernel(const float* __restrict__ noise, const float* __
   x[i] = __dadd_rn((double)t1, t2);
 }
 
+// Classifier-free guidance (CFG): the network runs once on a batch of 2B rows, rows [0, B) with the condition and
+// rows [B, 2B) with the all-zero condition, so F holds [F_c | F_u] with F_u starting `total` elements after F_c.
+// Every kernel below that reads F takes a CFG flag and reads the guided output
+//   F_w = (1+w)*F_c - w*F_u    (fp32; two products and one difference, each rounded: no FMA)
+// in place of F; the CFG = false instantiation is the unguided kernel, with the same arithmetic as before.
+// w_c = float(1+w) and w_u = float(w) are rounded on the host, so w = 0 gives the bits of F_c and w = -1 those of F_u.
+template <bool CFG>
+__device__ __forceinline__ float net_out(const float* __restrict__ F, long long i, long long total, float w_c,
+                                         float w_u) {
+  if constexpr (CFG) return __fsub_rn(__fmul_rn(w_c, F[i]), __fmul_rn(w_u, F[total + i]));
+  else return F[i];
+}
+
 // x_hat = x_cur + ((coef * S_noise) * eps) * m ;  x_in = float(x_hat) * c_in   (models/mcedm.py:607-608, 444, 454)
+// (CFG: x_in also to the unconditional half)
+template <bool CFG>
 __global__ void edm_churn_kernel(const double* __restrict__ x_cur, const double* __restrict__ eps,
                                  const float* __restrict__ mask, double coef, float c_in, long long total,
                                  double* __restrict__ x_hat, float* __restrict__ x_in) {
@@ -39,38 +56,47 @@ __global__ void edm_churn_kernel(const double* __restrict__ x_cur, const double*
   if (i >= total) return;
   const double xh = __dadd_rn(x_cur[i], __dmul_rn(__dmul_rn(coef, eps[i]), (double)mask[i]));
   x_hat[i] = xh;
-  x_in[i] = __fmul_rn(c_in, (float)xh);
+  const float xi = __fmul_rn(c_in, (float)xh);
+  x_in[i] = xi;
+  if constexpr (CFG) x_in[total + i] = xi;
 }
 
 // D = c_skip*float(x_hat) + c_out*F (fp32) ; d_cur = (x_hat - double(D)) / t_hat ;
 // x_next = x_hat + ((t_next - t_hat) * d_cur) * m ; x_in = float(x_next) * c_in_next   (models/mcedm.py:612-618)
+// (CFG: F_w in place of F, x_in to both halves)
+template <bool CFG>
 __global__ void edm_euler_kernel(const double* __restrict__ x_hat, const float* __restrict__ F,
                                  const float* __restrict__ mask, double t_hat, double dt, float c_skip, float c_out,
-                                 float c_in_next, long long total, double* __restrict__ d_cur,
+                                 float c_in_next, float w_c, float w_u, long long total, double* __restrict__ d_cur,
                                  double* __restrict__ x_next, float* __restrict__ x_in, float* __restrict__ D_out) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const double xh = x_hat[i];
-  const float D = __fadd_rn(__fmul_rn(c_skip, (float)xh), __fmul_rn(c_out, F[i]));
+  const float D = __fadd_rn(__fmul_rn(c_skip, (float)xh), __fmul_rn(c_out, net_out<CFG>(F, i, total, w_c, w_u)));
   const double d = __ddiv_rn(__dsub_rn(xh, (double)D), t_hat);
   const double xn = __dadd_rn(xh, __dmul_rn(__dmul_rn(dt, d), (double)mask[i]));
   d_cur[i] = d;
   x_next[i] = xn;
-  if (x_in) x_in[i] = __fmul_rn(c_in_next, (float)xn);
+  if (x_in) {
+    const float xi = __fmul_rn(c_in_next, (float)xn);
+    x_in[i] = xi;
+    if constexpr (CFG) x_in[total + i] = xi;
+  }
   if (D_out) D_out[i] = D;
 }
 
 // D2 = c_skip*float(x_e) + c_out*F2 ; d' = (x_e - double(D2)) / t_next ;
 // x_next = x_hat + ((t_next - t_hat) * (0.5*d_cur + 0.5*d')) * m     (models/mcedm.py:621-628)
+template <bool CFG>
 __global__ void edm_correct_kernel(const double* __restrict__ x_hat, const double* __restrict__ x_e,
                                    const float* __restrict__ F2, const double* __restrict__ d_cur,
                                    const float* __restrict__ mask, double t_next, double dt, float c_skip,
-                                   float c_out, long long total, double* __restrict__ x_next,
+                                   float c_out, float w_c, float w_u, long long total, double* __restrict__ x_next,
                                    float* __restrict__ D_out) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const double xe = x_e[i];
-  const float D = __fadd_rn(__fmul_rn(c_skip, (float)xe), __fmul_rn(c_out, F2[i]));
+  const float D = __fadd_rn(__fmul_rn(c_skip, (float)xe), __fmul_rn(c_out, net_out<CFG>(F2, i, total, w_c, w_u)));
   const double dp = __ddiv_rn(__dsub_rn(xe, (double)D), t_next);
   const double avg = __dadd_rn(__dmul_rn(0.5, d_cur[i]), __dmul_rn(0.5, dp));
   x_next[i] = __dadd_rn(x_hat[i], __dmul_rn(__dmul_rn(dt, avg), (double)mask[i]));
@@ -78,14 +104,19 @@ __global__ void edm_correct_kernel(const double* __restrict__ x_hat, const doubl
 }
 
 // D = c_skip[b]*x + c_out[b]*F with per-sample coefficients (training-time preconditioning,
-// models/mcedm.py:203-210); also used by get_denoised with a single sigma (stride 0).
+// models/mcedm.py:203-210); also used by get_denoised with a single sigma (stride 0).  CFG: F_w in place of F, and
+// F_w itself to F_out (get_denoised returns it)
+template <bool CFG>
 __global__ void edm_precond_out_kernel(const float* __restrict__ x, const float* __restrict__ F,
                                        const float* __restrict__ c_skip, const float* __restrict__ c_out,
-                                       int coef_stride, long long chw, long long total, float* __restrict__ D) {
+                                       int coef_stride, float w_c, float w_u, long long chw, long long total,
+                                       float* __restrict__ D, float* __restrict__ F_out) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const long long b = i / chw;
-  D[i] = __fadd_rn(__fmul_rn(c_skip[b * coef_stride], x[i]), __fmul_rn(c_out[b * coef_stride], F[i]));
+  const float f = net_out<CFG>(F, i, total, w_c, w_u);
+  D[i] = __fadd_rn(__fmul_rn(c_skip[b * coef_stride], x[i]), __fmul_rn(c_out[b * coef_stride], f));
+  if constexpr (CFG) F_out[i] = f;
 }
 
 // x_in = c_in[b] * x  (network input scaling, models/mcedm.py:208, :454)
@@ -98,11 +129,13 @@ __global__ void edm_precond_in_kernel(const float* __restrict__ x, const float* 
 
 // ---- PDE-guided variants (PlCondDdim.sample_edm with guide_dx, models/ddim.py:1566-1590) -------------------------
 // D = c_skip*float(x) + c_out*F, materialised because the guidance gradient is a stencil over D  (ddim.py:1756-1766)
+// (CFG: F_w in place of F)
+template <bool CFG>
 __global__ void edm_denoised_kernel(const double* __restrict__ x, const float* __restrict__ F, float c_skip, float c_out,
-                                    long long total, float* __restrict__ D) {
+                                    float w_c, float w_u, long long total, float* __restrict__ D) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
-  D[i] = __fadd_rn(__fmul_rn(c_skip, (float)x[i]), __fmul_rn(c_out, F[i]));
+  D[i] = __fadd_rn(__fmul_rn(c_skip, (float)x[i]), __fmul_rn(c_out, net_out<CFG>(F, i, total, w_c, w_u)));
 }
 
 // d_cur = (x_hat - double(D))/t_hat - double((5*dx)/float(t_hat)) ; x_next = x_hat + ((t_next - t_hat)*d_cur)*m
@@ -222,7 +255,7 @@ extern "C" int mcedm_edm_init(const float* noise, const float* cond, int Ccond, 
 extern "C" int mcedm_edm_churn(const double* x_cur, const double* eps, const float* mask, double coef, float c_in,
                                long long total, double* x_hat, float* x_in, void* stream) {
   using namespace mcedm;
-  edm_churn_kernel<<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(x_cur, eps, mask, coef, c_in,
+  edm_churn_kernel<false><<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(x_cur, eps, mask, coef, c_in,
                                                                                           total, x_hat, x_in);
   MCEDM_CUDA(cudaGetLastError());
   return 0;
@@ -232,8 +265,8 @@ extern "C" int mcedm_edm_euler(const double* x_hat, const float* F, const float*
                                float c_skip, float c_out, float c_in_next, long long total, double* d_cur,
                                double* x_next, float* x_in, float* D_out, void* stream) {
   using namespace mcedm;
-  edm_euler_kernel<<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      x_hat, F, mask, t_hat, t_next - t_hat, c_skip, c_out, c_in_next, total, d_cur, x_next, x_in, D_out);
+  edm_euler_kernel<false><<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      x_hat, F, mask, t_hat, t_next - t_hat, c_skip, c_out, c_in_next, 1.0f, 0.0f, total, d_cur, x_next, x_in, D_out);
   MCEDM_CUDA(cudaGetLastError());
   return 0;
 }
@@ -242,8 +275,8 @@ extern "C" int mcedm_edm_correct(const double* x_hat, const double* x_e, const f
                                  const float* mask, double t_hat, double t_next, float c_skip, float c_out,
                                  long long total, double* x_next, float* D_out, void* stream) {
   using namespace mcedm;
-  edm_correct_kernel<<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      x_hat, x_e, F2, d_cur, mask, t_next, t_next - t_hat, c_skip, c_out, total, x_next, D_out);
+  edm_correct_kernel<false><<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      x_hat, x_e, F2, d_cur, mask, t_next, t_next - t_hat, c_skip, c_out, 1.0f, 0.0f, total, x_next, D_out);
   MCEDM_CUDA(cudaGetLastError());
   return 0;
 }
@@ -252,8 +285,8 @@ extern "C" int mcedm_edm_precond_out(const float* x, const float* F, const float
                                      int coef_stride, int B, long long chw, float* D, void* stream) {
   using namespace mcedm;
   const long long total = (long long)B * chw;
-  edm_precond_out_kernel<<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      x, F, c_skip, c_out, coef_stride, chw, total, D);
+  edm_precond_out_kernel<false><<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      x, F, c_skip, c_out, coef_stride, 1.0f, 0.0f, chw, total, D, nullptr);
   MCEDM_CUDA(cudaGetLastError());
   return 0;
 }
@@ -271,8 +304,75 @@ extern "C" int mcedm_edm_precond_in(const float* x, const float* c_in, int coef_
 extern "C" int mcedm_edm_denoised(const double* x, const float* F, float c_skip, float c_out, long long total, float* D,
                                   void* stream) {
   using namespace mcedm;
-  edm_denoised_kernel<<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(x, F, c_skip, c_out, total,
-                                                                                             D);
+  edm_denoised_kernel<false><<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      x, F, c_skip, c_out, 1.0f, 0.0f, total, D);
+  MCEDM_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// ---- classifier-free guidance: F = [F_c | F_u] of a 2B-row network batch; w is rounded to fp32 here --------------
+static inline void cfg_weights(double w, float* w_c, float* w_u) {
+  *w_c = (float)(1.0 + w);
+  *w_u = (float)w;
+}
+
+extern "C" int mcedm_edm_churn_cfg(const double* x_cur, const double* eps, const float* mask, double coef, float c_in,
+                                   long long total, double* x_hat, float* x_in, void* stream) {
+  using namespace mcedm;
+  edm_churn_kernel<true><<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      x_cur, eps, mask, coef, c_in, total, x_hat, x_in);
+  MCEDM_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mcedm_edm_euler_cfg(const double* x_hat, const float* F, const float* mask, double t_hat, double t_next,
+                                   float c_skip, float c_out, float c_in_next, double w, long long total, double* d_cur,
+                                   double* x_next, float* x_in, float* D_out, void* stream) {
+  using namespace mcedm;
+  MCEDM_REQUIRE(std::isfinite(w), "edm_euler_cfg: guidance weight is not finite");
+  float w_c, w_u;
+  cfg_weights(w, &w_c, &w_u);
+  edm_euler_kernel<true><<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      x_hat, F, mask, t_hat, t_next - t_hat, c_skip, c_out, c_in_next, w_c, w_u, total, d_cur, x_next, x_in, D_out);
+  MCEDM_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mcedm_edm_correct_cfg(const double* x_hat, const double* x_e, const float* F2, const double* d_cur,
+                                     const float* mask, double t_hat, double t_next, float c_skip, float c_out, double w,
+                                     long long total, double* x_next, float* D_out, void* stream) {
+  using namespace mcedm;
+  MCEDM_REQUIRE(std::isfinite(w), "edm_correct_cfg: guidance weight is not finite");
+  float w_c, w_u;
+  cfg_weights(w, &w_c, &w_u);
+  edm_correct_kernel<true><<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      x_hat, x_e, F2, d_cur, mask, t_next, t_next - t_hat, c_skip, c_out, w_c, w_u, total, x_next, D_out);
+  MCEDM_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mcedm_edm_denoised_cfg(const double* x, const float* F, float c_skip, float c_out, double w,
+                                      long long total, float* D, void* stream) {
+  using namespace mcedm;
+  MCEDM_REQUIRE(std::isfinite(w), "edm_denoised_cfg: guidance weight is not finite");
+  float w_c, w_u;
+  cfg_weights(w, &w_c, &w_u);
+  edm_denoised_kernel<true><<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      x, F, c_skip, c_out, w_c, w_u, total, D);
+  MCEDM_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mcedm_edm_precond_out_cfg(const float* x, const float* F, const float* c_skip, const float* c_out,
+                                         int coef_stride, double w, int B, long long chw, float* D, float* F_w,
+                                         void* stream) {
+  using namespace mcedm;
+  MCEDM_REQUIRE(std::isfinite(w), "edm_precond_out_cfg: guidance weight is not finite");
+  float w_c, w_u;
+  cfg_weights(w, &w_c, &w_u);
+  const long long total = (long long)B * chw;
+  edm_precond_out_kernel<true><<<blocks_for(total), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      x, F, c_skip, c_out, coef_stride, w_c, w_u, chw, total, D, F_w);
   MCEDM_CUDA(cudaGetLastError());
   return 0;
 }

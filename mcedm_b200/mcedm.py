@@ -17,6 +17,14 @@ The arithmetic of the hot path runs in hand-written sm_100a kernels (include/mce
   * network evaluation           -> DhariwalUNet.forward (engine.py; K1 conv, K2 GroupNorm, K3 attention)
   * preconditioning              -> mcedm_edm_precond_in / _out (K4)
   * Heun / churn / mask blending -> mcedm_edm_init / _churn / _euler / _correct (K5), fp64 state
+  * classifier-free guidance     -> `sparams.w` / get_denoised's `w` with |w| >= 1e-3 and a condition (the gate of
+    :453-458): one network evaluation of 2B rows, rows [B, 2B) with the all-zero condition (what the training step's
+    condition drop feeds), combined as F_w = (1+w)*F_c - w*F_u in fp32 by mcedm_edm_*_cfg (K4/K5); the sampler
+    updates use D_w = c_skip*x + c_out*F_w, while mask blending and the known values still come from `cond`
+
+What is not mirrored: `dx_cond` (rejected in __init__), self-conditioning, the PDE guidance of this module's sampler
+(`guide_dx` raises, as :501-517 does in the reference), and guided get_denoised under autograd in train mode (raises
+NotImplementedError; the reference only calls it from no_grad sampling).
 
 Host-side differences that do not change results: the sigma schedule, gamma and the per-step fp32
 preconditioning scalars are computed on the host (the reference computes them on the device and
@@ -44,6 +52,19 @@ from .runner import LightningModule
 
 def _f32(x) -> np.float32:
     return np.float32(x)
+
+
+def guidance_weight(w, cond) -> Optional[float]:
+    """The classifier-free-guidance weight to sample with, or None when guidance is off.  Guidance is on under the gate
+    of get_denoised (:453-458): w is not None, |w| >= 1e-3 and there is a condition to drop.  A non-finite w raises
+    ValueError.  Guided, the network output is F_w = (1+w)*F_c - w*F_u (F_c with cond, F_u with the all-zero
+    condition), evaluated in fp32 by the mcedm_edm_*_cfg kernels on one network batch of 2B rows."""
+    if w is None:
+        return None
+    w = float(w)
+    if not math.isfinite(w):
+        raise ValueError(f"the guidance weight w must be finite, got {w}")
+    return w if abs(w) >= 1e-3 and cond is not None else None
 
 
 def precond_scalars(sigma: float):
@@ -211,8 +232,10 @@ class PlMcedm(LightningModule):
     def _unet_of(model):
         return model.ma_model if isinstance(model, EmaModel) else model
 
-    def _precond_apply(self, model, x, sigma, cond):
-        """(D_x, F_x) for per-sample or scalar sigma; x fp32 NCHW on the GPU."""
+    def _precond_apply(self, model, x, sigma, cond, w=None):
+        """(D_x, F_x) for per-sample or scalar sigma; x fp32 NCHW on the GPU.  With a guidance weight w (see
+        guidance_weight; cond not None) the network runs once on 2B rows, [x_in | x_in] with [cond | 0], and the pair
+        returned is (D_w, F_w)."""
         lib = L.lib()
         unet = self._unet_of(model)
         B = x.shape[0]
@@ -228,8 +251,18 @@ class PlMcedm(LightningModule):
             raise ValueError(f"sigma must have 1 or {B} entries")
         st = L.stream_ptr()
         x = x.contiguous()
-        x_in = torch.empty_like(x)
+        x_in = torch.empty_like(x) if w is None else x.new_empty((2 * B,) + tuple(x.shape[1:]))
         L.check(lib.mcedm_edm_precond_in(L.ptr(x), L.ptr(c_in), stride, B, chw, L.ptr(x_in), st), "precond_in")
+        if w is not None:
+            x_in[B:].copy_(x_in[:B])
+            cond = cond.to(torch.float32)
+            F2 = unet(x_in, c_noise.repeat(2) if stride else c_noise, torch.cat([cond, torch.zeros_like(cond)]))
+            if F2.shape[1:] != x.shape[1:]:
+                raise ValueError("classifier-free guidance needs a network output shaped like its input")
+            D_x, F_x = torch.empty_like(x), torch.empty_like(x)
+            L.check(lib.mcedm_edm_precond_out_cfg(L.ptr(x), L.ptr(F2), L.ptr(c_skip), L.ptr(c_out), stride, w, B, chw,
+                                                  L.ptr(D_x), L.ptr(F_x), st), "precond_out_cfg")
+            return D_x, F_x
         F_x = unet(x_in, c_noise, cond)
         D_x = torch.empty_like(x)
         L.check(lib.mcedm_edm_precond_out(L.ptr(x), L.ptr(F_x), L.ptr(c_skip), L.ptr(c_out), stride, B, chw,
@@ -299,10 +332,13 @@ class PlMcedm(LightningModule):
     def get_denoised(self, model, xt, t, cond=None, x_self_cond=None, dx=None, w=None):
         if x_self_cond is not None or dx is not None:
             raise NotImplementedError("self-conditioning / dx conditioning are not supported")
-        if not (w is None or abs(w) < 0.001 or cond is None):
-            raise NotImplementedError("classifier-free guidance (w != 0) is not supported")
+        w = guidance_weight(w, cond)
+        if w is not None and torch.is_grad_enabled() and self._unet_of(model).training:
+            # the reference only calls get_denoised from no_grad sampling; the guided pair has no backward here
+            raise NotImplementedError("classifier-free guidance (w != 0) runs on the inference path only (no_grad or "
+                                      "eval mode)")
         t = torch.as_tensor(t, device=xt.device)
-        return self._precond_apply(model, xt.to(torch.float32), t, cond)
+        return self._precond_apply(model, xt.to(torch.float32), t, cond, w)
 
     def round_sigma(self, sigma, return_index=False):
         return 0 if return_index else torch.as_tensor(sigma)
@@ -536,20 +572,21 @@ class PlMcedm(LightningModule):
     def sample_edm(self, hu, cond, hu_mask, sparams, return_last=True, guide_dx=False):
         if guide_dx:
             self.get_dx_pde(cond, hu)                                 # raises: see get_dx_pde
-        w = sparams.w
-        if not (w is None or abs(w) < 0.001):
-            raise NotImplementedError("classifier-free guidance (w != 0) is not supported")
+        w = guidance_weight(sparams.w, cond)
         if not hu.is_cuda:
             raise L.McedmError("sample_edm needs CUDA tensors: the sm_100a kernels have no CPU fallback")
         hu_noise = self._randn_like("init", hu)                     # :576
-        return self._sample_core(hu_noise, cond, hu_mask, sparams, return_last)
+        return self._sample_core(hu_noise, cond, hu_mask, sparams, return_last, w=w)
 
     @torch.no_grad()
-    def _sample_core(self, hu_noise, cond, hu_mask, sparams, return_last=True, guide_fn=None):
+    def _sample_core(self, hu_noise, cond, hu_mask, sparams, return_last=True, guide_fn=None, w=0.0):
         """Stochastic Heun with mask blending on the kernels, given the initial N(0,1) draw `hu_noise` [B,C,H,W]
         (shared with PlCondEdm, whose sampler takes the draw from its caller and uses an all-ones mask).
         guide_fn(cond, D fp32 [B,C,H,W]) -> fp32 [B,C,H,W]: the PDE-guidance gradient of PlCondDdim.sample_edm
-        (ddim.py:1569-1571, :1588-1590); the updates then subtract (5*dx)/t_hat from both slopes."""
+        (ddim.py:1569-1571, :1588-1590); the updates then subtract (5*dx)/t_hat from both slopes.
+        w: classifier-free guidance weight (see guidance_weight).  Guided, every evaluation is one network batch of 2B
+        rows (rows [B, 2B) see the all-zero condition) and the updates use D_w = c_skip*x + c_out*F_w; the mask blending
+        and the known values still come from `cond`, and no extra noise is drawn."""
         hu = hu_noise
         lib = L.lib()
         model = self.ema_model if self.ema_model is not None else self.model
@@ -559,16 +596,21 @@ class PlMcedm(LightningModule):
         B, C, H, W = hu.shape
         total = hu.numel()
         dev = hu.device
-        bufs = self._sampler_buffers(B, C, H, W, cond.shape[1], unet.out_channels, dev)
+        w = guidance_weight(w, cond)
+        cfg = w is not None
+        if cfg and unet.out_channels != C:
+            raise ValueError("classifier-free guidance needs a network output shaped like the sampler state")
+        bufs = self._sampler_buffers(B, C, H, W, cond.shape[1], unet.out_channels, dev, cfg)
         cond_s, mask_s = bufs["cond"], bufs["mask"]
-        cond_s.copy_(cond)                                          # static addresses -> the captured graph is reused
+        cond_s[:B].copy_(cond)                                      # static addresses -> the captured graph is reused
         mask_s.copy_(hu_mask)
-        cond, mask = cond_s, mask_s
+        cond, mask = cond_s[:B], mask_s
         hu_noise = hu_noise.to(torch.float32).contiguous()
         x_cur, x_hat, x_e, d_cur = bufs["x_cur"], bufs["x_hat"], bufs["x_e"], bufs["d_cur"]
         x_in, F_buf, nl = bufs["x_in"], bufs["F"], bufs["nl"]
         c_noise_all = []
-        D_buf = torch.empty_like(x_in) if (self._trace is not None or guide_fn is not None) else None
+        D_buf = (torch.empty(B, C, H, W, device=dev, dtype=torch.float32)
+                 if (self._trace is not None or guide_fn is not None) else None)
         st = L.stream_ptr()
         L.check(lib.mcedm_edm_init(L.ptr(hu_noise), L.ptr(cond), cond.shape[1], L.ptr(mask), t_steps[0], B, C, H, W,
                                    L.ptr(x_cur), st), "edm_init")
@@ -583,7 +625,7 @@ class PlMcedm(LightningModule):
             c_noise_all.append(precond_scalars(t_steps[i + 1])[3] if i < num_steps - 1 else 0.0)
         c_noise_dev = torch.tensor(c_noise_all, dtype=torch.float32).to(dev)
         engine = unet.engine()
-        x_in_c, cond_c = engine._check_inputs(x_in, nl, cond)[0::2]
+        x_in_c, cond_c = engine._check_inputs(x_in, nl, cond_s)[0::2]
         assert x_in_c.data_ptr() == x_in.data_ptr()
 
         # all (scale | shift) rows of the trajectory's noise levels from one embedding-MLP launch; an evaluation then
@@ -596,40 +638,46 @@ class PlMcedm(LightningModule):
             nl.copy_(c_noise_dev[k:k + 1])
             return engine.forward_static(x_in, nl, cond_c, F_buf, use_graph=self.use_cuda_graph)
 
+        # guided: the *_cfg kernels, which take w after the fp32 coefficients and read F = [F_c | F_u]
+        wa = (w,) if cfg else ()
+        churn = lib.mcedm_edm_churn_cfg if cfg else lib.mcedm_edm_churn
+        euler = lib.mcedm_edm_euler_cfg if cfg else lib.mcedm_edm_euler
+        correct = lib.mcedm_edm_correct_cfg if cfg else lib.mcedm_edm_correct
+        denoised = lib.mcedm_edm_denoised_cfg if cfg else lib.mcedm_edm_denoised
+
         for i in range(num_steps):
             t_cur, t_next = t_steps[i], t_steps[i + 1]
             t_hat = t_hats[i]
             coef = math.sqrt(t_hat ** 2 - t_cur ** 2) * sparams.S_noise
             eps = self._randn_like("step", x_cur)                   # fp64, :608
             c_skip, c_out, c_in, c_noise = precond_scalars(t_hat)
-            L.check(lib.mcedm_edm_churn(L.ptr(x_cur), L.ptr(eps), L.ptr(mask), coef, c_in, total, L.ptr(x_hat),
-                                        L.ptr(x_in), st), "edm_churn")
+            L.check(churn(L.ptr(x_cur), L.ptr(eps), L.ptr(mask), coef, c_in, total, L.ptr(x_hat), L.ptr(x_in), st),
+                    "edm_churn")
             F1 = net_eval(2 * i)
             last = i == num_steps - 1
             c_skip2, c_out2, c_in2, c_noise2 = precond_scalars(t_next) if not last else (0.0, 0.0, 0.0, 0.0)
             # Euler step; on the last step x_e already is the result (t_next = 0, no correction)
             out_e = x_cur if last else x_e
             if guide_fn is None:
-                L.check(lib.mcedm_edm_euler(L.ptr(x_hat), L.ptr(F1), L.ptr(mask), t_hat, t_next, c_skip, c_out, c_in2,
-                                            total, L.ptr(d_cur), L.ptr(out_e), None if last else L.ptr(x_in),
-                                            L.ptr(D_buf), st), "edm_euler")
+                L.check(euler(L.ptr(x_hat), L.ptr(F1), L.ptr(mask), t_hat, t_next, c_skip, c_out, c_in2, *wa, total,
+                              L.ptr(d_cur), L.ptr(out_e), None if last else L.ptr(x_in), L.ptr(D_buf), st), "edm_euler")
             else:
-                L.check(lib.mcedm_edm_denoised(L.ptr(x_hat), L.ptr(F1), c_skip, c_out, total, L.ptr(D_buf), st),
-                        "edm_denoised")
+                L.check(denoised(L.ptr(x_hat), L.ptr(F1), c_skip, c_out, *wa, total, L.ptr(D_buf), st), "edm_denoised")
                 gdx = guide_fn(cond, D_buf)
                 L.check(lib.mcedm_edm_euler_guided(L.ptr(x_hat), L.ptr(D_buf), L.ptr(gdx), L.ptr(mask), t_hat, t_next,
                                                    c_in2, total, L.ptr(d_cur), L.ptr(out_e),
                                                    None if last else L.ptr(x_in), st), "edm_euler_guided")
+                if cfg and not last:
+                    x_in[B:].copy_(x_in[:B])                        # the unconditional half sees the same input
             if self._trace is not None:
                 self._trace.append((i, 0, t_hat, D_buf.clone(), x_hat.clone()))
             if not last:
                 F2 = net_eval(2 * i + 1)
                 if guide_fn is None:
-                    L.check(lib.mcedm_edm_correct(L.ptr(x_hat), L.ptr(x_e), L.ptr(F2), L.ptr(d_cur), L.ptr(mask),
-                                                  t_hat, t_next, c_skip2, c_out2, total, L.ptr(x_cur), L.ptr(D_buf),
-                                                  st), "edm_correct")
+                    L.check(correct(L.ptr(x_hat), L.ptr(x_e), L.ptr(F2), L.ptr(d_cur), L.ptr(mask), t_hat, t_next,
+                                    c_skip2, c_out2, *wa, total, L.ptr(x_cur), L.ptr(D_buf), st), "edm_correct")
                 else:
-                    L.check(lib.mcedm_edm_denoised(L.ptr(x_e), L.ptr(F2), c_skip2, c_out2, total, L.ptr(D_buf), st),
+                    L.check(denoised(L.ptr(x_e), L.ptr(F2), c_skip2, c_out2, *wa, total, L.ptr(D_buf), st),
                             "edm_denoised")
                     gdx = guide_fn(cond, D_buf)
                     L.check(lib.mcedm_edm_correct_guided(L.ptr(x_hat), L.ptr(x_e), L.ptr(D_buf), L.ptr(gdx),
@@ -642,20 +690,23 @@ class PlMcedm(LightningModule):
         xs = torch.stack(xs, dim=0) if xs is not None else x_cur.clone().unsqueeze(0)
         return rearrange(xs, "t b c h w -> b t h w c")
 
-    def _sampler_buffers(self, B, C, H, W, Cc, Cout, dev):
-        """Persistent device buffers of one sampling batch shape (state fp64, network I/O fp32)."""
+    def _sampler_buffers(self, B, C, H, W, Cc, Cout, dev, cfg=False):
+        """Persistent device buffers of one sampling batch shape (state fp64, network I/O fp32).  cfg: the network input,
+        output and condition hold the 2B rows of a guided evaluation; condition rows [B, 2B) are zeroed here, once."""
         cache = self.__dict__.setdefault("_sampler_buf_cache", {})
-        key = (B, C, H, W, Cc, Cout, str(dev))
+        key = (B, C, H, W, Cc, Cout, str(dev), cfg)
         bufs = cache.get(key)
         if bufs is None:
             if len(cache) > 4:
                 cache.clear()
             f64 = dict(device=dev, dtype=torch.float64)
             f32 = dict(device=dev, dtype=torch.float32)
+            rows = 2 * B if cfg else B
             bufs = dict(x_cur=torch.empty(B, C, H, W, **f64), x_hat=torch.empty(B, C, H, W, **f64),
                         x_e=torch.empty(B, C, H, W, **f64), d_cur=torch.empty(B, C, H, W, **f64),
-                        x_in=torch.empty(B, C, H, W, **f32), F=torch.empty(B, Cout, H, W, **f32),
-                        cond=torch.empty(B, Cc, H, W, **f32), mask=torch.empty(B, C, H, W, **f32),
+                        x_in=torch.empty(rows, C, H, W, **f32), F=torch.empty(rows, Cout, H, W, **f32),
+                        cond=torch.empty(rows, Cc, H, W, **f32), mask=torch.empty(B, C, H, W, **f32),
                         nl=torch.empty(1, **f32))
+            bufs["cond"][B:].zero_()
             cache[key] = bufs
         return bufs
