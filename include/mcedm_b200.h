@@ -141,6 +141,19 @@ MCEDM_API int mcedm_gn_coef(const float* partial, int parts_per_img, const float
 MCEDM_API int mcedm_gn_apply16(const void* x16, int in_pitch, int in_blk, const float* coef, int act, int resample,
                                int B, int Hin, int Win, int out_pitch, int out_blk, void* out16, void* out_pooled16,
                                int op_fmt, void* stream);
+/* Dropout of the training forward (UNetBlock.forward, adm_blocks.py:167: conv1's operand).
+ * mcedm_gn_apply16_dropout: mcedm_gn_apply16 with act = 1, resample = 0, then out = 16-bit(silu(a*x + b) * scale) where
+ *   the element is kept and 0 elsewhere (one rounding, exact SiLU).  Layouts in / out as in mcedm_gn_apply16 (padding
+ *   positions of a padded-flat output are not written).
+ * mcedm_dropout_bwd16: g16 (dense: pitch = 0, or padded-flat) <- 16-bit(g16 * scale) where kept, 0 elsewhere, in place.
+ * Mask of element (b, y, x, c) at H x W: logical index n = ((b*H + y)*W + x)*64 + c in either layout; Philox4x32-10 with
+ *   counter (n >> 2, n >> 34, layer, step) and key (seed_lo, seed_hi), word n & 3; kept iff word >= threshold
+ *   (= min(2^32 - 1, floor(p * 2^32))).  rng: device uint32 {seed_lo, seed_hi, step}, read at run time. */
+MCEDM_API int mcedm_gn_apply16_dropout(const void* x16, int in_pitch, int in_blk, const float* coef, int B, int H, int W,
+                                       int out_pitch, int out_blk, void* out16, unsigned int threshold, float scale,
+                                       int layer, const unsigned int* rng, int op_fmt, void* stream);
+MCEDM_API int mcedm_dropout_bwd16(void* g16, int pitch, int blk, int B, int H, int W, unsigned int threshold, float scale,
+                                  int layer, const unsigned int* rng, int op_fmt, void* stream);
 MCEDM_API int mcedm_conv_rows_fused(const void* const* halo_src, const float* const* halo_coef, int n_halo,
                                     const void* const* ctr_src, int n_ctr, const void* w_packed, const float* bias,
                                     int B, int H, int N, int n_off, int n_total, void* out, int out_16,

@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("MCEDM_LIB") or os.path.join(_HERE, "lib", "libmcedm_b
 
 _vp = C.c_void_p
 _i = C.c_int
+_u = C.c_uint
 _f = C.c_float
 _d = C.c_double
 _ip = C.POINTER(C.c_int)
@@ -28,6 +29,8 @@ _PROTOTYPES = {
     "mcedm_conv_rows": [_vpp, _i, _vpp, _i, _vp, _vp, _i, _i, _i, _vp, _i, _vp, _i, _vp, _i, _vp],
     "mcedm_gn_coef": [_vp, _i, _vp, _vp, _vp, _i, _i, _f, _i, _i, _i, _vp, _vp, _vp],
     "mcedm_gn_apply16": [_vp, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _i, _vp],
+    "mcedm_gn_apply16_dropout": [_vp, _i, _i, _vp, _i, _i, _i, _i, _i, _vp, _u, _f, _i, _vp, _i, _vp],
+    "mcedm_dropout_bwd16": [_vp, _i, _i, _i, _i, _i, _u, _f, _i, _vp, _i, _vp],
     "mcedm_conv_rows_fused": [_vpp, _vpp, _i, _vpp, _i, _vp, _vp, _i, _i, _i, _i, _i, _vp, _i, _vp, _i, _i, _i, _vp, _i,
                               _vp],
     "mcedm_conv_head_fused": [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _i, _vp],

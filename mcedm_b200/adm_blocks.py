@@ -11,6 +11,12 @@ What differs is everything below the Python surface: the sub-modules here are pa
 only; the arithmetic runs in hand-written sm_100a kernels through `mcedm_b200.engine.UNetEngine`
 (C ABI in include/mcedm_b200.h).  There is no PyTorch/CPU fallback: calling forward on a non-CUDA tensor,
 or without the built library, raises.
+
+`dropout` (p in [0, 1)) applies where the reference applies it, to conv1's operand in every UNetBlock, and only in
+training mode: there every forward runs the fp16 training plan (train16_engine.py), whose kernels draw the masks from a
+counter-based Philox stream keyed by the engine's `dropout_seed` and `dropout_step` (DESIGN.md §3).  The masks are
+i.i.d. Bernoulli(1 - p) with scale 1 / (1 - p), as in the reference, but not torch's bits; dropout draws nothing from
+torch's generators.  In eval mode p plays no part, so a checkpoint trained with dropout samples on the inference plans.
 """
 from __future__ import annotations
 
@@ -141,6 +147,9 @@ class DhariwalUNet(torch.nn.Module):
         self.resolution = resolution
         augment_dim, label_dim = m.augment_dim, m.label_dim
         dropout, self.label_dropout = m.dropout, m.label_dropout
+        if not 0.0 <= float(dropout) < 1.0:
+            raise ValueError(f"dropout must lie in [0, 1), got {dropout}")
+        self.dropout = float(dropout)                  # one p for every UNetBlock, as in the reference
         emb_channels = ch
         init = dict(init_mode="kaiming_uniform", init_weight=np.sqrt(1 / 3), init_bias=np.sqrt(1 / 3))
         init_zero = dict(init_mode="kaiming_uniform", init_weight=0, init_bias=0)
@@ -158,8 +167,6 @@ class DhariwalUNet(torch.nn.Module):
             unsupported.append("augment_dim")
         if label_dim:
             unsupported.append("label_dim")
-        if dropout:
-            unsupported.append("dropout>0")
         if cond_channels > 0 and not self.cat_condition:
             unsupported.append("cat_cond=False (separate conditioning encoder)")
         if ch != 64 or any(int(c) != 1 for c in channel_mult):
@@ -262,4 +269,11 @@ class DhariwalUNet(torch.nn.Module):
             from .autograd import UNetFunction
 
             return UNetFunction.apply(self, x, noise_labels, cond, *self.parameters())
+        if self.training and self.dropout > 0:
+            # only the training forward has dropout kernels: a training-mode call without autograd runs it as well
+            # (its saved tape is dropped), so no training-mode evaluation silently skips the masks
+            eng = self.engine()
+            out = eng.forward_train(x, noise_labels, cond)
+            eng._tape = None
+            return out
         return self.engine().forward(x, noise_labels, cond)

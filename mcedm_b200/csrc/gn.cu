@@ -12,6 +12,7 @@
 // loads/stores, one pass.  Statistics arrive as per-128-pixel-tile partial sums (sum, sum of
 // squares per group) that the conv epilogue already produced (conv_igemm.cu); they are folded in
 // fp64 in a fixed order here, so results are run-to-run deterministic.
+#include "philox.cuh"
 #include "ptx.cuh"
 #include "runtime.cuh"
 #include "../../include/mcedm_b200.h"
@@ -232,8 +233,18 @@ __device__ __forceinline__ long long gn_in_index(const GnApplyParams& p, int b, 
   return (long long)b * p.Hin * p.Win + ip;
 }
 
-template <bool X16>
-__global__ void __launch_bounds__(256) gn_apply_kernel(const GnApplyParams p) {
+// dropout of the training forward (gn_apply_dropout_kernel; mask definition in philox.cuh)
+struct GnDropout {
+  uint32_t thr;              // keep iff mask word >= thr
+  float scale;               // 1 / (1 - p), rounded to fp32 on the host
+  int layer;                 // the block's layer id (aff_index)
+  const uint32_t* rng;       // device {seed_lo, seed_hi, step}
+};
+
+// DROP: resample 0 and SiLU only; SiLU in the exact form (not the MUFU.TANH one of the 16-bit inference instantiation),
+// operand = fp16(silu(a*x + b) * s) where kept, 0 elsewhere.  DROP = false compiles to the kernel without dropout.
+template <bool X16, bool DROP>
+__device__ __forceinline__ void gn_apply_body(const GnApplyParams& p, const GnDropout& d) {
   pdl_wait();
   pdl_trigger();
   const int b = blockIdx.y;
@@ -245,7 +256,7 @@ __global__ void __launch_bounds__(256) gn_apply_kernel(const GnApplyParams p) {
   const int pix0 = blockIdx.x * p.pix_per_cta;
   uint4* out = reinterpret_cast<uint4*>(p.out);
 
-  if (p.resample == 0) {
+  if (DROP || p.resample == 0) {
     // 4 pixels (8 x 128-bit loads) in flight per thread before any dependent work
     for (int i = ps; i < p.pix_per_cta; i += 128) {
       float4 lo[4], hi[4];
@@ -268,7 +279,14 @@ __global__ void __launch_bounds__(256) gn_apply_kernel(const GnApplyParams p) {
             const int y = ip / p.Win;
             opix = gn_out_index(p, b, y, ip - y * p.Win, p.Hin, p.Win);
           }
-          const float4 yl = gn_act4<X16>(lo[k], a_lo, b_lo, p.act, p.fast_act), yh = gn_act4<X16>(hi[k], a_hi, b_hi, p.act, p.fast_act);
+          float4 yl = gn_act4<X16 && !DROP>(lo[k], a_lo, b_lo, p.act, p.fast_act),
+                 yh = gn_act4<X16 && !DROP>(hi[k], a_hi, b_hi, p.act, p.fast_act);
+          if constexpr (DROP) {
+            // logical NHWC index of channel 8*c8 is pix*64 + 8*c8: Philox counters pix*16 + 2*c8 and the next one
+            const unsigned long long q = (unsigned long long)pix * 16ull + 2ull * (unsigned)c8;
+            yl = dropout_apply4(yl, dropout_words(q, d.layer, d.rng), d.thr, d.scale);
+            yh = dropout_apply4(yh, dropout_words(q + 1, d.layer, d.rng), d.thr, d.scale);
+          }
           const uint4 yo = pack8(yl, yh, p.fmt);
           out[opix * 8 + c8] = yo;
           if (p.out_lo) reinterpret_cast<uint4*>(p.out_lo)[opix * 8 + c8] = pack8_rem(yl, yh, yo);
@@ -355,6 +373,64 @@ __global__ void __launch_bounds__(256) gn_apply_kernel(const GnApplyParams p) {
       }
     }
   }
+}
+
+template <bool X16>
+__global__ void __launch_bounds__(256) gn_apply_kernel(const GnApplyParams p) {
+  gn_apply_body<X16, false>(p, GnDropout{});
+}
+
+struct GnApplyDropParams {
+  GnApplyParams g;
+  GnDropout d;
+};
+__global__ void __launch_bounds__(256) gn_apply_dropout_kernel(const GnApplyDropParams p) {
+  gn_apply_body<true, true>(p.g, p.d);
+}
+
+// in-place g = fp16(g * keep * s) on a 16-bit [B, H, W, 64] tensor (dense, or padded-flat with row pitch `pitch` and
+// `blk` positions per image); one thread per (pixel, 8-channel chunk), padding positions are never touched
+__global__ void __launch_bounds__(256) dropout_bwd16_kernel(void* __restrict__ g, int pitch, int blk, int B, int H, int W,
+                                                            GnDropout d, int fmt) {
+  pdl_wait();
+  pdl_trigger();
+  const long long hw = (long long)H * W;
+  const long long n_chunks = (long long)B * hw * 8;
+  uint4* gp = reinterpret_cast<uint4*>(g);
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n_chunks; i += (long long)gridDim.x * blockDim.x) {
+    const long long pix = i >> 3;
+    const int c8 = (int)(i & 7);
+    long long spix = pix;
+    if (pitch > 0) {
+      const long long b = pix / hw;
+      const int ip = (int)(pix - b * hw);
+      const int y = ip / W;
+      spix = b * blk + (long long)(y + 1) * pitch + (ip - y * W);
+    }
+    const uint4 v = gp[spix * 8 + c8];
+    float4 lo, hi;
+    if (fmt) {
+      const float2 a = unpack_f16x2(v.x), b = unpack_f16x2(v.y), c = unpack_f16x2(v.z), e = unpack_f16x2(v.w);
+      lo = make_float4(a.x, a.y, b.x, b.y);
+      hi = make_float4(c.x, c.y, e.x, e.y);
+    } else {
+      lo = make_float4(bf16_lo(v.x), bf16_hi(v.x), bf16_lo(v.y), bf16_hi(v.y));
+      hi = make_float4(bf16_lo(v.z), bf16_hi(v.z), bf16_lo(v.w), bf16_hi(v.w));
+    }
+    const unsigned long long q = (unsigned long long)pix * 16ull + 2ull * (unsigned)c8;
+    lo = dropout_apply4(lo, dropout_words(q, d.layer, d.rng), d.thr, d.scale);
+    hi = dropout_apply4(hi, dropout_words(q + 1, d.layer, d.rng), d.thr, d.scale);
+    gp[spix * 8 + c8] = pack8(lo, hi, fmt);
+  }
+}
+
+// CTAs of <= 512 work pixels; keep >= ~4 CTAs per SM when the batch allows it (0: `work` cannot be tiled)
+static int gn_apply16_pix_per_cta(int work, int B) {
+  int per = 512;
+  while (per > 32 && ((work % per) != 0 || (long long)(work / per) * B < 4LL * num_sms())) per >>= 1;
+  if (per < 32) per = 32;
+  while (per > 32 && (work % per) != 0) per >>= 1;
+  return work % per == 0 ? per : 0;
 }
 
 }  // namespace mcedm
@@ -493,13 +569,59 @@ extern "C" int mcedm_gn_apply16(const void* x16, int in_pitch, int in_blk, const
   p.coef = const_cast<float*>(coef);
   p.fmt = op_fmt ? 1 : 0;
   const int work = (resample == 2) ? (Hin * Win / 4) : (Hin * Win);
-  int per = 512;
-  while (per > 32 && ((work % per) != 0 || (long long)(work / per) * B < 4LL * num_sms())) per >>= 1;
-  if (per < 32) per = 32;
-  while (per > 32 && (work % per) != 0) per >>= 1;
-  MCEDM_REQUIRE(work % per == 0, "gn_apply16: cannot tile %d pixels", work);
+  const int per = gn_apply16_pix_per_cta(work, B);
+  MCEDM_REQUIRE(per > 0, "gn_apply16: cannot tile %d pixels", work);
   p.pix_per_cta = per;
   dim3 grid(work / per, B);
   MCEDM_CUDA(launch_pdl(gn_apply_kernel<true>, grid, dim3(256), 0, reinterpret_cast<cudaStream_t>(stream), p));
+  return 0;
+}
+
+extern "C" int mcedm_gn_apply16_dropout(const void* x16, int in_pitch, int in_blk, const float* coef, int B, int H, int W,
+                                        int out_pitch, int out_blk, void* out16, unsigned int threshold, float scale,
+                                        int layer, const unsigned int* rng, int op_fmt, void* stream) {
+  using namespace mcedm;
+  MCEDM_REQUIRE(B >= 1 && (H * W) % 128 == 0, "gn_apply16_dropout: H*W=%d must be a multiple of 128", H * W);
+  MCEDM_REQUIRE(coef != nullptr && rng != nullptr && x16 != nullptr && out16 != nullptr,
+                "gn_apply16_dropout: input, coefficients, output and the rng words are required");
+  MCEDM_REQUIRE(scale >= 1.f && layer >= 0, "gn_apply16_dropout: scale=%g layer=%d", (double)scale, layer);
+  GnApplyDropParams p;
+  memset(&p, 0, sizeof(p));
+  p.g.x = reinterpret_cast<const float*>(x16);
+  p.g.x16 = 1;
+  p.g.in_pitch = in_pitch;
+  p.g.in_blk = in_blk;
+  p.g.act = 1;
+  p.g.resample = 0;
+  p.g.Hin = H;
+  p.g.Win = W;
+  p.g.out = out16;
+  p.g.out_pitch = out_pitch;
+  p.g.out_blk = out_blk;
+  p.g.coef = const_cast<float*>(coef);
+  p.g.fmt = op_fmt ? 1 : 0;
+  p.d.thr = threshold;
+  p.d.scale = scale;
+  p.d.layer = layer;
+  p.d.rng = rng;
+  const int per = gn_apply16_pix_per_cta(H * W, B);
+  MCEDM_REQUIRE(per > 0, "gn_apply16_dropout: cannot tile %d pixels", H * W);
+  p.g.pix_per_cta = per;
+  MCEDM_CUDA(launch_pdl(gn_apply_dropout_kernel, dim3(H * W / per, B), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream), p));
+  return 0;
+}
+
+extern "C" int mcedm_dropout_bwd16(void* g16, int pitch, int blk, int B, int H, int W, unsigned int threshold, float scale,
+                                   int layer, const unsigned int* rng, int op_fmt, void* stream) {
+  using namespace mcedm;
+  MCEDM_REQUIRE(g16 != nullptr && rng != nullptr && B >= 1 && H >= 1 && W >= 1, "dropout_bwd16: bad arguments");
+  MCEDM_REQUIRE(scale >= 1.f && layer >= 0, "dropout_bwd16: scale=%g layer=%d", (double)scale, layer);
+  MCEDM_REQUIRE(pitch == 0 || (pitch >= W + 1 && blk >= (H + 1) * pitch), "dropout_bwd16: bad padded layout");
+  const GnDropout d{threshold, scale, layer, rng};
+  const long long chunks = (long long)B * H * W * 8;
+  long long grid = (chunks + 255) / 256;
+  if (grid > 8LL * num_sms()) grid = 8LL * num_sms();
+  MCEDM_CUDA(launch_pdl(dropout_bwd16_kernel, dim3((unsigned)grid), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream), g16,
+                        pitch, blk, B, H, W, d, op_fmt ? 1 : 0));
   return 0;
 }

@@ -129,6 +129,10 @@ class UNetEngine(TrainMixin, Train16Mixin, FusedMixin, PreciseMixin, PackMixin):
         # training plan: "fused16" = 16-bit activations end to end, fp16 operands, loss-scaled fp16 gradients
         # (train16_engine.py); "fp32" = the fp32-stream plan with bf16 operands (train_engine.py; any field width)
         self.train_plan = os.environ.get("MCEDM_TRAIN_PLAN", "fused16")
+        # dropout masks of the training forward (train16_engine.py): Philox key = seed (torch.initial_seed() when the
+        # engine first trains, unless set), counter word = step (one per training-mode forward)
+        self.dropout_seed: Optional[int] = None
+        self.dropout_step = 0
         # inference plan: True = GroupNorm fused into the convs + 16-bit activations (fused_engine.py);
         # False = the unfused fp32-stream plan below (what training's forward uses)
         self.fused = os.environ.get("MCEDM_FUSED", "1") != "0"

@@ -200,10 +200,22 @@ class FusedMixin:
         out = self._fact(ws, n, B, H, W, dev)
         rec = dict(blk=blk, inputs=list(inputs), coef0=coef0, mr0=mr0, h=h, coef1=coef1, mr1=mr1, out=out, final=out,
                    H=H, W=W, rs=rs) if train else None
+        src1, coefs1 = [h], [coef1]
+        drop = self._drop if train else None
+        if drop is not None:
+            # dropout (adm_blocks.py:167, training forward only): conv1's operand is materialised with the mask applied
+            # and kept for the backward (the weight gradient contracts it, the data gradient takes the same mask)
+            op1 = self._fact(ws, uq(f"op1.{H}"), B, H, W, dev, stats=False)
+            thr, scale, rng = drop
+            ip, ib = h.flat if h.flat is not None else (0, 0)
+            L.check(self.lib.mcedm_gn_apply16_dropout(L.ptr(h.t), ip, ib, L.ptr(coef1), B, H, W, ip, ib, L.ptr(op1.t), thr,
+                                                      scale, blk.aff_index, L.ptr(rng), self._fmt, st), "gn_apply16_dropout")
+            src1, coefs1 = [op1], None
+            rec["op1"] = op1
         if blk.skip_conv:
-            self._fconv([h], [coef1], blk.w1, blk.b1, B, out, None, 0, st, ctr=inputs, ws=ws)
+            self._fconv(src1, coefs1, blk.w1, blk.b1, B, out, None, 0, st, ctr=inputs, ws=ws)
         else:
-            self._fconv([h], [coef1], blk.w1, blk.b1, B, out, x_res, res_mode, st, ws=ws)
+            self._fconv(src1, coefs1, blk.w1, blk.b1, B, out, x_res, res_mode, st, ws=ws)
         if blk.attn:
             coef2 = self._fcoef(ws, f"{n}.2", out, blk.g2, blk.be2, None, 0, eps, B, st, save_mr=train)
             mr2 = None

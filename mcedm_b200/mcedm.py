@@ -67,6 +67,11 @@ def guidance_weight(w, cond) -> Optional[float]:
     return w if abs(w) >= 1e-3 and cond is not None else None
 
 
+def _dropout_active(unet) -> bool:
+    """True for a network in training mode with dropout > 0: only its training forward applies the masks."""
+    return bool(unet.training and getattr(unet, "dropout", 0.0))
+
+
 def precond_scalars(sigma: float):
     """fp32 (c_skip, c_out, c_in, c_noise) of one sigma with sigma_data = 1, evaluated with the same
     sequence of fp32 operations as :203-206 / :448-451 (IEEE mul, add, sqrt, div; log)."""
@@ -337,6 +342,9 @@ class PlMcedm(LightningModule):
             # the reference only calls get_denoised from no_grad sampling; the guided pair has no backward here
             raise NotImplementedError("classifier-free guidance (w != 0) runs on the inference path only (no_grad or "
                                       "eval mode)")
+        if w is not None and _dropout_active(self._unet_of(model)):
+            raise NotImplementedError("classifier-free guidance runs on the inference path, which has no dropout: put "
+                                      "the module in eval mode")
         t = torch.as_tensor(t, device=xt.device)
         return self._precond_apply(model, xt.to(torch.float32), t, cond, w)
 
@@ -591,6 +599,9 @@ class PlMcedm(LightningModule):
         lib = L.lib()
         model = self.ema_model if self.ema_model is not None else self.model
         unet = self._unet_of(model)
+        if _dropout_active(unet):
+            raise NotImplementedError("the sampler runs the inference plan, which has no dropout, on a network in "
+                                      "training mode with dropout > 0: put the module in eval mode")
         t_steps = self.edm_time_steps(sparams)
         num_steps = sparams.timesteps
         B, C, H, W = hu.shape

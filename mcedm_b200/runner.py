@@ -204,6 +204,10 @@ class Trainer:
                 self.optimizer.load_state_dict(ckpt["optimizer_states"][0])
             module.global_step = step = int(ckpt.get("global_step", 0))
             first_epoch = int(ckpt.get("epoch", -1)) + 1
+            net = getattr(module, "model", None)
+            if getattr(net, "dropout", 0.0):
+                # dropout masks are keyed by the step counter: a resumed run continues it instead of repeating masks
+                net.engine().dropout_step = step
         history = []
         for epoch in range(first_epoch, self.max_epochs):
             module.current_epoch = epoch

@@ -29,9 +29,11 @@ PlMcedm.training_step (models/mcedm.py:254-281).
 """
 from __future__ import annotations
 
+import math
 import os
 from typing import Dict, List, Optional
 
+import numpy as np
 import torch
 
 from . import _lib as L
@@ -46,6 +48,32 @@ class Train16Mixin:
     # weight-gradient launches on a side stream / parallel graph branch (backward16); MCEDM_WGRAD_SIDE=0 disables
     WGRAD_SIDE_STREAM = True
 
+    # ------------------------------------------------------------------ dropout state
+    def dropout_p(self) -> float:
+        return float(getattr(self.unet, "dropout", 0.0) or 0.0)
+
+    def dropout_args(self):
+        """(threshold, scale) of the dropout kernels: keep iff mask word >= threshold = min(2^32 - 1, floor(p 2^32)),
+        both computed in double; scale = 1 / (1 - p) rounded to fp32."""
+        p = self.dropout_p()
+        return min(2 ** 32 - 1, math.floor(p * 2.0 ** 32)), float(np.float32(1.0 / (1.0 - p)))
+
+    def dropout_rng(self, dev) -> torch.Tensor:
+        """The device words {seed_lo, seed_hi, step} the kernels read (one buffer per engine: graphs capture its address)."""
+        buf = getattr(self, "_rng_words", None)
+        if buf is None or buf.device != dev:
+            buf = self._rng_words = torch.zeros(3, dtype=torch.int32, device=dev)
+        return buf
+
+    def dropout_fill(self, dev):
+        """Writes {seed, step} to the device words: three stream-ordered fills, no host synchronisation."""
+        if self.dropout_seed is None:
+            self.dropout_seed = torch.initial_seed()          # reads the seed, draws nothing
+        s = int(self.dropout_seed) & (2 ** 64 - 1)
+        buf = self.dropout_rng(dev)
+        for i, v in enumerate((s & 0xFFFFFFFF, s >> 32, int(self.dropout_step) & 0xFFFFFFFF)):
+            buf[i].fill_(v - 2 ** 32 if v >= 2 ** 31 else v)
+
     # ------------------------------------------------------------------ forward
     def forward_train16(self, x: torch.Tensor, nl: torch.Tensor, cond: Optional[torch.Tensor]) -> torch.Tensor:
         u = self.unet
@@ -55,6 +83,14 @@ class Train16Mixin:
         dev = x.device
         st = L.stream_ptr()
         ws = self._fws(B, H, W, dev, tag="train16")
+        self._drop = None
+        if self.dropout_p() > 0:
+            # eager: this forward's {seed, step} go to the device words now; under graph capture the kernels only
+            # capture the words' address and TrainStepGraph.load writes them before every replay
+            if not torch.cuda.is_current_stream_capturing():
+                self.dropout_fill(dev)
+                self.dropout_step += 1
+            self._drop = self.dropout_args() + (self.dropout_rng(dev),)
         self._ss_external = False
         self._ss_rows = B
         ss = ws["ss"] = self._fbuf(ws, "ss_buf", (self.n_aff * B * 128,), torch.float32, dev)
@@ -69,7 +105,7 @@ class Train16Mixin:
         out = torch.empty(B, u.out_channels, H, W, device=dev, dtype=torch.float32)
         tape: dict = {}
         self._launch_rest_fused(x, cond, out, ws, B, H, dev, 128, st, tape=tape)
-        tape.update(plan="fused16", ws=ws, B=B, H=H, W=W)
+        tape.update(plan="fused16", ws=ws, B=B, H=H, W=W, drop=self._drop)
         self._tape = tape
         return out
 
@@ -271,8 +307,12 @@ class Train16Mixin:
             # out = conv1(a1) + b1 + skip(x)
             self._bias_grad(gs, B, G(m.conv1.bias), st)
             h: Act = rec["h"]
-            wgrad_side(ws, gs["bf"], is_flat, 64, 0, h.t, is_flat, B, Hb, Wb, 9, G(m.conv1.weight), 64, 0, st,
-                       a_coef=rec["coef1"])
+            op1: Optional[Act] = rec.get("op1")
+            if op1 is None:
+                wgrad_side(ws, gs["bf"], is_flat, 64, 0, h.t, is_flat, B, Hb, Wb, 9, G(m.conv1.weight), 64, 0, st,
+                           a_coef=rec["coef1"])
+            else:      # dropout: conv1 contracted the materialised, masked operand the forward kept
+                wgrad_side(ws, gs["bf"], is_flat, 64, 0, op1.t, is_flat, B, Hb, Wb, 9, G(m.conv1.weight), 64, 0, st)
             if blk.skip_conv:
                 self._bias_grad(gs, B, G(m.skip.bias), st)
                 for i, xi in enumerate(rec["inputs"]):
@@ -280,6 +320,10 @@ class Train16Mixin:
                                64 * blk.n_src, 64 * i, st)
             d_a1 = self._buf16(ws, ("d16", Hb, Wb), B, Hb, Wb, dev)
             self._dgrad16(ws, gs["bf"], blk.wd1, B, Hb, Wb, d_a1, st)
+            if op1 is not None:
+                thr, scale, rng = T["drop"]
+                L.check(lib.mcedm_dropout_bwd16(L.ptr(d_a1), lay[0], lay[1], B, Hb, Wb, thr, scale, blk.aff_index,
+                                                L.ptr(rng), fmt, st), "dropout_bwd16")
             d_hb = self._buf16(ws, ("d_h16", Hb, Wb), B, Hb, Wb, dev)
             hset = dict(f32=None, bf=d_hb, dense=None, cs=None, n_cta=lib.mcedm_gn_bwd16_ctas_per_img(Hb, Wb, B))
             self._gn_bwd16(ws, d_a1, lay, h, rec["mr1"], rec["coef1"], blk.g1, blk.be1, ss_all[blk.aff_index], 1, 0, B,

@@ -176,6 +176,9 @@ class TrainMixin:
         B, _, H, W = x.shape
         if nl.numel() == 1:
             nl = nl.expand(B).contiguous()
+        if self.dropout_p() > 0 and (self.train_plan != "fused16" or W != 128):
+            raise NotImplementedError("dropout > 0 has kernels in the fp16 training plan only (MCEDM_TRAIN_PLAN=fused16, "
+                                      "128-pixel-wide fields)")
         if self.train_plan == "fused16" and W != 128:
             self.train_plan = "fp32"          # the 16-bit plan is laid out for 128-pixel-wide fields
         if self.train_plan == "fused16":

@@ -65,9 +65,12 @@ class TrainStepGraph:
         self.pl.model.engine().backward(self.dF)
 
     def capture(self):
+        eng = self.pl.model.engine()
+        step = eng.dropout_step
         with torch.no_grad():
             self._fwd()                      # eager warm-up: allocates workspaces, sets kernel attributes
             self._bwd()
+            eng.dropout_step = step          # the warm-up is not a training step: it draws no dropout masks of its own
             torch.cuda.current_stream().synchronize()
             n0 = L.LAUNCHES[0]
             self.g_fwd = torch.cuda.CUDAGraph()
@@ -93,6 +96,9 @@ class TrainStepGraph:
                 self.cond.copy_(cond)
         self.sigma.copy_(sigma.reshape(-1))
         self.weight.copy_(weight.reshape(-1))
+        eng = self.pl.model.engine()
+        if eng.dropout_p() > 0:
+            eng.dropout_fill(self.dev)       # {seed, step} of the next replay (GraphedLossFunction advances the step)
 
 
 class GraphedLossFunction(torch.autograd.Function):
@@ -100,6 +106,9 @@ class GraphedLossFunction(torch.autograd.Function):
     def forward(ctx, tg, trigger):
         tg.g_fwd.replay()
         L.LAUNCHES[0] += tg.launches[0]
+        eng = tg.pl.model.engine()
+        if eng.dropout_p() > 0:
+            eng.dropout_step += 1
         ctx.tg = tg
         return tg.loss.clone()
 
