@@ -19,6 +19,9 @@
  *     16-bit output): 0 = bf16, 1 = fp16 (same layouts, same tensor throughput; names keep the `_bf16` suffix).
  *     Training uses bf16 throughout (gradients need its range); inference may use fp16, whose 11 significand bits
  *     cut the operand-rounding error of the network output ~8x (activations are normalised, weights are O(1)).
+ *     MCEDM_FMT_F16_INF (3) = fp16 whose stores round a value beyond +-65504 to +-inf instead of clamping it: the
+ *     16-bit gradient stores of dynamic loss scaling, so that an overflow reaches the fp32 flat gradient as inf / NaN
+ *     and the optimizer step skips.  Accepted only by the gradient-writing entries whose comment names it.
  *   - there is NO CPU implementation behind any of these: without an sm_100 device they fail.
  */
 #ifndef MCEDM_B200_H
@@ -29,6 +32,7 @@ extern "C" {
 #endif
 
 #define MCEDM_ABI_VERSION 1
+#define MCEDM_FMT_F16_INF 3
 #if defined(__GNUC__)
 #define MCEDM_API __attribute__((visibility("default")))
 #else
@@ -61,6 +65,8 @@ MCEDM_API int mcedm_check_watchdog(void* stream);
  *   stats_partial: NULL, or fp32 [B*H*W/128][N/4][2] receiving per-128-pixel-tile (sum, sum of squares)
  *                 of the stored values per 4-channel GroupNorm group (feeds mcedm_gn_apply).
  * Requires W | 128, 128 | H*W.
+ * op_fmt MCEDM_FMT_F16_INF (N = 64, out_bf16 = 1): fp16 output without saturation (the 1x1 data gradients of dynamic
+ * loss scaling).
  */
 MCEDM_API int mcedm_conv_igemm(const void* const* src, int n_src, const int* seg_src, const int* seg_dy, const int* seg_dx,
                      int n_seg, const void* w_packed, const float* bias, int B, int H, int W, int N, void* out,
@@ -119,6 +125,9 @@ MCEDM_API int mcedm_conv_flat(const void* src_flat, const void* w_packed, const 
  *   halo_coef == NULL (or all entries NULL): the halo sources are already-normalised operands (no transform);
  *   likewise coef == NULL in mcedm_conv_flat_fused (the conv0 of an up/down block reads mcedm_gn_apply16 output)
  *   stats_partial              NULL or fp32 [B*H][4][n_total/4][2] (this launch fills groups n_off/4 ...)
+ *   op_fmt                     1, or MCEDM_FMT_F16_INF for the data gradient of a 3x3 conv under dynamic loss
+ *                              scaling (N = 64, no coefficients, no residual, 16-bit out without saturation); the
+ *                              same holds for mcedm_conv_flat_fused
  * mcedm_conv_flat_fused (W <= 64): src/out/res in the padded-flat layout of mcedm_flat_geometry
  *   out_flat   16-bit [B*blk][64] (out_f32 = 0) or fp32 [B*blk][64] (out_f32 = 1, K-split partial); only data
  *              positions are written (padding must have been zeroed once by the owner)
@@ -148,7 +157,8 @@ MCEDM_API int mcedm_gn_apply16(const void* x16, int in_pitch, int in_blk, const 
  * mcedm_dropout_bwd16: g16 (dense: pitch = 0, or padded-flat) <- 16-bit(g16 * scale) where kept, 0 elsewhere, in place.
  * Mask of element (b, y, x, c) at H x W: logical index n = ((b*H + y)*W + x)*64 + c in either layout; Philox4x32-10 with
  *   counter (n >> 2, n >> 34, layer, step) and key (seed_lo, seed_hi), word n & 3; kept iff word >= threshold
- *   (= min(2^32 - 1, floor(p * 2^32))).  rng: device uint32 {seed_lo, seed_hi, step}, read at run time. */
+ *   (= min(2^32 - 1, floor(p * 2^32))).  rng: device uint32 {seed_lo, seed_hi, step}, read at run time.
+ *   mcedm_dropout_bwd16 also takes op_fmt MCEDM_FMT_F16_INF (fp16 without saturation, dynamic loss scaling). */
 MCEDM_API int mcedm_gn_apply16_dropout(const void* x16, int in_pitch, int in_blk, const float* coef, int B, int H, int W,
                                        int out_pitch, int out_blk, void* out16, unsigned int threshold, float scale,
                                        int layer, const unsigned int* rng, int op_fmt, void* stream);
@@ -268,7 +278,8 @@ MCEDM_API int mcedm_gn_bwd(const float* dy, const float* x, const float* meanrst
  * grid is resident at once (ctas_per_img * B <= 2 x SM count) both passes run as ONE kernel: the sample's other CTAs
  * wait for that fold in the kernel and re-read their slice from L2 (words [B..3B) are the flag and the departure count).
  * Win must be a power of two.  red_partial / dgb_partial / colsum_partial as in mcedm_gn_bwd, sized with
- * mcedm_gn_bwd16_ctas_per_img.
+ * mcedm_gn_bwd16_ctas_per_img.  op_fmt MCEDM_FMT_F16_INF: fp16 whose dx16 / dx16_dense stores do not saturate (dynamic
+ * loss scaling).
  */
 MCEDM_API int mcedm_gn_bwd16_ctas_per_img(int Hin, int Win, int B);
 MCEDM_API int mcedm_gn_bwd16(const void* dy16, int dy_pitch, int dy_blk, const void* x16, int x_pitch, int x_blk,
@@ -355,7 +366,8 @@ MCEDM_API int mcedm_attention(const void* qkv_bf16, int B, int L, void* out_bf16
  */
 MCEDM_API int mcedm_attention_bwd(const void* qkv_bf16, const void* out_bf16, const void* d_out_bf16, const float* lse,
                                   int B, int L, float* dvec, void* dq_bf16, void* dk_bf16, void* dv_bf16, void* stream);
-/* The same with every 16-bit tensor (inputs, P / dS operand tiles, outputs) in op_fmt (0 bf16, 1 fp16). */
+/* The same with every 16-bit tensor (inputs, P / dS operand tiles, outputs) in op_fmt (0 bf16, 1 fp16;
+ * MCEDM_FMT_F16_INF: fp16 whose dS tiles and outputs do not saturate, dynamic loss scaling). */
 MCEDM_API int mcedm_attention_bwd16(const void* qkv16, const void* out16, const void* d_out16, const float* lse, int B,
                                     int L, float* dvec, void* dq16, void* dk16, void* dv16, int op_fmt, void* stream);
 
@@ -508,6 +520,12 @@ MCEDM_API int mcedm_nchw_to_nhwc_pad16(const float* a, int Ca, const float* b, i
                                        int c_dst0, float scale, int op_fmt, void* stream);
 MCEDM_API int mcedm_colsum16(const void* x16, long long pixels, int C, int c_off, float* partial, int n_ctas, int op_fmt,
                              void* stream);
+/* The pad variant under dynamic loss scaling: the scale is read from device memory (*scale, so a graph replay uses the
+ * current one) and op_fmt must be MCEDM_FMT_F16_INF (scale * dL/dF beyond fp16's range becomes inf). */
+MCEDM_API int mcedm_nchw_to_nhwc_pad16_scaled(const float* a, int Ca, const float* b, int Cb, int B, int H, int W,
+                                              void* dst16, int c_dst0, const float* scale, int op_fmt, void* stream);
+/* g <- g * (1 / *scale): the loss scale comes off the fp32 flat gradient (exact for power-of-two scales). */
+MCEDM_API int mcedm_grad_unscale(float* g, long long n, const float* scale, void* stream);
 /* backward of mcedm_emb_mlp: dss fp32 [n_aff][B][128] = gradient of every block's (scale | shift);
  * vec_scratch fp32 [B][320]; outputs in the reference parameter shapes (affine [n_aff][128][64] / [n_aff][128],
  * map_layer1, map_layer0 [64][64] / [64]) */
@@ -525,6 +543,19 @@ MCEDM_API int mcedm_adam_step(float* p, const float* g, float* m, float* v, long
                               int n_partial, float max_norm, float grad_scale, float* norm_out, void* stream);
 /* ema = ema*beta + (1-beta)*p   (ddim_blocks.py:48-56) */
 MCEDM_API int mcedm_ema_update(float* ema, const float* p, long long n, float beta, void* stream);
+/* mcedm_adam_step under dynamic loss scaling.  norm_partial (mcedm_sumsq_partial of g) is required; clipping runs iff
+ * max_norm > 0.  A non-finite sum of squares sets *found_inf = 1 (else 0) and the step writes nothing to p, m, v.  The
+ * bias corrections use step = *step_count + 1 (the applied-step count, in device memory; mcedm_loss_scale_update
+ * advances it).  No host synchronisation. */
+MCEDM_API int mcedm_adam_step_dyn(float* p, const float* g, float* m, float* v, long long n, float lr, float beta1,
+                                  float beta2, float eps, float weight_decay, const int* step_count,
+                                  const double* norm_partial, int n_partial, float max_norm, float grad_scale,
+                                  float* norm_out, float* found_inf, void* stream);
+/* torch._amp_update_scale_ on device words: found_inf != 0 -> scale *= backoff, tracker = 0; else tracker + 1 reaching
+ * growth_interval -> scale *= growth (kept if finite), tracker = 0, otherwise tracker += 1.  When the step applied
+ * (found_inf == 0) *step_count += 1 (step_count may be NULL).  One thread. */
+MCEDM_API int mcedm_loss_scale_update(float* scale, int* growth_tracker, const float* found_inf, int* step_count,
+                                      float growth_factor, float backoff_factor, int growth_interval, void* stream);
 /* All packed operand copies of the parameters in one launch (replaces the per-tensor permute / flip / cast passes of
  * the weight re-pack after every optimizer step; adm_blocks.py:58 casts the weights per call in the reference).
  * dst16[i] = round16(base[idx_a[i]]) for i < n16 (fmt 0 bf16, 1 fp16; idx -1 = zero padding);

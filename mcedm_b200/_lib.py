@@ -64,6 +64,10 @@ _PROTOTYPES = {
     "mcedm_sumsq_partial": [_vp, C.c_longlong, _vp, _i, _vp],
     "mcedm_adam_step": [_vp, _vp, _vp, _vp, C.c_longlong, _f, _f, _f, _f, _f, _i, _vp, _i, _f, _f, _vp, _vp],
     "mcedm_ema_update": [_vp, _vp, C.c_longlong, _f, _vp],
+    "mcedm_nchw_to_nhwc_pad16_scaled": [_vp, _i, _vp, _i, _i, _i, _i, _vp, _i, _vp, _i, _vp],
+    "mcedm_grad_unscale": [_vp, C.c_longlong, _vp, _vp],
+    "mcedm_adam_step_dyn": [_vp, _vp, _vp, _vp, C.c_longlong, _f, _f, _f, _f, _f, _vp, _vp, _i, _f, _f, _vp, _vp, _vp],
+    "mcedm_loss_scale_update": [_vp, _vp, _vp, _vp, _f, _f, _i, _vp],
     "mcedm_pack_gather": [_vp, _vp, _vp, C.c_longlong, C.c_longlong, _i, _vp, _vp, _vp],
     "mcedm_wgrad_ctas": [_i, _i, _i],
     "mcedm_conv_wgrad": [_vp, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp],
@@ -126,6 +130,8 @@ _lib = None
 # number of kernel launches issued through the C ABI by this process (every successful call below launches
 # exactly one kernel; graph replays are added by the engine); bench.py reports it as gpu_launches
 LAUNCHES = [0]
+# op_fmt of fp16 stores without saturation (include/mcedm_b200.h MCEDM_FMT_F16_INF): dynamic loss scaling's gradients
+FMT_F16_INF = 3
 
 
 class McedmError(RuntimeError):

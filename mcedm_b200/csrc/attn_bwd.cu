@@ -73,7 +73,8 @@ struct AttnBwdParams {
   int fmt;              // 16-bit format of every operand / output: 0 bf16, 1 fp16
 };
 
-template <int MODE>
+// INF: the dS tiles and the dQ / dK / dV stores in fp16 without saturation (op_fmt MCEDM_FMT_F16_INF)
+template <int MODE, bool INF = false>
 __global__ void __launch_bounds__(192, 1)
 attn_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_constant__ CUtensorMap tm_do,
                 const AttnBwdParams p) {
@@ -249,7 +250,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_constan
             const float ds0 = p0 * (__uint_as_float(g[i0]) - d0) * 0.125f;
             const float ds1 = p1 * (__uint_as_float(g[i0 + 1]) - d1) * 0.125f;
             pp[e] = pack_op2(p0, p1, p.fmt);
-            dp[e] = pack_op2(ds0, ds1, p.fmt);
+            dp[e] = pack_op2_g<INF>(ds0, ds1, p.fmt);
           }
           const int unit = ((c & 1) * 4 + u) ^ (row & 7);
           if (MODE == 1) *reinterpret_cast<uint4*>(prow + (c >> 1) * kBTile + unit * 16) = po;
@@ -277,10 +278,10 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_constan
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
           uint4 o;
-          o.x = pack_op2(__uint_as_float(v[u * 8 + 0]), __uint_as_float(v[u * 8 + 1]), p.fmt);
-          o.y = pack_op2(__uint_as_float(v[u * 8 + 2]), __uint_as_float(v[u * 8 + 3]), p.fmt);
-          o.z = pack_op2(__uint_as_float(v[u * 8 + 4]), __uint_as_float(v[u * 8 + 5]), p.fmt);
-          o.w = pack_op2(__uint_as_float(v[u * 8 + 6]), __uint_as_float(v[u * 8 + 7]), p.fmt);
+          o.x = pack_op2_g<INF>(__uint_as_float(v[u * 8 + 0]), __uint_as_float(v[u * 8 + 1]), p.fmt);
+          o.y = pack_op2_g<INF>(__uint_as_float(v[u * 8 + 2]), __uint_as_float(v[u * 8 + 3]), p.fmt);
+          o.z = pack_op2_g<INF>(__uint_as_float(v[u * 8 + 4]), __uint_as_float(v[u * 8 + 5]), p.fmt);
+          o.w = pack_op2_g<INF>(__uint_as_float(v[u * 8 + 6]), __uint_as_float(v[u * 8 + 7]), p.fmt);
           *reinterpret_cast<uint4*>(dst + c * 32 + u * 8) = o;
         }
       }
@@ -295,6 +296,37 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_constan
   }
 }
 
+}  // namespace mcedm
+
+namespace mcedm {
+template <bool INF>
+static int attn_bwd_launch(const CUtensorMap& tm_qkv, const CUtensorMap& tm_do, int L, const float* lse, float* dvec,
+                           void* dq_bf16, void* dk_bf16, void* dv_bf16, int op_fmt, int B, cudaStream_t st) {
+  AttnBwdParams p;
+  p.L = L;
+  p.lse = lse;
+  p.dvec = dvec;
+  p.fmt = op_fmt ? 1 : 0;
+  p.err = watchdog_ptr();
+  MCEDM_REQUIRE(p.err != nullptr, "attention_bwd: no watchdog word");
+  const int smem = 1024 + 2 * kBTile + kBStages * 2 * kBTile + 4 * kBTile + 2 * 256 * 4 + 256;
+  static bool attr_set = false;
+  if (!attr_set) {
+    MCEDM_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<0, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    MCEDM_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<1, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    attr_set = true;
+  }
+  const unsigned grid = (unsigned)(B * (L / 128));
+  p.out1 = nullptr;
+  p.out2 = reinterpret_cast<__nv_bfloat16*>(dq_bf16);
+  attn_bwd_kernel<0, INF><<<grid, 192, smem, st>>>(tm_qkv, tm_do, p);
+  MCEDM_CUDA(cudaGetLastError());
+  p.out1 = reinterpret_cast<__nv_bfloat16*>(dv_bf16);
+  p.out2 = reinterpret_cast<__nv_bfloat16*>(dk_bf16);
+  attn_bwd_kernel<1, INF><<<grid, 192, smem, st>>>(tm_qkv, tm_do, p);
+  MCEDM_CUDA(cudaGetLastError());
+  return 0;
+}
 }  // namespace mcedm
 
 extern "C" int mcedm_attention_bwd(const void* qkv_bf16, const void* out_bf16, const void* d_out_bf16,
@@ -318,28 +350,6 @@ extern "C" int mcedm_attention_bwd16(const void* qkv_bf16, const void* out_bf16,
   attn_bwd_prep_kernel<<<(unsigned)((rows + 127) / 128), 128, 0, st>>>(
       reinterpret_cast<const uint4*>(out_bf16), reinterpret_cast<const uint4*>(d_out_bf16), rows, dvec, op_fmt ? 1 : 0);
   MCEDM_CUDA(cudaGetLastError());
-  AttnBwdParams p;
-  p.L = L;
-  p.lse = lse;
-  p.dvec = dvec;
-  p.fmt = op_fmt ? 1 : 0;
-  p.err = watchdog_ptr();
-  MCEDM_REQUIRE(p.err != nullptr, "attention_bwd: no watchdog word");
-  const int smem = 1024 + 2 * kBTile + kBStages * 2 * kBTile + 4 * kBTile + 2 * 256 * 4 + 256;
-  static bool attr_set = false;
-  if (!attr_set) {
-    MCEDM_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    MCEDM_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    attr_set = true;
-  }
-  const unsigned grid = (unsigned)(B * (L / 128));
-  p.out1 = nullptr;
-  p.out2 = reinterpret_cast<__nv_bfloat16*>(dq_bf16);
-  attn_bwd_kernel<0><<<grid, 192, smem, st>>>(tm_qkv, tm_do, p);
-  MCEDM_CUDA(cudaGetLastError());
-  p.out1 = reinterpret_cast<__nv_bfloat16*>(dv_bf16);
-  p.out2 = reinterpret_cast<__nv_bfloat16*>(dk_bf16);
-  attn_bwd_kernel<1><<<grid, 192, smem, st>>>(tm_qkv, tm_do, p);
-  MCEDM_CUDA(cudaGetLastError());
-  return 0;
+  return op_fmt == MCEDM_FMT_F16_INF ? attn_bwd_launch<true>(tm_qkv, tm_do, L, lse, dvec, dq_bf16, dk_bf16, dv_bf16, 1, B, st)
+                                   : attn_bwd_launch<false>(tm_qkv, tm_do, L, lse, dvec, dq_bf16, dk_bf16, dv_bf16, op_fmt, B, st);
 }

@@ -179,7 +179,8 @@ __device__ __forceinline__ uint32_t flat_xf_pair(uint32_t v, float a0, float b0,
 
 // FM (fused only): epilogue variant folded at compile time: 0 fast path without residual, 1 fast path with a
 // same-resolution 16-bit residual, 2 general path (resampled / fp32 residual, fp32 output); -1 = legacy unfused epilogue
-template <int N, bool FUSED, int FM = -1>
+// INF: fp16 stores without saturation (the data-gradient convs of dynamic loss scaling, op_fmt MCEDM_FMT_F16_INF)
+template <int N, bool FUSED, int FM = -1, bool INF = false>
 __global__ void __launch_bounds__(FlatCfg<N, FUSED>::THREADS, 1)
 conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_a,
                  const FlatParams p) {
@@ -415,10 +416,10 @@ conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
           uint4 o;
-          o.x = pack_f16x2(__uint_as_float(v[8 * c + 0]), __uint_as_float(v[8 * c + 1]));
-          o.y = pack_f16x2(__uint_as_float(v[8 * c + 2]), __uint_as_float(v[8 * c + 3]));
-          o.z = pack_f16x2(__uint_as_float(v[8 * c + 4]), __uint_as_float(v[8 * c + 5]));
-          o.w = pack_f16x2(__uint_as_float(v[8 * c + 6]), __uint_as_float(v[8 * c + 7]));
+          o.x = pack_f16x2_g<INF>(__uint_as_float(v[8 * c + 0]), __uint_as_float(v[8 * c + 1]));
+          o.y = pack_f16x2_g<INF>(__uint_as_float(v[8 * c + 2]), __uint_as_float(v[8 * c + 3]));
+          o.z = pack_f16x2_g<INF>(__uint_as_float(v[8 * c + 4]), __uint_as_float(v[8 * c + 5]));
+          o.w = pack_f16x2_g<INF>(__uint_as_float(v[8 * c + 6]), __uint_as_float(v[8 * c + 7]));
           sts128(st16 + lane * 64 + ((c ^ ((lane >> 1) & 3)) << 4), o);
         }
         __syncwarp();
@@ -448,10 +449,10 @@ conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
           sb1 += (a[4] + a[5]) + (a[6] + a[7]);
           sb2 += (a[4] * a[4] + a[5] * a[5]) + (a[6] * a[6] + a[7] * a[7]);
           uint4 o;
-          o.x = pack_f16x2(a[0], a[1]);
-          o.y = pack_f16x2(a[2], a[3]);
-          o.z = pack_f16x2(a[4], a[5]);
-          o.w = pack_f16x2(a[6], a[7]);
+          o.x = pack_f16x2_g<INF>(a[0], a[1]);
+          o.y = pack_f16x2_g<INF>(a[2], a[3]);
+          o.z = pack_f16x2_g<INF>(a[4], a[5]);
+          o.w = pack_f16x2_g<INF>(a[6], a[7]);
           *reinterpret_cast<uint4*>(o16 + base + it * 8 * N) = o;
         }
         if (p.stats) {
@@ -715,7 +716,7 @@ extern "C" int mcedm_flat_geometry(int H, int W, int* pitch, int* block_position
 }
 
 namespace mcedm {
-template <bool FUSED, int FM = -1>
+template <bool FUSED, int FM = -1, bool INF = false>
 static int launch_flat(FlatParams p, const void* src_flat, const void* w_packed, int B, int blk, cudaStream_t st) {
   using Cfg = FlatCfg<64, FUSED>;
   const int N = 64;
@@ -736,11 +737,11 @@ static int launch_flat(FlatParams p, const void* src_flat, const void* w_packed,
   if (rc) return rc;
   static bool attr_set = false;
   if (!attr_set) {
-    MCEDM_CUDA(cudaFuncSetAttribute(conv_flat_kernel<64, FUSED, FM>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
+    MCEDM_CUDA(cudaFuncSetAttribute(conv_flat_kernel<64, FUSED, FM, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
     attr_set = true;
   }
   long long grid = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
-  MCEDM_CUDA(launch_pdl(conv_flat_kernel<64, FUSED, FM>, dim3((unsigned)grid), dim3(Cfg::THREADS), (size_t)smem, st, tm_w, tm_a, p));
+  MCEDM_CUDA(launch_pdl(conv_flat_kernel<64, FUSED, FM, INF>, dim3((unsigned)grid), dim3(Cfg::THREADS), (size_t)smem, st, tm_w, tm_a, p));
   return 0;
 }
 }  // namespace mcedm
@@ -779,7 +780,8 @@ extern "C" int mcedm_conv_flat_fused(const void* src_flat16, const float* coef, 
   int rc = mcedm_flat_geometry(H, W, &P, &blk);
   if (rc) return rc;
   MCEDM_REQUIRE(N == 64, "conv_flat_fused: N=%d unsupported (64)", N);
-  MCEDM_REQUIRE(op_fmt == 1, "conv_flat_fused: the fused inference kernels are fp16-only (op_fmt = 1)");
+  MCEDM_REQUIRE(op_fmt == 1 || op_fmt == MCEDM_FMT_F16_INF,
+                "conv_flat_fused: the fused inference kernels are fp16-only (op_fmt = 1)");
   MCEDM_REQUIRE(res_mode >= 0 && res_mode <= 3 && (res_mode == 0 || res != nullptr), "conv_flat_fused: bad residual mode");
   MCEDM_REQUIRE(!res_f32 || res_mode == 1, "conv_flat_fused: an fp32 residual must be same-resolution padded-flat");
   FlatParams p;
@@ -802,6 +804,12 @@ extern "C" int mcedm_conv_flat_fused(const void* src_flat16, const float* coef, 
   p.coef = coef;
   if (const char* e = getenv("MCEDM_DBG")) p.dbg = atoi(e);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (op_fmt == MCEDM_FMT_F16_INF) {
+    // the data gradient of a 3x3 conv (no transform, no residual) is the one gradient this kernel writes
+    MCEDM_REQUIRE(!p.out_f32 && p.res_mode == 0 && coef == nullptr,
+                  "conv_flat_fused: op_fmt MCEDM_FMT_F16_INF is the data-gradient launch (16-bit out, no coefficients, no residual)");
+    return launch_flat<true, 0, true>(p, src_flat16, w_packed, B, blk, st);
+  }
   if (!p.out_f32 && p.res_mode == 0) return launch_flat<true, 0>(p, src_flat16, w_packed, B, blk, st);
   if (!p.out_f32 && p.res_mode == 1 && !p.res_f32) return launch_flat<true, 1>(p, src_flat16, w_packed, B, blk, st);
   return launch_flat<true, 2>(p, src_flat16, w_packed, B, blk, st);

@@ -76,7 +76,8 @@ struct ConvCfg {
 template <int THREADS>
 __device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, %0;" ::"n"(THREADS) : "memory"); }
 
-template <int N>
+// INF: 16-bit output without saturation (the 1x1 data gradients of dynamic loss scaling, op_fmt MCEDM_FMT_F16_INF)
+template <int N, bool INF = false>
 __global__ void __launch_bounds__(ConvCfg<N>::THREADS, 1)
 conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_a0,
                   const __grid_constant__ CUtensorMap tm_a1, const __grid_constant__ CUtensorMap tm_a2,
@@ -298,8 +299,8 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constan
           s2 += (a.x * a.x + a.y * a.y) + (a.z * a.z + a.w * a.w);
           if (p.out_bf16) {
             uint2 o;
-            o.x = pack_op2(a.x, a.y, p.fmt);
-            o.y = pack_op2(a.z, a.w, p.fmt);
+            o.x = pack_op2_g<INF>(a.x, a.y, p.fmt);
+            o.y = pack_op2_g<INF>(a.z, a.w, p.fmt);
             *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(p.out) + opix[itr] * N + c0) = o;
           } else {
             *reinterpret_cast<float4*>(reinterpret_cast<float*>(p.out) + opix[itr] * N + c0) = a;
@@ -339,7 +340,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constan
   }
 }
 
-template <int N>
+template <int N, bool INF = false>
 static int launch_conv(const CUtensorMap& tm_w, const CUtensorMap* tm_a, const ConvParams& p, cudaStream_t stream) {
   using Cfg = ConvCfg<N>;
   ConvParams q = p;
@@ -352,12 +353,12 @@ static int launch_conv(const CUtensorMap& tm_w, const CUtensorMap* tm_a, const C
   static bool attr_set = false;
   static int attr_smem = 0;
   if (!attr_set || smem > attr_smem) {
-    MCEDM_CUDA(cudaFuncSetAttribute(conv_igemm_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
+    MCEDM_CUDA(cudaFuncSetAttribute(conv_igemm_kernel<N, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
     attr_set = true;
     attr_smem = 232448;
   }
   int grid = q.n_tiles < num_sms() ? q.n_tiles : num_sms();
-  MCEDM_CUDA(launch_pdl(conv_igemm_kernel<N>, dim3(grid), dim3(Cfg::THREADS), (size_t)smem, stream, tm_w, tm_a[0], tm_a[1], tm_a[2],
+  MCEDM_CUDA(launch_pdl(conv_igemm_kernel<N, INF>, dim3(grid), dim3(Cfg::THREADS), (size_t)smem, stream, tm_w, tm_a[0], tm_a[1], tm_a[2],
                         tm_a[3], q));
   return 0;
 }
@@ -416,6 +417,10 @@ static int conv_igemm_impl(const void* const* src, int n_src, const int* seg_src
     if (rc) return rc;
   }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (op_fmt == MCEDM_FMT_F16_INF) {
+    MCEDM_REQUIRE(N == 64 && out_bf16, "conv_igemm: op_fmt MCEDM_FMT_F16_INF is the N = 64 16-bit data-gradient launch");
+    return launch_conv<64, true>(tm_w, tm_a, p, st);
+  }
   switch (N) {
     case 16: return launch_conv<16>(tm_w, tm_a, p, st);
     case 64: return launch_conv<64>(tm_w, tm_a, p, st);

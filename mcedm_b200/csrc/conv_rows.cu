@@ -169,7 +169,8 @@ __device__ __forceinline__ uint32_t xf_pair(uint32_t v, float a0, float b0, floa
 }
 
 // RM: residual mode folded at compile time (fused N = 64 instantiations; -1 = runtime p.res_mode)
-template <int N, bool FUSED, int RM = -1, int EP = 0>
+// INF: fp16 stores without saturation (the data-gradient convs of dynamic loss scaling, op_fmt MCEDM_FMT_F16_INF)
+template <int N, bool FUSED, int RM = -1, int EP = 0, bool INF = false>
 __global__ void __launch_bounds__(RowsCfg<N, FUSED>::THREADS, 1)
 conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_h0,
                  const __grid_constant__ CUtensorMap tm_h1, const __grid_constant__ CUtensorMap tm_c0,
@@ -697,8 +698,8 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
             const float aa[4] = {a0, a1, a2, a3};
             sat_audit(p.err, aa);
           }
-          o[2 * c] = pack_f16x2(a0, a1);
-          o[2 * c + 1] = pack_f16x2(a2, a3);
+          o[2 * c] = pack_f16x2_g<INF>(a0, a1);
+          o[2 * c + 1] = pack_f16x2_g<INF>(a2, a3);
         }
         uint16_t* dst = out16p + (r * 128 + q * 32 + lane) * NT + cg;
         stg256(dst, o);
@@ -808,10 +809,10 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
           uint4 o;
-          o.x = pack_f16x2(__uint_as_float(v[8 * c + 0]), __uint_as_float(v[8 * c + 1]));
-          o.y = pack_f16x2(__uint_as_float(v[8 * c + 2]), __uint_as_float(v[8 * c + 3]));
-          o.z = pack_f16x2(__uint_as_float(v[8 * c + 4]), __uint_as_float(v[8 * c + 5]));
-          o.w = pack_f16x2(__uint_as_float(v[8 * c + 6]), __uint_as_float(v[8 * c + 7]));
+          o.x = pack_f16x2_g<INF>(__uint_as_float(v[8 * c + 0]), __uint_as_float(v[8 * c + 1]));
+          o.y = pack_f16x2_g<INF>(__uint_as_float(v[8 * c + 2]), __uint_as_float(v[8 * c + 3]));
+          o.z = pack_f16x2_g<INF>(__uint_as_float(v[8 * c + 4]), __uint_as_float(v[8 * c + 5]));
+          o.w = pack_f16x2_g<INF>(__uint_as_float(v[8 * c + 6]), __uint_as_float(v[8 * c + 7]));
           sts128(st16 + lane * 64 + ((c ^ ((lane >> 1) & 3)) << 4), o);
         }
         __syncwarp();
@@ -838,10 +839,10 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
           sb2 += (a[4] * a[4] + a[5] * a[5]) + (a[6] * a[6] + a[7] * a[7]);
           if (p.dbg & 4) sat_audit(p.err, a);
           uint4 o;
-          o.x = pack_f16x2(a[0], a[1]);
-          o.y = pack_f16x2(a[2], a[3]);
-          o.z = pack_f16x2(a[4], a[5]);
-          o.w = pack_f16x2(a[6], a[7]);
+          o.x = pack_f16x2_g<INF>(a[0], a[1]);
+          o.y = pack_f16x2_g<INF>(a[2], a[3]);
+          o.z = pack_f16x2_g<INF>(a[4], a[5]);
+          o.w = pack_f16x2_g<INF>(a[6], a[7]);
           *reinterpret_cast<uint4*>(out16p + (pix0 + rr) * NT + cg) = o;
         }
         if ((r & 3) == 3) {
@@ -1103,7 +1104,7 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
   }
 }
 
-template <int N, bool FUSED, int RM = -1, int EP = 0>
+template <int N, bool FUSED, int RM = -1, int EP = 0, bool INF = false>
 static int launch_rows(const CUtensorMap& tm_w, const CUtensorMap* tm_h, const CUtensorMap* tm_c, RowsParams p,
                        cudaStream_t stream) {
   using Cfg = RowsCfg<N, FUSED>;
@@ -1135,12 +1136,12 @@ static int launch_rows(const CUtensorMap& tm_w, const CUtensorMap* tm_h, const C
   const int smem = fixed + slots * slot_bytes + p.n_cslots * kCtrBytes;
   static bool attr_set = false;
   if (!attr_set) {
-    MCEDM_CUDA(cudaFuncSetAttribute(conv_rows_kernel<N, FUSED, RM, EP>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
+    MCEDM_CUDA(cudaFuncSetAttribute(conv_rows_kernel<N, FUSED, RM, EP, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
     attr_set = true;
   }
   const long long units = p.total_rows / p.row_align;
   long long grid = units < num_sms() ? units : num_sms();
-  MCEDM_CUDA(launch_pdl(conv_rows_kernel<N, FUSED, RM, EP>, dim3((unsigned)grid), dim3(Cfg::THREADS), (size_t)smem, stream, tm_w,
+  MCEDM_CUDA(launch_pdl(conv_rows_kernel<N, FUSED, RM, EP, INF>, dim3((unsigned)grid), dim3(Cfg::THREADS), (size_t)smem, stream, tm_w,
                         tm_h[0], tm_h[1], tm_c[0], tm_c[1], p));
   return 0;
 }
@@ -1232,9 +1233,16 @@ extern "C" int mcedm_conv_rows_fused(const void* const* halo_src, const float* c
   int rc = rows_common(p, tm_w, tm_h, tm_c, halo_src, n_halo, ctr_src, n_ctr, w_packed, B, H, N);
   if (rc) return rc;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  MCEDM_REQUIRE(op_fmt == 1, "conv_rows_fused: the fused inference kernels are fp16-only (op_fmt = 1)");
+  MCEDM_REQUIRE(op_fmt == 1 || op_fmt == MCEDM_FMT_F16_INF,
+                "conv_rows_fused: the fused inference kernels are fp16-only (op_fmt = 1)");
   MCEDM_REQUIRE(N != 64 || out_16 == 1, "conv_rows_fused: N = 64 writes 16-bit output");
   MCEDM_REQUIRE(N == 32 || n_halo == 1, "conv_rows_fused: N = 16 / 64 take one halo source (K-split 128-channel convs)");
+  if (op_fmt == MCEDM_FMT_F16_INF) {
+    // the data gradient of a 3x3 conv (no transform, no residual) is the one gradient this kernel writes
+    MCEDM_REQUIRE(N == 64 && res_mode == 0 && p.coef[0] == nullptr && !(p.dbg & 128),
+                  "conv_rows_fused: op_fmt MCEDM_FMT_F16_INF is the N = 64 data-gradient launch (no coefficients, no residual)");
+    return launch_rows<64, true, 0, 0, true>(tm_w, tm_h, tm_c, p, st);
+  }
   switch (N) {
     case 16: return launch_rows<16, true>(tm_w, tm_h, tm_c, p, st);
     case 32: return launch_rows<32, true>(tm_w, tm_h, tm_c, p, st);

@@ -121,6 +121,15 @@ __device__ __forceinline__ uint4 pack8(const float4 lo, const float4 hi, int fmt
   o.w = pack_op2(hi.z, hi.w, fmt);
   return o;
 }
+template <bool INF>
+__device__ __forceinline__ uint4 pack8_g(const float4 lo, const float4 hi, int fmt) {
+  uint4 o;
+  o.x = pack_op2_g<INF>(lo.x, lo.y, fmt);
+  o.y = pack_op2_g<INF>(lo.z, lo.w, fmt);
+  o.z = pack_op2_g<INF>(hi.x, hi.y, fmt);
+  o.w = pack_op2_g<INF>(hi.z, hi.w, fmt);
+  return o;
+}
 
 // second term of the split operand: what the 16-bit rounding of (lo, hi) dropped (fp32-accuracy mode, fp16 only)
 __device__ __forceinline__ uint4 pack8_rem(const float4 lo, const float4 hi, const uint4 r) {
@@ -389,7 +398,9 @@ __global__ void __launch_bounds__(256) gn_apply_dropout_kernel(const GnApplyDrop
 }
 
 // in-place g = fp16(g * keep * s) on a 16-bit [B, H, W, 64] tensor (dense, or padded-flat with row pitch `pitch` and
-// `blk` positions per image); one thread per (pixel, 8-channel chunk), padding positions are never touched
+// `blk` positions per image); one thread per (pixel, 8-channel chunk), padding positions are never touched.
+// INF: fp16 stores without saturation (op_fmt MCEDM_FMT_F16_INF, dynamic loss scaling)
+template <bool INF = false>
 __global__ void __launch_bounds__(256) dropout_bwd16_kernel(void* __restrict__ g, int pitch, int blk, int B, int H, int W,
                                                             GnDropout d, int fmt) {
   pdl_wait();
@@ -420,7 +431,7 @@ __global__ void __launch_bounds__(256) dropout_bwd16_kernel(void* __restrict__ g
     const unsigned long long q = (unsigned long long)pix * 16ull + 2ull * (unsigned)c8;
     lo = dropout_apply4(lo, dropout_words(q, d.layer, d.rng), d.thr, d.scale);
     hi = dropout_apply4(hi, dropout_words(q + 1, d.layer, d.rng), d.thr, d.scale);
-    gp[spix * 8 + c8] = pack8(lo, hi, fmt);
+    gp[spix * 8 + c8] = pack8_g<INF>(lo, hi, fmt);
   }
 }
 
@@ -621,7 +632,8 @@ extern "C" int mcedm_dropout_bwd16(void* g16, int pitch, int blk, int B, int H, 
   const long long chunks = (long long)B * H * W * 8;
   long long grid = (chunks + 255) / 256;
   if (grid > 8LL * num_sms()) grid = 8LL * num_sms();
-  MCEDM_CUDA(launch_pdl(dropout_bwd16_kernel, dim3((unsigned)grid), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream), g16,
-                        pitch, blk, B, H, W, d, op_fmt ? 1 : 0));
+  MCEDM_CUDA(launch_pdl(op_fmt == MCEDM_FMT_F16_INF ? dropout_bwd16_kernel<true> : dropout_bwd16_kernel<false>,
+                        dim3((unsigned)grid), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream), g16, pitch, blk, B, H, W,
+                        d, op_fmt ? 1 : 0));
   return 0;
 }

@@ -460,6 +460,15 @@ __device__ __forceinline__ uint4 pack8v(const float (&v)[8], int fmt) {
   o.w = pack_op2(v[6], v[7], fmt);
   return o;
 }
+template <bool INF>
+__device__ __forceinline__ uint4 pack8v_g(const float (&v)[8], int fmt) {
+  uint4 o;
+  o.x = pack_op2_g<INF>(v[0], v[1], fmt);
+  o.y = pack_op2_g<INF>(v[2], v[3], fmt);
+  o.z = pack_op2_g<INF>(v[4], v[5], fmt);
+  o.w = pack_op2_g<INF>(v[6], v[7], fmt);
+  return o;
+}
 __device__ __forceinline__ uint4 ldg16(const void* base, long long pix, int oct) {
   return reinterpret_cast<const uint4*>(base)[pix * 8 + oct];
 }
@@ -710,7 +719,8 @@ __global__ void __launch_bounds__(256) gn_bwd16_reduce_kernel(const GnBwd16Param
 }
 
 // pass 2 of one CTA: dx = k0 du - (k1 + xh k2) + residual-path gradients, 16-bit out, column sums
-template <bool FAST, bool STAGED = false>
+// INF: 16-bit gradient stores without saturation (op_fmt MCEDM_FMT_F16_INF, dynamic loss scaling)
+template <bool FAST, bool STAGED = false, bool INF = false>
 __device__ __forceinline__ void gn16_pass2(const GnBwd16Params& p, float (*red)[64], uint32_t stage = 0) {
   const int b = blockIdx.y;
   const int oct = threadIdx.x & 7, pl = threadIdx.x >> 3;
@@ -786,7 +796,7 @@ __device__ __forceinline__ void gn16_pass2(const GnBwd16Params& p, float (*red)[
         q[0] = make_float4(o[0], o[1], o[2], o[3]);
         q[1] = make_float4(o[4], o[5], o[6], o[7]);
       }
-      const uint4 ov = pack8v(o, p.fmt);
+      const uint4 ov = pack8v_g<INF>(o, p.fmt);
       if (p.dx16) reinterpret_cast<uint4*>(p.dx16)[px * 8 + oct] = ov;
       if (p.dx16_dense) reinterpret_cast<uint4*>(p.dx16_dense)[((long long)b * p.Hin * p.Win + ip) * 8 + oct] = ov;
     }
@@ -840,7 +850,7 @@ __device__ __forceinline__ void gn16_pass2(const GnBwd16Params& p, float (*red)[
             q[0] = make_float4(o[0], o[1], o[2], o[3]);
             q[1] = make_float4(o[4], o[5], o[6], o[7]);
           }
-          const uint4 ov = pack8v(o, p.fmt);
+          const uint4 ov = pack8v_g<INF>(o, p.fmt);
           if (p.dx16) reinterpret_cast<uint4*>(p.dx16)[pix[u] * 8 + oct] = ov;
           if (p.dx16_dense) {
             const int ip = pix0 + i + 32 * u;
@@ -883,7 +893,7 @@ __device__ __forceinline__ void gn16_pass2(const GnBwd16Params& p, float (*red)[
         q[0] = make_float4(o[0], o[1], o[2], o[3]);
         q[1] = make_float4(o[4], o[5], o[6], o[7]);
       }
-      const uint4 ov = pack8v(o, p.fmt);
+      const uint4 ov = pack8v_g<INF>(o, p.fmt);
       if (p.dx16) reinterpret_cast<uint4*>(p.dx16)[pix * 8 + oct] = ov;
       if (p.dx16_dense) reinterpret_cast<uint4*>(p.dx16_dense)[((long long)b * p.Hin * p.Win + ip) * 8 + oct] = ov;
     }
@@ -901,10 +911,10 @@ __device__ __forceinline__ void gn16_pass2(const GnBwd16Params& p, float (*red)[
   }
 }
 
-template <bool FAST>
+template <bool FAST, bool INF = false>
 __global__ void __launch_bounds__(256, 2) gn_bwd16_apply_kernel(const GnBwd16Params p) {
   __shared__ float red[32][64];
-  gn16_pass2<FAST>(p, red);
+  gn16_pass2<FAST, false, INF>(p, red);
 }
 
 // Both passes in ONE kernel (p.fused).  The grid is about one wave of co-resident CTAs (pick_pix_per_cta16; the launcher
@@ -915,7 +925,7 @@ __global__ void __launch_bounds__(256, 2) gn_bwd16_apply_kernel(const GnBwd16Par
 // departures (the last one clears the flag): every word is zero again when the launch ends.  The spin is bounded like the
 // mbarrier waits (a protocol bug must not hang the GPU): on timeout the CTA goes on with whatever kcoef holds and
 // records the tag in *err.
-template <bool FAST1, bool FAST2>
+template <bool FAST1, bool FAST2, bool INF = false>
 __global__ void __launch_bounds__(256, 2) gn_bwd16_fused_kernel(const GnBwd16Params p) {
   __shared__ float red[32][64][2];
   __shared__ float sG1[64], sG2[64];
@@ -939,7 +949,7 @@ __global__ void __launch_bounds__(256, 2) gn_bwd16_fused_kernel(const GnBwd16Par
     __threadfence();
   }
   __syncthreads();
-  gn16_pass2<FAST2, FAST2>(p, reinterpret_cast<float(*)[64]>(&red[0][0][0]), stage);
+  gn16_pass2<FAST2, FAST2, INF>(p, reinterpret_cast<float(*)[64]>(&red[0][0][0]), stage);
   __syncthreads();
   if (threadIdx.x == 0) {
     if (atomicAdd(p.ticket + 2 * p.B + b, 1u) == (unsigned)p.ctas_per_img - 1u) {
@@ -1018,6 +1028,43 @@ extern "C" int mcedm_gn_bwd(const float* dy, const float* x, const float* meanrs
 }
 
 
+namespace mcedm {
+template <bool INF>
+static int gn_bwd16_launch(GnBwd16Params& p, dim3 grid, int resample, bool fast2, int split, cudaStream_t st) {
+  // one kernel when every CTA of the grid is resident at once (2 per SM): the in-kernel wait needs the sample's CTAs live
+  if (!split && (long long)p.ctas_per_img * p.B <= 2LL * num_sms() && p.pix_per_cta % 64 == 0) {   // (staged batches: 64 pixels)
+    p.fused = 1;
+    p.err = watchdog_ptr();
+    MCEDM_REQUIRE(p.err != nullptr, "gn_bwd16: cannot allocate the watchdog word");
+    static bool attr = false;
+    if (!attr) {
+      MCEDM_CUDA(cudaFuncSetAttribute(gn_bwd16_fused_kernel<true, true, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize, kGnStageBytes));
+      MCEDM_CUDA(cudaFuncSetAttribute(gn_bwd16_fused_kernel<true, false, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize, kGnStageBytes));
+      attr = true;
+    }
+    if (resample == 0 && fast2) gn_bwd16_fused_kernel<true, true, INF><<<grid, 256, kGnStageBytes, st>>>(p);
+    else if (resample == 0) gn_bwd16_fused_kernel<true, false, INF><<<grid, 256, kGnStageBytes, st>>>(p);
+    else gn_bwd16_fused_kernel<false, false, INF><<<grid, 256, 0, st>>>(p);
+    MCEDM_CUDA(cudaGetLastError());
+    return 0;
+  }
+  if (resample == 0) {
+    gn_bwd16_reduce_kernel<true><<<grid, 256, 0, st>>>(p);
+  } else {
+    gn_bwd16_reduce_kernel<false><<<grid, 256, 0, st>>>(p);
+  }
+  MCEDM_CUDA(cudaGetLastError());
+  if (fast2) {      // the batched pass takes 16-bit residual-path gradients at the same resolution only
+    gn_bwd16_apply_kernel<true, INF><<<grid, 256, 0, st>>>(p);
+  } else {
+    gn_bwd16_apply_kernel<false, INF><<<grid, 256, 0, st>>>(p);
+  }
+  MCEDM_CUDA(cudaGetLastError());
+  return 0;
+}
+
+}  // namespace mcedm
+
 extern "C" int mcedm_gn_bwd16(const void* dy16, int dy_pitch, int dy_blk, const void* x16, int x_pitch, int x_blk,
                               int op_fmt, const float* meanrstd, const float* coef_ab, const float* gamma,
                               const float* beta, const float* scale_shift, int emb_batch_stride, int emb_shift_offset,
@@ -1064,38 +1111,8 @@ extern "C" int mcedm_gn_bwd16(const void* dy16, int dy_pitch, int dy_blk, const 
     const char* e = getenv("MCEDM_GNBWD_SPLIT");
     split = (e && atoi(e)) ? 1 : 0;
   }
-  // one kernel when every CTA of the grid is resident at once (2 per SM): the in-kernel wait needs the sample's CTAs live
-  if (!split && (long long)p.ctas_per_img * B <= 2LL * num_sms() && p.pix_per_cta % 64 == 0) {   // (staged batches: 64 pixels)
-    p.fused = 1;
-    p.err = watchdog_ptr();
-    MCEDM_REQUIRE(p.err != nullptr, "gn_bwd16: cannot allocate the watchdog word");
-    static bool attr = false;
-    if (!attr) {
-      MCEDM_CUDA(cudaFuncSetAttribute(gn_bwd16_fused_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kGnStageBytes));
-      MCEDM_CUDA(cudaFuncSetAttribute(gn_bwd16_fused_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kGnStageBytes));
-      attr = true;
-    }
-    if (resample == 0 && fast2) gn_bwd16_fused_kernel<true, true><<<grid, 256, kGnStageBytes, st>>>(p);
-    else if (resample == 0) gn_bwd16_fused_kernel<true, false><<<grid, 256, kGnStageBytes, st>>>(p);
-    else gn_bwd16_fused_kernel<false, false><<<grid, 256, 0, st>>>(p);
-    MCEDM_CUDA(cudaGetLastError());
-    return 0;
-  }
-  if (resample == 0) {
-    gn_bwd16_reduce_kernel<true><<<grid, 256, 0, st>>>(p);
-  } else {
-    gn_bwd16_reduce_kernel<false><<<grid, 256, 0, st>>>(p);
-  }
-  MCEDM_CUDA(cudaGetLastError());
-  // the batched pass takes 16-bit residual-path gradients at the same resolution only
-  const bool fast = resample == 0 && (add0 == nullptr || (add0_mode == 0 && p.add16)) && (add1 == nullptr || p.add16);
-  if (fast) {
-    gn_bwd16_apply_kernel<true><<<grid, 256, 0, st>>>(p);
-  } else {
-    gn_bwd16_apply_kernel<false><<<grid, 256, 0, st>>>(p);
-  }
-  MCEDM_CUDA(cudaGetLastError());
-  return 0;
+  if (op_fmt == MCEDM_FMT_F16_INF) return gn_bwd16_launch<true>(p, grid, resample, fast2, split, st);
+  return gn_bwd16_launch<false>(p, grid, resample, fast2, split, st);
 }
 
 extern "C" int mcedm_reduce_rows(const float* in, int n_rows, long long stride_r, int n_cols, long long stride_j,

@@ -291,6 +291,22 @@ __device__ __forceinline__ uint32_t pack_f16x2(float lo, float hi) {
 __device__ __forceinline__ uint32_t pack_op2(float lo, float hi, int fmt) {
   return fmt ? pack_f16x2(lo, hi) : pack_bf16x2(lo, hi);
 }
+// Gradient stores of dynamic loss scaling (op_fmt MCEDM_FMT_F16_INF): no `satfinite`, so a value beyond fp16's range
+// becomes inf, reaches the fp32 flat gradient through the weight-gradient contractions and makes the step skip.
+// INF = false is the saturating conversion above, instruction for instruction.
+__device__ __forceinline__ uint32_t pack_f16x2_inf(float lo, float hi) {
+  uint32_t r;
+  asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+  return r;
+}
+template <bool INF>
+__device__ __forceinline__ uint32_t pack_f16x2_g(float lo, float hi) {
+  return INF ? pack_f16x2_inf(lo, hi) : pack_f16x2(lo, hi);
+}
+template <bool INF>
+__device__ __forceinline__ uint32_t pack_op2_g(float lo, float hi, int fmt) {
+  return INF ? pack_f16x2_inf(lo, hi) : pack_op2(lo, hi, fmt);
+}
 __device__ __forceinline__ float2 unpack_f16x2(uint32_t v) {
   float lo, hi;
   asm("{\n\t.reg .b16 l, h;\n\tmov.b32 {l, h}, %2;\n\tcvt.f32.f16 %0, l;\n\tcvt.f32.f16 %1, h;\n\t}\n"

@@ -101,6 +101,22 @@ nchw_to_nhwc_pad_kernel(const float* __restrict__ a, int Ca, const float* __rest
     d[Ca + c] = (unsigned short)(pack_op2(scale * bsrc[(b * Cb + c) * HW + hw], 0.f, fmt) & 0xffffu);
 }
 
+// the same for the loss-scaled dL/dF of dynamic loss scaling: the scale is read from device memory (a graph replay sees
+// the current one) and the fp16 conversion does not saturate (S * dL/dF beyond 65504 becomes inf: the step skips)
+__global__ void __launch_bounds__(256)
+nchw_to_nhwc_pad_scaled_kernel(const float* __restrict__ a, int Ca, const float* __restrict__ bsrc, int Cb, long long HW,
+                               long long total_pix, unsigned short* __restrict__ dst, int c_dst0,
+                               const float* __restrict__ scale_dev) {
+  const long long pix = (long long)blockIdx.x * 256 + threadIdx.x;
+  if (pix >= total_pix) return;
+  const float scale = *scale_dev;
+  const long long b = pix / HW, hw = pix - b * HW;
+  unsigned short* d = dst + pix * 64 + c_dst0;
+  for (int c = 0; c < Ca; ++c) d[c] = (unsigned short)(pack_f16x2_inf(scale * a[(b * Ca + c) * HW + hw], 0.f) & 0xffffu);
+  for (int c = 0; c < Cb; ++c)
+    d[Ca + c] = (unsigned short)(pack_f16x2_inf(scale * bsrc[(b * Cb + c) * HW + hw], 0.f) & 0xffffu);
+}
+
 // grid = n_ctas, block = 256 = 8 channel-octets x 32 pixel lanes; x is [pixels][C] bf16, this launch sums the
 // 64 channels starting at c_off.  partial[cta][64]
 __global__ void __launch_bounds__(256)
@@ -256,25 +272,45 @@ sumsq_partial_kernel(const float* __restrict__ g, long long n, double* __restric
 
 // torch.optim.Adam (single-tensor path, no amsgrad, coupled weight decay) with the clip_grad_norm_ coefficient
 // folded in:  g <- g * min(1, max_norm / (||g|| + 1e-6)).  norm_partial may be NULL (no clipping).
+// DYN (dynamic loss scaling): norm_partial is always given and clipping runs iff max_norm > 0; a non-finite sum of
+// squares is found-inf (block 0 stores it) and the step writes nothing; the bias corrections come from the applied-step
+// count in device memory (*step_count + 1; mcedm_loss_scale_update advances it).
+template <bool DYN = false>
 __global__ void __launch_bounds__(256)
 adam_step_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
                  long long n, float lr, float beta1, float beta2, float eps, float weight_decay, float bc1, float bc2_sqrt,
                  const double* __restrict__ norm_partial, int n_partial, float max_norm, float grad_scale,
-                 float* __restrict__ norm_out) {
-  __shared__ float s_coef;
+                 float* __restrict__ norm_out, const int* __restrict__ step_count, float* __restrict__ found_inf) {
+  __shared__ float s_coef, s_bc1, s_bc2;
+  __shared__ int s_skip;
   if (threadIdx.x == 0) {
     float coef = grad_scale;
     if (norm_partial) {
       double t = 0.0;
       for (int i = 0; i < n_partial; ++i) t += norm_partial[i];
       const float nrm = (float)sqrt(t) * grad_scale;
-      const float c = max_norm / (nrm + 1e-6f);
-      coef *= c < 1.0f ? c : 1.0f;
-      if (norm_out && blockIdx.x == 0) *norm_out = nrm;
+      if (!DYN || max_norm > 0.f) {
+        const float c = max_norm / (nrm + 1e-6f);
+        coef *= c < 1.0f ? c : 1.0f;
+        if (norm_out && blockIdx.x == 0) *norm_out = nrm;
+      }
+      if (DYN) {
+        const bool inf = !isfinite(t);
+        if (blockIdx.x == 0) *found_inf = inf ? 1.0f : 0.0f;
+        s_skip = inf ? 1 : 0;
+        const double step = (double)(*step_count + 1);
+        s_bc1 = (float)(1.0 - pow((double)beta1, step));
+        s_bc2 = (float)sqrt(1.0 - pow((double)beta2, step));
+      }
     }
     s_coef = coef;
   }
   __syncthreads();
+  if (DYN) {
+    if (s_skip) return;
+    bc1 = s_bc1;
+    bc2_sqrt = s_bc2;
+  }
   const float coef = s_coef;
   const float step_size = lr / bc1;
   for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n; i += (long long)gridDim.x * 256) {
@@ -288,6 +324,35 @@ adam_step_kernel(float* __restrict__ p, const float* __restrict__ g, float* __re
     const float denom = sqrtf(vi) / bc2_sqrt + eps;
     p[i] = pi - step_size * (mi / denom);
   }
+}
+
+// torch._amp_update_scale_ (aten/src/ATen/native/cuda/AmpKernels.cu) on one thread, plus the applied-step count of the
+// fused Adam: +1 when the step applied
+__global__ void __launch_bounds__(32)
+loss_scale_update_kernel(float* __restrict__ scale, int* __restrict__ tracker, const float* __restrict__ found_inf,
+                         int* __restrict__ step_count, float growth, float backoff, int interval) {
+  if (threadIdx.x != 0) return;
+  if (*found_inf != 0.0f) {
+    *scale = *scale * backoff;
+    *tracker = 0;
+    return;
+  }
+  if (step_count) *step_count += 1;
+  const int successful = *tracker + 1;
+  if (successful == interval) {
+    const float grown = *scale * growth;
+    if (isfinite(grown)) *scale = grown;          // never grows past fp32's range
+    *tracker = 0;
+  } else {
+    *tracker = successful;
+  }
+}
+
+// g <- g * (1 / scale): the loss scale comes off the flat gradient (power-of-two scales: exact)
+__global__ void __launch_bounds__(256)
+grad_unscale_kernel(float* __restrict__ g, long long n, const float* __restrict__ scale) {
+  const float inv = 1.0f / *scale;
+  for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n; i += (long long)gridDim.x * 256) g[i] *= inv;
 }
 
 __global__ void __launch_bounds__(256)
@@ -380,6 +445,18 @@ extern "C" int mcedm_nchw_to_nhwc_pad16(const float* a, int Ca, const float* b, 
   return 0;
 }
 
+extern "C" int mcedm_nchw_to_nhwc_pad16_scaled(const float* a, int Ca, const float* b, int Cb, int B, int H, int W,
+                                               void* dst16, int c_dst0, const float* scale, int op_fmt, void* stream) {
+  using namespace mcedm;
+  MCEDM_REQUIRE(Ca >= 0 && Cb >= 0 && Ca + Cb >= 1 && c_dst0 >= 0 && c_dst0 + Ca + Cb <= 64, "nchw_to_nhwc_pad: channels");
+  MCEDM_REQUIRE(scale && op_fmt == MCEDM_FMT_F16_INF, "nchw_to_nhwc_pad16_scaled: needs a device scale and op_fmt 3");
+  const long long HW = (long long)H * W, total = HW * B;
+  nchw_to_nhwc_pad_scaled_kernel<<<(unsigned)((total + 255) / 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      a, Ca, b, Cb, HW, total, reinterpret_cast<unsigned short*>(dst16), c_dst0, scale);
+  MCEDM_CUDA(cudaGetLastError());
+  return 0;
+}
+
 extern "C" int mcedm_nchw_to_nhwc_pad(const float* a, int Ca, const float* b, int Cb, int B, int H, int W, void* dst_bf16,
                                       int c_dst0, void* stream) {
   return mcedm_nchw_to_nhwc_pad16(a, Ca, b, Cb, B, H, W, dst_bf16, c_dst0, 1.0f, 0, stream);
@@ -434,7 +511,42 @@ extern "C" int mcedm_adam_step(float* p, const float* g, float* m, float* v, lon
   if (grid > 4 * num_sms()) grid = 4 * num_sms();
   adam_step_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
       p, g, m, v, n, lr, beta1, beta2, eps, weight_decay, (float)bc1, (float)sqrt(bc2), norm_partial, n_partial,
-      max_norm, grad_scale, norm_out);
+      max_norm, grad_scale, norm_out, nullptr, nullptr);
+  MCEDM_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mcedm_adam_step_dyn(float* p, const float* g, float* m, float* v, long long n, float lr, float beta1,
+                                   float beta2, float eps, float weight_decay, const int* step_count,
+                                   const double* norm_partial, int n_partial, float max_norm, float grad_scale,
+                                   float* norm_out, float* found_inf, void* stream) {
+  using namespace mcedm;
+  MCEDM_REQUIRE(n >= 1 && n_partial >= 1 && step_count && norm_partial && found_inf, "adam_step_dyn: bad arguments");
+  int grid = (int)((n + 255) / 256);
+  if (grid > 4 * num_sms()) grid = 4 * num_sms();
+  adam_step_kernel<true><<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      p, g, m, v, n, lr, beta1, beta2, eps, weight_decay, 1.0f, 1.0f, norm_partial, n_partial, max_norm, grad_scale,
+      norm_out, step_count, found_inf);
+  MCEDM_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mcedm_loss_scale_update(float* scale, int* growth_tracker, const float* found_inf, int* step_count,
+                                       float growth_factor, float backoff_factor, int growth_interval, void* stream) {
+  using namespace mcedm;
+  MCEDM_REQUIRE(scale && growth_tracker && found_inf && growth_interval >= 1, "loss_scale_update: bad arguments");
+  loss_scale_update_kernel<<<1, 32, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      scale, growth_tracker, found_inf, step_count, growth_factor, backoff_factor, growth_interval);
+  MCEDM_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mcedm_grad_unscale(float* g, long long n, const float* scale, void* stream) {
+  using namespace mcedm;
+  MCEDM_REQUIRE(n >= 1 && scale, "grad_unscale: bad arguments");
+  int grid = (int)((n + 255) / 256);
+  if (grid > 4 * num_sms()) grid = 4 * num_sms();
+  grad_unscale_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(g, n, scale);
   MCEDM_CUDA(cudaGetLastError());
   return 0;
 }

@@ -133,6 +133,8 @@ class UNetEngine(TrainMixin, Train16Mixin, FusedMixin, PreciseMixin, PackMixin):
         # engine first trains, unless set), counter word = step (one per training-mode forward)
         self.dropout_seed: Optional[int] = None
         self.dropout_step = 0
+        # dynamic loss scaling of the fused16 plan's backward (loss_scale.LossScaler; None = the static scale)
+        self.loss_scaler = None
         # inference plan: True = GroupNorm fused into the convs + 16-bit activations (fused_engine.py);
         # False = the unfused fp32-stream plan below (what training's forward uses)
         self.fused = os.environ.get("MCEDM_FUSED", "1") != "0"
@@ -228,11 +230,11 @@ class UNetEngine(TrainMixin, Train16Mixin, FusedMixin, PreciseMixin, PackMixin):
         return t
 
     # ------------------------------------------------------------------ launches
-    def _conv(self, srcs, segs, w, bias, B, H, W, N, out, out_bf16, res, res_mode, stats, st):
+    def _conv(self, srcs, segs, w, bias, B, H, W, N, out, out_bf16, res, res_mode, stats, st, fmt=None):
         L.check(self.lib.mcedm_conv_igemm(
             L.ptr_array(srcs), len(srcs), L.int_array([s[0] for s in segs]), L.int_array([s[1] for s in segs]),
             L.int_array([s[2] for s in segs]), len(segs), L.ptr(w), L.ptr(bias), B, H, W, N, L.ptr(out), out_bf16,
-            L.ptr(res), res_mode, L.ptr(stats), self._fmt, st), "conv_igemm")
+            L.ptr(res), res_mode, L.ptr(stats), self._fmt if fmt is None else fmt, st), "conv_igemm")
 
     def _flat_geom(self, H, W):
         pitch, blk = C.c_int(0), C.c_int(0)

@@ -45,6 +45,7 @@ from einops import rearrange
 from . import _lib as L
 from .adm_blocks import DhariwalUNet
 from .config import AttrDict
+from .loss_scale import active_scaler
 from .nn_misc import EmaModel, MaskedLoss, NoiseEstimationLoss, Normalizer, fused_masked_mae
 from .pde_loss import DarcyLoss, get_pde_loss_function
 from .runner import LightningModule
@@ -184,6 +185,7 @@ class PlMcedm(LightningModule):
             opt = FusedAdam(params, lr=self.lr, weight_decay=self.weight_decay, betas=(self.beta1, 0.999),
                             amsgrad=self.amsgrad, eps=self.eps)
             opt.grad_provider = lambda: self.model.engine().flat_grad()
+            opt.loss_scaler_provider = lambda: active_scaler(self.model)
         elif self.optimizer == "RMSProp":
             opt = torch.optim.RMSprop(params, lr=self.lr, weight_decay=self.weight_decay)
         elif self.optimizer == "SGD":
@@ -320,7 +322,8 @@ class PlMcedm(LightningModule):
 
         unet = self.model
         params = list(unet.parameters())
-        key = (tuple(x.shape), x.device.index, params[0].data_ptr(), params[-1].data_ptr())
+        # the backward graph captures the loss-scaling mode and the scaler's device words
+        key = (tuple(x.shape), x.device.index, params[0].data_ptr(), params[-1].data_ptr(), active_scaler(unet))
         graphs = self.__dict__.setdefault("_train_graphs", {})
         tg = graphs.get(key)
         if tg is None:

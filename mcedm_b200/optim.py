@@ -5,6 +5,10 @@ configs/trainer/trainer_ddim.yaml:8-9 gradient_clip_val).
 `FusedAdam` keeps torch.optim.Adam's constructor arguments, `param_groups` and `state_dict()` layout
 (`step`, `exp_avg`, `exp_avg_sq` per parameter) so checkpoints interchange; the parameters are re-bound as views
 of one contiguous buffer, which is also what the data-parallel gradient all-reduce runs on.
+
+Under dynamic loss scaling (loss_scale.py; `loss_scaler_provider` returns the engine's LossScaler) a step is
+sum-of-squares partials -> Adam that writes nothing when they are not finite (found-inf) -> the scale update.  The
+applied-step count then lives in device memory (no host synchronisation per step); `state_dict()` reads it back.
 """
 from __future__ import annotations
 
@@ -62,6 +66,8 @@ class FusedAdam(torch.optim.Adam):
         self.max_grad_norm = max_grad_norm      # set by the trainer from gradient_clip_val
         self.grad_scale = 1.0                   # 1/world_size when the all-reduce sums
         self.grad_provider = None               # callable -> the engine's flat gradient buffer (zero-copy path)
+        self.loss_scaler_provider = None        # callable -> the engine's LossScaler or None (dynamic loss scaling)
+        self._step_dev = None                   # int32 [1]: applied steps, while dynamic loss scaling steps
         self._params = list(self.param_groups[0]["params"])
         self._flat_p = None
         self._flat_g = None
@@ -72,6 +78,7 @@ class FusedAdam(torch.optim.Adam):
             self._bind()
 
     def _bind(self):
+        self._sync_steps()
         if not self._params[0].is_cuda:
             raise L.McedmError("FusedAdam needs CUDA parameters: the optimizer kernels have no CPU path")
         dev = self._params[0].device
@@ -146,6 +153,34 @@ class FusedAdam(torch.optim.Adam):
         torch._foreach_copy_(views, srcs)
         return self._flat_g
 
+    def _sync_steps(self):
+        """Host step counter <- the device one (synchronises; only while dynamic loss scaling has stepped)."""
+        if self._step_dev is not None:
+            self._steps = int(self._step_dev.item())
+            self._step_t.fill_(float(self._steps))
+
+    def state_dict(self):
+        self._sync_steps()
+        return super().state_dict()
+
+    def _step_dynamic(self, scaler, p, g, grp, st):
+        lib = L.lib()
+        dev = p.device
+        scaler.state(dev)
+        if self._step_dev is None or self._step_dev.device != dev:
+            self._sync_steps()
+            self._step_dev = torch.full((1,), self._steps, dtype=torch.int32, device=dev)
+        n = p.numel()
+        clip = self.max_grad_norm is not None and self.max_grad_norm > 0
+        L.check(lib.mcedm_sumsq_partial(L.ptr(g), n, L.ptr(self._partial), self._n_partial, st), "sumsq_partial")
+        L.check(lib.mcedm_adam_step_dyn(L.ptr(p), L.ptr(g), L.ptr(self._m), L.ptr(self._v), n, float(grp["lr"]),
+                                        float(grp["betas"][0]), float(grp["betas"][1]), float(grp["eps"]),
+                                        float(grp["weight_decay"]), L.ptr(self._step_dev), L.ptr(self._partial),
+                                        self._n_partial, float(self.max_grad_norm) if clip else 0.0,
+                                        float(self.grad_scale), L.ptr(self.last_grad_norm), L.ptr(scaler.found_inf_t),
+                                        st), "adam_step_dyn")
+        scaler.update(self._step_dev, st)
+
     @torch.no_grad()
     def step(self, closure=None, flat_grads: Optional[torch.Tensor] = None):
         loss = closure() if closure is not None else None
@@ -156,6 +191,15 @@ class FusedAdam(torch.optim.Adam):
         p = self.flat_params()
         g = flat_grads if flat_grads is not None else self.flat_grads()
         st = L.stream_ptr()
+        scaler = self.loss_scaler_provider() if self.loss_scaler_provider is not None else None
+        if scaler is not None:
+            self._step_dynamic(scaler, p, g, grp, st)
+            self._pending_g = None
+            WEIGHT_EPOCH[0] += 1
+            return loss
+        if self._step_dev is not None:          # dynamic loss scaling was switched off: the host counter continues
+            self._sync_steps()
+            self._step_dev = None
         n = p.numel()
         self._steps += 1
         clip = self.max_grad_norm is not None and self.max_grad_norm > 0
@@ -184,6 +228,8 @@ class FusedAdam(torch.optim.Adam):
             s["step"] = self._step_t
             off += n
         self._step_t.fill_(float(self._steps))
+        if self._step_dev is not None:
+            self._step_dev.fill_(self._steps)
 
 
 def ema_update_(ema_params, cur_params, beta: float, state: dict):

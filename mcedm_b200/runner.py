@@ -13,7 +13,9 @@ this module provides the minimum that keeps the reference's module code shape in
     clip -> optimizer_step (module hook, which also updates the EMA) -> validation_step / test_step;
   * `ModelCheckpoint` — `checkpoints/last.ckpt` with Lightning's top-level key layout (`state_dict`,
     `optimizer_states`, `epoch`, `global_step`, `hyper_parameters`, ...); `fit(ckpt_path=...)` resumes like
-    `trainer.fit(ckpt_path=...)` of run.py:99: weights, Adam moments + step counter, global step, next epoch.
+    `trainer.fit(ckpt_path=...)` of run.py:99: weights, Adam moments + step counter, global step, next epoch;
+  * `precision=16` / "16" / "16-mixed" — dynamic loss scaling (loss_scale.py) of a network training on the fp16 plan,
+    checkpointed as Lightning's `native_amp_scaling_state` (torch.amp.GradScaler.state_dict() layout).
 
 Data parallelism is THIS trainer's flat all-reduce; the kernels' autograd nodes bind `p.grad` to slices of the engine's
 flat gradient buffer directly, so the per-parameter reducer hooks of `torch.nn.parallel.DistributedDataParallel`
@@ -101,6 +103,9 @@ class ModelCheckpoint:
         }
         if trainer.optimizer is not None:
             ckpt["optimizer_states"] = [trainer.optimizer.state_dict()]
+        scaler = trainer.loss_scaler(module)
+        if scaler is not None:
+            ckpt["native_amp_scaling_state"] = scaler.state_dict()
         torch.save(ckpt, os.path.join(self.dirpath, f"{self.format_name(epoch, module.global_step)}.ckpt"))
         if self.save_last:
             torch.save(ckpt, os.path.join(self.dirpath, "last.ckpt"))
@@ -116,6 +121,7 @@ class Trainer:
             raise NotImplementedError("only gradient_clip_algorithm='norm' is supported")
         self.max_epochs, self.max_steps = max_epochs, max_steps
         self.gradient_clip_val = gradient_clip_val
+        self.precision = precision
         self.check_val_every_n_epoch = check_val_every_n_epoch
         self.callbacks = list(callbacks or [])
         self.datamodule = None
@@ -143,6 +149,31 @@ class Trainer:
             out[name] = float(m)
         self.metrics.clear()
         return out
+
+    # ---- dynamic loss scaling --------------------------------------------------------------------
+    def loss_scaler(self, module):
+        """The LossScaler of the module's network when it trains on the fp16 plan with dynamic scaling, else None."""
+        from .loss_scale import active_scaler
+
+        net = getattr(module, "model", None)
+        return active_scaler(net) if net is not None else None
+
+    def _enable_loss_scaling(self, module):
+        """precision 16 / "16" / "16-mixed": a LossScaler on the network's engine when its backward runs on the fp16
+        plan (other precision values and the fp32-stream plan keep the static path)."""
+        from .loss_scale import LossScaler, dynamic_precision
+
+        net = getattr(module, "model", None)
+        if not dynamic_precision(self.precision) or net is None or not hasattr(net, "engine"):
+            return
+        eng = net.engine()
+        if getattr(eng, "train_plan", None) == "fused16" and getattr(eng, "loss_scaler", None) is None:
+            from .optim import FusedAdam
+
+            if not isinstance(self.optimizer, FusedAdam):
+                raise NotImplementedError("dynamic loss scaling skips steps inside the fused Adam kernel: precision=16 "
+                                          "needs optimizer 'Adam'")
+            eng.loss_scaler = LossScaler()
 
     # ---- data-parallel gradient exchange -------------------------------------------------------
     def _allreduce_grads(self, params):
@@ -186,6 +217,7 @@ class Trainer:
         module.setup("fit")
         self.optimizer = module.configure_optimizers()["optimizer"]
         self.optimizers = [self.optimizer]
+        self._enable_loss_scaling(module)
         params = [p for g in self.optimizer.param_groups for p in g["params"]]
         from .optim import FusedAdam
 
@@ -202,6 +234,9 @@ class Trainer:
             module.load_state_dict(ckpt["state_dict"])
             if ckpt.get("optimizer_states"):
                 self.optimizer.load_state_dict(ckpt["optimizer_states"][0])
+            scaler = self.loss_scaler(module)
+            if scaler is not None and ckpt.get("native_amp_scaling_state"):
+                scaler.load_state_dict(ckpt["native_amp_scaling_state"])
             module.global_step = step = int(ckpt.get("global_step", 0))
             first_epoch = int(ckpt.get("epoch", -1)) + 1
             net = getattr(module, "model", None)

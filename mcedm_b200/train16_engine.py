@@ -12,6 +12,9 @@ inference data flow (fused_engine.py) for the forward and mirrors it in the back
   backward  = fp16 as well, LOSS-SCALED: dL/dF enters as S * dL/dF (S = 1024; with EDM preconditioning
               dL/dF = (2/B) m (F - F_target), O(1/B) for every noise level, so a static scale is enough; conversions
               saturate instead of overflowing) and the flat gradient buffer is multiplied by 1/S at the end.
+              With a LossScaler on the engine (loss_scale.py) S is read from device memory and the gradient stores
+              do not saturate (op_fmt MCEDM_FMT_F16_INF): an overflow reaches the flat gradient as inf / NaN and
+              the optimizer step skips.
               * data gradients of the 3x3 convs = the fused forward kernels on 16-bit gradients (no transform),
                 writing 16-bit;
               * GroupNorm(+SiLU, scale/shift, resample) backward = mcedm_gn_bwd16: raw fp16 x, 16-bit dy, 16-bit
@@ -141,10 +144,10 @@ class Train16Mixin:
         flat = self._fgeom(ws, H, W)
         if flat is None:
             L.check(self.lib.mcedm_conv_rows_fused(L.ptr_array([src]), None, 1, None, 0, L.ptr(wd), None, B, H, 64, 0, 64,
-                                                   L.ptr(out), 1, None, 0, 0, 0, None, self._fmt, st), "conv_rows_fused")
+                                                   L.ptr(out), 1, None, 0, 0, 0, None, self._gfmt, st), "conv_rows_fused")
         else:
             L.check(self.lib.mcedm_conv_flat_fused(L.ptr(src), None, L.ptr(wd), None, B, H, W, 64, L.ptr(out), 0, None, 0,
-                                                   0, 0, 0, None, self._fmt, st), "conv_flat_fused")
+                                                   0, 0, 0, None, self._gfmt, st), "conv_flat_fused")
 
     def _gn_bwd16(self, ws, dy, dy_lay, x: Act, mr, coef, gamma, beta, ss, act, rs, B, dgamma, dbeta, dss, add0, add0_mode,
                   add0_lay, add1, pend, gs, want_dense, st):
@@ -168,7 +171,7 @@ class Train16Mixin:
         else:
             dx16 = pend
         xl = x.flat if x.flat is not None else (0, 0)
-        L.check(lib.mcedm_gn_bwd16(L.ptr(dy), dy_lay[0], dy_lay[1], L.ptr(x.t), xl[0], xl[1], self._fmt, L.ptr(mr),
+        L.check(lib.mcedm_gn_bwd16(L.ptr(dy), dy_lay[0], dy_lay[1], L.ptr(x.t), xl[0], xl[1], self._gfmt, L.ptr(mr),
                                    L.ptr(coef), L.ptr(gamma), L.ptr(beta), L.ptr(ss), 128, 64, act, rs, B, Hin, Win, L.ptr(red),
                                    L.ptr(kcoef), L.ptr(ticket), L.ptr(dgb), L.ptr(dss), 128, L.ptr(add0), add0_mode,
                                    add0_lay[0], add0_lay[1], L.ptr(add1), 0 if self.GRAD_MASTER_FP32 else 1,
@@ -179,7 +182,8 @@ class Train16Mixin:
         self._reduce_rows(flat_dgb[1:], B, 128, 64, 2, dbeta, st)
 
     def _igemm1x1(self, srcs, w, B, H, W, N, out, out16, st):
-        self._conv(srcs, [(i, 0, 0) for i in range(len(srcs))], w, None, B, H, W, N, out, out16, None, 0, None, st)
+        self._conv(srcs, [(i, 0, 0) for i in range(len(srcs))], w, None, B, H, W, N, out, out16, None, 0, None, st,
+                   fmt=self._gfmt if out16 else None)
 
     # ------------------------------------------------------------------ backward
     @torch.no_grad()
@@ -192,6 +196,9 @@ class Train16Mixin:
         st = L.stream_ptr()
         G = self.grad_of
         fmt = self._fmt
+        scaler = self.loss_scaler.state(dev) if self.loss_scaler is not None else None
+        # format of the 16-bit gradient stores: fp16 without saturation under dynamic loss scaling
+        self._gfmt = L.FMT_F16_INF if scaler is not None else fmt
         S = float(self.LOSS_SCALE)
         dF = dF.contiguous()
         self._jid, self._rjobs, self._wjobs, self._job_refs, self._post_copies = 0, [], [], [], []
@@ -248,8 +255,12 @@ class Train16Mixin:
 
         # ---- head: out_conv(silu(out_norm(x)))
         dFp = self._fbuf(ws, "dFp", (B, H, W, 64), self._dt16(), dev, zero=True)
-        L.check(lib.mcedm_nchw_to_nhwc_pad16(L.ptr(dF), u.out_channels, None, 0, B, H, W, L.ptr(dFp), 0, S, fmt, st),
-                "pad dF")
+        if scaler is None:
+            L.check(lib.mcedm_nchw_to_nhwc_pad16(L.ptr(dF), u.out_channels, None, 0, B, H, W, L.ptr(dFp), 0, S, fmt, st),
+                    "pad dF")
+        else:
+            L.check(lib.mcedm_nchw_to_nhwc_pad16_scaled(L.ptr(dF), u.out_channels, None, 0, B, H, W, L.ptr(dFp), 0,
+                                                        L.ptr(scaler.scale_t), self._gfmt, st), "pad dF")
         last: Act = T["last"]
         wgrad_side(ws, dFp, False, 64, 0, last.t, False, B, H, W, 9, G(u.out_conv.weight), 64, 0, st,
                    co_count=u.out_channels, a_coef=T["coef_out"])
@@ -286,7 +297,8 @@ class Train16Mixin:
                 dq, dk, dv = (self._fbuf(ws, n_, (B * Lq, 64), self._dt16(), dev) for n_ in ("dq", "dk", "dv"))
                 dvec = self._fbuf(ws, "dvec", (B, Lq), torch.float32, dev)
                 L.check(lib.mcedm_attention_bwd16(L.ptr(qkv), L.ptr(att), L.ptr(d_att), L.ptr(rec["lse"]), B, Lq,
-                                                  L.ptr(dvec), L.ptr(dq), L.ptr(dk), L.ptr(dv), fmt, st), "attention_bwd")
+                                                  L.ptr(dvec), L.ptr(dq), L.ptr(dk), L.ptr(dv), self._gfmt, st),
+                        "attention_bwd")
                 L.LAUNCHES[0] += 2
                 qb = self._t(ws, ("qkv_bias_tmp", blk.name), (3, 64), torch.float32)
                 for j, dj in enumerate((dq, dk, dv)):
@@ -323,7 +335,7 @@ class Train16Mixin:
             if op1 is not None:
                 thr, scale, rng = T["drop"]
                 L.check(lib.mcedm_dropout_bwd16(L.ptr(d_a1), lay[0], lay[1], B, Hb, Wb, thr, scale, blk.aff_index,
-                                                L.ptr(rng), fmt, st), "dropout_bwd16")
+                                                L.ptr(rng), self._gfmt, st), "dropout_bwd16")
             d_hb = self._buf16(ws, ("d_h16", Hb, Wb), B, Hb, Wb, dev)
             hset = dict(f32=None, bf=d_hb, dense=None, cs=None, n_cta=lib.mcedm_gn_bwd16_ctas_per_img(Hb, Wb, B))
             self._gn_bwd16(ws, d_a1, lay, h, rec["mr1"], rec["coef1"], blk.g1, blk.be1, ss_all[blk.aff_index], 1, 0, B,
@@ -395,5 +407,9 @@ class Train16Mixin:
         self._flush_deferred(ws, st)
         for dst, src in self._post_copies:
             dst.copy_(src.t())
-        self._gflat.mul_(1.0 / S)             # loss scale off (a power of two: exact)
+        if scaler is None:
+            self._gflat.mul_(1.0 / S)             # loss scale off (a power of two: exact)
+        else:
+            L.check(lib.mcedm_grad_unscale(L.ptr(self._gflat), self._gflat.numel(), L.ptr(scaler.scale_t), st),
+                    "grad_unscale")
         return self._gflat
