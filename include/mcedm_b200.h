@@ -541,6 +541,10 @@ MCEDM_API int mcedm_sumsq_partial(const float* g, long long n, double* partial, 
 MCEDM_API int mcedm_adam_step(float* p, const float* g, float* m, float* v, long long n, float lr, float beta1,
                               float beta2, float eps, float weight_decay, int step, const double* norm_partial,
                               int n_partial, float max_norm, float grad_scale, float* norm_out, void* stream);
+/* Gradient accumulation over a window of micro-batches: acc = (first ? 0 : acc) + alpha * g in fp32 (alpha = 1/N; the
+ * first micro-batch of a window does not read acc).  n fp32 elements, acc and g 16-byte aligned.  Non-finite values
+ * propagate.  No host synchronisation. */
+MCEDM_API int mcedm_grad_accumulate(float* acc, const float* g, long long n, float alpha, int first, void* stream);
 /* ema = ema*beta + (1-beta)*p   (ddim_blocks.py:48-56) */
 MCEDM_API int mcedm_ema_update(float* ema, const float* p, long long n, float beta, void* stream);
 /* mcedm_adam_step under dynamic loss scaling.  norm_partial (mcedm_sumsq_partial of g) is required; clipping runs iff

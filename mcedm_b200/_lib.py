@@ -64,6 +64,7 @@ _PROTOTYPES = {
     "mcedm_sumsq_partial": [_vp, C.c_longlong, _vp, _i, _vp],
     "mcedm_adam_step": [_vp, _vp, _vp, _vp, C.c_longlong, _f, _f, _f, _f, _f, _i, _vp, _i, _f, _f, _vp, _vp],
     "mcedm_ema_update": [_vp, _vp, C.c_longlong, _f, _vp],
+    "mcedm_grad_accumulate": [_vp, _vp, C.c_longlong, _f, _i, _vp],
     "mcedm_nchw_to_nhwc_pad16_scaled": [_vp, _i, _vp, _i, _i, _i, _i, _vp, _i, _vp, _i, _vp],
     "mcedm_grad_unscale": [_vp, C.c_longlong, _vp, _vp],
     "mcedm_adam_step_dyn": [_vp, _vp, _vp, _vp, C.c_longlong, _f, _f, _f, _f, _f, _vp, _vp, _i, _f, _f, _vp, _vp, _vp],

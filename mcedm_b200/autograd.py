@@ -27,6 +27,10 @@ class UNetFunction(torch.autograd.Function):
     def backward(ctx, dF):
         eng = ctx.eng
         eng.backward(dF)
+        if eng.accumulate_grads:
+            # `.grad` is bound to the window buffer directly: returned gradients would be added onto it a second time
+            eng.fold_grads()
+            return (None,) * (4 + ctx.n_params)
         grads = [eng.grad_of(p) if p.requires_grad else None for p in eng.unet.parameters()]
         assert len(grads) == ctx.n_params
         return (None, None, None, None, *grads)

@@ -8,6 +8,7 @@
 //   * sumsq_partial / adam_step / ema_update — gradient-norm clipping (clip_grad_norm_ semantics,
 //                        configs/trainer/trainer_ddim.yaml:8-9), torch.optim.Adam update (models/mcedm.py:141) and
 //                        EmaModel.update (models/ddim_blocks.py:48-56) on flat fp32 buffers
+//   * grad_accumulate  — the gradient-accumulation fold: window buffer (+)= micro-batch flat gradient / N
 #include "ptx.cuh"
 #include "runtime.cuh"
 #include "../../include/mcedm_b200.h"
@@ -355,6 +356,29 @@ grad_unscale_kernel(float* __restrict__ g, long long n, const float* __restrict_
   for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n; i += (long long)gridDim.x * 256) g[i] *= inv;
 }
 
+// Gradient accumulation: acc <- (first ? 0 : acc) + alpha * g over the flat fp32 gradient, four elements per
+// 128-bit access.  `first` does not read acc (a window's first micro-batch overwrites whatever the buffer held);
+// otherwise one fma per element.  inf / nan in g or acc stay non-finite, so an overflowed micro-batch still makes the
+// window's gradient non-finite for the loss-scaled Adam step.
+__global__ void __launch_bounds__(256)
+grad_accumulate_kernel(float* __restrict__ acc, const float* __restrict__ g, long long n, float alpha, int first) {
+  const long long n4 = n >> 2, tid = (long long)blockIdx.x * 256 + threadIdx.x, stride = (long long)gridDim.x * 256;
+  float4* acc4 = reinterpret_cast<float4*>(acc);
+  const float4* g4 = reinterpret_cast<const float4*>(g);
+  for (long long i = tid; i < n4; i += stride) {
+    const float4 v = g4[i];
+    float4 a;
+    if (first) {
+      a = make_float4(alpha * v.x, alpha * v.y, alpha * v.z, alpha * v.w);
+    } else {
+      a = acc4[i];
+      a = make_float4(fmaf(alpha, v.x, a.x), fmaf(alpha, v.y, a.y), fmaf(alpha, v.z, a.z), fmaf(alpha, v.w, a.w));
+    }
+    acc4[i] = a;
+  }
+  for (long long i = 4 * n4 + tid; i < n; i += stride) acc[i] = first ? alpha * g[i] : fmaf(alpha, g[i], acc[i]);
+}
+
 __global__ void __launch_bounds__(256)
 ema_update_kernel(float* __restrict__ ema, const float* __restrict__ p, long long n, float beta) {
   for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n; i += (long long)gridDim.x * 256)
@@ -547,6 +571,19 @@ extern "C" int mcedm_grad_unscale(float* g, long long n, const float* scale, voi
   int grid = (int)((n + 255) / 256);
   if (grid > 4 * num_sms()) grid = 4 * num_sms();
   grad_unscale_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(g, n, scale);
+  MCEDM_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mcedm_grad_accumulate(float* acc, const float* g, long long n, float alpha, int first, void* stream) {
+  using namespace mcedm;
+  MCEDM_REQUIRE(acc && g && n >= 1, "grad_accumulate: bad arguments");
+  MCEDM_REQUIRE(((reinterpret_cast<uintptr_t>(acc) | reinterpret_cast<uintptr_t>(g)) & 15) == 0,
+                "grad_accumulate: buffers must be 16-byte aligned");
+  int grid = (int)((n / 4 + 255) / 256);
+  if (grid < 1) grid = 1;
+  if (grid > 8 * num_sms()) grid = 8 * num_sms();
+  grad_accumulate_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(acc, g, n, alpha, first);
   MCEDM_CUDA(cudaGetLastError());
   return 0;
 }

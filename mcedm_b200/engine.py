@@ -135,6 +135,9 @@ class UNetEngine(TrainMixin, Train16Mixin, FusedMixin, PreciseMixin, PackMixin):
         self.dropout_step = 0
         # dynamic loss scaling of the fused16 plan's backward (loss_scale.LossScaler; None = the static scale)
         self.loss_scaler = None
+        # gradient accumulation over windows of N micro-batches (train_engine.TrainMixin.fold_grads; None = off: every
+        # backward's gradient is `.grad`)
+        self.accumulate_grads: Optional[int] = None
         # inference plan: True = GroupNorm fused into the convs + 16-bit activations (fused_engine.py);
         # False = the unfused fp32-stream plan below (what training's forward uses)
         self.fused = os.environ.get("MCEDM_FUSED", "1") != "0"

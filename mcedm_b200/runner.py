@@ -8,14 +8,23 @@ this module provides the minimum that keeps the reference's module code shape in
     `optimizer_step` (if pytorch_lightning is importable its class is used instead, so the same
     `PlMcedm` also runs under a real Lightning Trainer);
   * `Trainer.fit / validate / test` — one process per GPU (torchrun), NCCL gradient all-reduce on one
-    flat buffer per step, gradient-norm clipping as `gradient_clip_val` (trainer_ddim.yaml:8-9),
+    flat buffer per optimizer step, gradient-norm clipping as `gradient_clip_val` (trainer_ddim.yaml:8-9),
     hooks called in Lightning's order: setup('fit') -> training_step -> backward -> [all-reduce] ->
     clip -> optimizer_step (module hook, which also updates the EMA) -> validation_step / test_step;
   * `ModelCheckpoint` — `checkpoints/last.ckpt` with Lightning's top-level key layout (`state_dict`,
     `optimizer_states`, `epoch`, `global_step`, `hyper_parameters`, ...); `fit(ckpt_path=...)` resumes like
     `trainer.fit(ckpt_path=...)` of run.py:99: weights, Adam moments + step counter, global step, next epoch;
   * `precision=16` / "16" / "16-mixed" — dynamic loss scaling (loss_scale.py) of a network training on the fp16 plan,
-    checkpointed as Lightning's `native_amp_scaling_state` (torch.amp.GradScaler.state_dict() layout).
+    checkpointed as Lightning's `native_amp_scaling_state` (torch.amp.GradScaler.state_dict() layout);
+  * `accumulate_grad_batches=N` — Lightning 1.8's gradient accumulation (`accumulation_schedule`): the optimizer steps
+    after every N-th training batch and after an epoch's last one, on the window's gradient sum / N (the partial
+    window at an epoch's end is divided by N too).  The all-reduce, clipping, the `optimizer_step` hook (Adam + EMA)
+    and `zero_grad` run once per window; `global_step` and `max_steps` count optimizer steps; `train_loss` is logged
+    per batch.  A kernel-trained network folds each backward's gradient / N into a window buffer
+    (`UNetEngine.accumulate_grads`); other modules backpropagate loss / N into torch's accumulating `.grad`.  Under
+    dynamic loss scaling one overflowing micro-batch skips the whole window and backs the scale off once.  The
+    checkpoint's additive `train_batches` key counts training forwards, where a resumed run continues the dropout
+    mask counter.  `{epoch: N}` schedules are not supported.
 
 Data parallelism is THIS trainer's flat all-reduce; the kernels' autograd nodes bind `p.grad` to slices of the engine's
 flat gradient buffer directly, so the per-parameter reducer hooks of `torch.nn.parallel.DistributedDataParallel`
@@ -24,7 +33,7 @@ flat gradient buffer directly, so the per-parameter reducer hooks of `torch.nn.p
 from __future__ import annotations
 
 import os
-from typing import Any, Dict, Optional
+from typing import Any, Dict, List, Optional, Tuple
 
 import torch
 import torch.distributed as dist
@@ -78,6 +87,16 @@ class _ShimLightningModule(torch.nn.Module):
 LightningModule = _PlBase if HAVE_LIGHTNING else _ShimLightningModule
 
 
+def accumulation_schedule(num_batches: int, accumulate_grad_batches: int) -> List[Tuple[int, float]]:
+    """Gradient accumulation as Lightning 1.8 runs it over an epoch of `num_batches` training batches:
+    [(batch index after which the optimizer steps, factor on each micro-batch gradient of the window it closes)].
+    The optimizer steps after every N-th batch and after the epoch's last one, which closes a partial window; windows
+    never cross an epoch boundary.  The factor is 1/N for every window, the partial one included (Lightning divides
+    the closure loss by `accumulate_grad_batches`, not by the window's length)."""
+    n = accumulate_grad_batches
+    return [(k, 1.0 / n) for k in range(num_batches) if (k + 1) % n == 0 or k == num_batches - 1]
+
+
 class ModelCheckpoint:
     def __init__(self, dirpath="checkpoints/", filename="epoch", save_last=True, **_unused):
         self.dirpath, self.filename, self.save_last = dirpath, filename, save_last
@@ -106,6 +125,9 @@ class ModelCheckpoint:
         scaler = trainer.loss_scaler(module)
         if scaler is not None:
             ckpt["native_amp_scaling_state"] = scaler.state_dict()
+        # training forwards run so far (with gradient accumulation more than `global_step`): where a resumed run
+        # continues the dropout mask counter
+        ckpt["train_batches"] = trainer.train_batches
         torch.save(ckpt, os.path.join(self.dirpath, f"{self.format_name(epoch, module.global_step)}.ckpt"))
         if self.save_last:
             torch.save(ckpt, os.path.join(self.dirpath, "last.ckpt"))
@@ -116,9 +138,17 @@ class Trainer:
 
     def __init__(self, max_epochs=500, accelerator="gpu", devices=1, num_nodes=1, precision=32, strategy="ddp",
                  gradient_clip_algorithm="norm", gradient_clip_val=1.0, check_val_every_n_epoch=1, callbacks=None,
-                 max_steps=None, **_unused):
+                 max_steps=None, accumulate_grad_batches=1, **_unused):
         if gradient_clip_algorithm != "norm":
             raise NotImplementedError("only gradient_clip_algorithm='norm' is supported")
+        if isinstance(accumulate_grad_batches, dict):
+            raise NotImplementedError("accumulate_grad_batches as an {epoch: N} schedule "
+                                      "(GradientAccumulationScheduler) is not supported: pass one int N >= 1")
+        if isinstance(accumulate_grad_batches, bool) or not isinstance(accumulate_grad_batches, int) \
+                or accumulate_grad_batches < 1:
+            raise ValueError(f"accumulate_grad_batches must be an int >= 1, got {accumulate_grad_batches!r}")
+        self.accumulate_grad_batches = accumulate_grad_batches
+        self.train_batches = 0                  # training batches (forwards) run, over resumes
         self.max_epochs, self.max_steps = max_epochs, max_steps
         self.gradient_clip_val = gradient_clip_val
         self.precision = precision
@@ -238,20 +268,46 @@ class Trainer:
             if scaler is not None and ckpt.get("native_amp_scaling_state"):
                 scaler.load_state_dict(ckpt["native_amp_scaling_state"])
             module.global_step = step = int(ckpt.get("global_step", 0))
+            # checkpoints without the key were written one forward per optimizer step
+            self.train_batches = int(ckpt.get("train_batches", step))
             first_epoch = int(ckpt.get("epoch", -1)) + 1
             net = getattr(module, "model", None)
             if getattr(net, "dropout", 0.0):
-                # dropout masks are keyed by the step counter: a resumed run continues it instead of repeating masks
-                net.engine().dropout_step = step
+                # dropout masks are keyed by a per-forward counter: a resumed run continues it, never repeating masks
+                net.engine().dropout_step = self.train_batches
+        n_acc = self.accumulate_grad_batches
+        net = getattr(module, "model", None)
+        eng = net.engine() if n_acc > 1 and hasattr(net, "engine") else None
+        if eng is not None:
+            eng_acc, eng.accumulate_grads = eng.accumulate_grads, n_acc
+        try:
+            return self._fit_loop(module, datamodule, params, fused, first_epoch, step, n_acc, eng is not None)
+        finally:
+            if eng is not None:
+                eng.accumulate_grads = eng_acc
+
+    def _fit_loop(self, module, datamodule, params, fused, first_epoch, step, n_acc, engine_acc):
         history = []
         for epoch in range(first_epoch, self.max_epochs):
             module.current_epoch = epoch
             module.train()
-            for batch_idx, batch in enumerate(datamodule.train_dataloader()):
+            loader = datamodule.train_dataloader()
+            # N > 1: the batch indices that close a window (the loader must know its length to find the last one)
+            ends = None if n_acc == 1 else {k for k, _ in accumulation_schedule(len(loader), n_acc)}
+            window_open = False
+            for batch_idx, batch in enumerate(loader):
                 batch = self._to_device(batch)
-                self.optimizer.zero_grad(set_to_none=True)
+                if not window_open:
+                    self.optimizer.zero_grad(set_to_none=True)
                 loss = module.training_step(batch, batch_idx)
-                loss.backward()
+                self.train_batches += 1
+                if n_acc == 1 or engine_acc:
+                    loss.backward()                 # the engine folds gradient / N into its window buffer
+                else:
+                    (loss / n_acc).backward()       # torch's .grad accumulation
+                window_open = ends is not None and batch_idx not in ends
+                if window_open:
+                    continue
                 if fused:
                     # gradients already live in one flat buffer: all-reduce it in place (sum; the 1/world factor and
                     # the clip coefficient are folded into the Adam kernel).  flat_grads() is idempotent within a step,

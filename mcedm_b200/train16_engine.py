@@ -194,7 +194,7 @@ class Train16Mixin:
         self._fmt = self.train_fmt
         dev = ws["dev"]
         st = L.stream_ptr()
-        G = self.grad_of
+        G = self._step_grad
         fmt = self._fmt
         scaler = self.loss_scaler.state(dev) if self.loss_scaler is not None else None
         # format of the 16-bit gradient stores: fp16 without saturation under dynamic loss scaling

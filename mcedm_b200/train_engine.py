@@ -15,7 +15,8 @@ differentiate it inside PlMcedm.training_step (models/mcedm.py:254-281), built o
 Activations saved by the training forward: every GroupNorm input (fp32; these are the residual-stream tensors and
 conv0 outputs the forward writes anyway), its (mean, rstd), and every bf16 tensor-core operand.  Gradients are
 written (never accumulated across calls) into one flat fp32 buffer whose slices are returned as the parameters'
-`.grad`, so the data-parallel all-reduce and the fused Adam step work on a single contiguous tensor.
+`.grad`, so the data-parallel all-reduce and the fused Adam step work on a single contiguous tensor.  Gradient
+accumulation (`accumulate_grads`) leaves the backward as it is and folds that buffer into a second one per call.
 """
 from __future__ import annotations
 
@@ -43,27 +44,58 @@ def pack_dgrad1x1(weight2d: torch.Tensor, dtype=torch.bfloat16) -> torch.Tensor:
     return weight2d.detach().t().reshape(1, weight2d.shape[1], weight2d.shape[0]).to(DGRAD_DTYPE[0] or dtype).contiguous()
 
 
+def _flat_views(flat, params) -> dict:
+    views, off = {}, 0
+    for p in params:
+        views[id(p)] = flat[off:off + p.numel()].view(p.shape)
+        off += p.numel()
+    return views
+
+
 class TrainMixin:
     # ------------------------------------------------------------------ gradient storage
+    # Every backward writes its micro-batch gradient into `_gflat` (`_step_grad` views).  With `accumulate_grads = N`
+    # (gradient accumulation over windows of N micro-batches) one fold launch after each backward adds _gflat / N into
+    # `_gacc`, a second buffer of the same layout, and `.grad` / `grad_of` / `flat_grad` hand out `_gacc` instead.
     def _grad_layout(self):
         params = list(self.unet.parameters())
         key = tuple((id(p), p.numel()) for p in params)
         if getattr(self, "_glayout_key", None) != key or self._gflat.device != params[0].device:
             n = sum(p.numel() for p in params)
             self._gflat = torch.zeros(n, device=params[0].device, dtype=torch.float32)
-            self._gview = {}
-            off = 0
-            for p in params:
-                self._gview[id(p)] = self._gflat[off:off + p.numel()].view(p.shape)
-                off += p.numel()
+            self._gview = _flat_views(self._gflat, params)
+            self._gacc = None
             self._glayout_key = key
+        if self.accumulate_grads and self._gacc is None:
+            self._gacc = torch.zeros_like(self._gflat)
+            self._aview = _flat_views(self._gacc, params)
         return self._gflat
 
-    def grad_of(self, p) -> torch.Tensor:
+    def _step_grad(self, p) -> torch.Tensor:
+        """The slice of the micro-batch gradient buffer the backward writes p's gradient to."""
         return self._gview[id(p)]
 
+    def grad_of(self, p) -> torch.Tensor:
+        """p's gradient as `.grad` aliases it: the last backward's, or the accumulation window's."""
+        return (self._aview if self.accumulate_grads else self._gview)[id(p)]
+
     def flat_grad(self) -> torch.Tensor:
-        return self._grad_layout()
+        g = self._grad_layout()
+        return self._gacc if self.accumulate_grads else g
+
+    def fold_grads(self):
+        """Accumulation mode: adds the micro-batch gradient / N into the window buffer (one launch), overwriting it on
+        a window's first backward (the parameters' `.grad` is None after zero_grad(set_to_none=True)), and binds every
+        parameter's `.grad` to its window slice.  The 1/N is applied here, never to dL/dF: the fp16 backward keeps the
+        range of a plain step, which its loss scale is sized for."""
+        params = [p for p in self.unet.parameters() if p.requires_grad]
+        first = params[0].grad is None
+        self._grad_layout()
+        L.check(self.lib.mcedm_grad_accumulate(L.ptr(self._gacc), L.ptr(self._gflat), self._gflat.numel(),
+                                               1.0 / self.accumulate_grads, int(first), L.stream_ptr()),
+                "grad_accumulate")
+        for p in params:
+            p.grad = self._aview[id(p)]
 
     # ------------------------------------------------------------------ packed weights of the data-gradient convs
     def pack_train(self, force: bool = False):
@@ -343,7 +375,7 @@ class TrainMixin:
         B, H, W, tw, tape = T["B"], T["H"], T["W"], T["tw"], T["tape"]
         dev = tw["dev"]
         st = L.stream_ptr()
-        G = self.grad_of
+        G = self._step_grad
         dF = dF.contiguous()
         pool = tw["pool"]
         self._jid, self._rjobs, self._wjobs, self._job_refs, self._post_copies = 0, [], [], [], []

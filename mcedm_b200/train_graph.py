@@ -10,7 +10,8 @@ host-bound.  `TrainStepGraph` captures them once per batch shape into two graphs
 
 `GraphedLossFunction` replays them from `loss = ...` / `loss.backward()`, so the reference's training loop
 (models/mcedm.py:254-281 under a Lightning-style trainer) is unchanged.  Parameter `.grad`s are bound to slices of
-the flat buffer (written, not accumulated: one backward per optimizer step, as in the reference).
+the flat buffer (written, not accumulated: one backward per optimizer step, as in the reference), or, with gradient
+accumulation on (`UNetEngine.accumulate_grads`), to the window buffer one fold launch after the replay adds into.
 """
 from __future__ import annotations
 
@@ -118,6 +119,10 @@ class GraphedLossFunction(torch.autograd.Function):
         tg.g_bwd.replay()
         L.LAUNCHES[0] += tg.launches[1]
         eng = tg.pl.model.engine()
+        if eng.accumulate_grads:
+            eng._gflat.mul_(g)
+            eng.fold_grads()
+            return None, None
         flat = eng.flat_grad()
         flat.mul_(g)                          # dL/dloss (1 under a plain loss.backward())
         for p in eng.unet.parameters():
