@@ -640,6 +640,9 @@ MCEDM_API int mcedm_corr_minmax(const double* pred, const float* target, int b, 
 /* bring-up instrumentation of the product kernels (the checker / probe kernels live in their own   */
 /* library: include/mcedm_b200_check.h, libmcedm_b200_check.so)                                     */
 /* -------------------------------------------------------------------------------------------- */
+/* MCEDM_DBG (environment, bit mask read by the fused convolutions): 2 drain-only conv_rows epilogue, 4 saturation audit
+ * (below), 16 conv_flat_fused transforms TMA-loaded chunks instead of loading them itself, 32 / 64 per-role wait and
+ * MMA-issue timers of conv_rows (mcedm_debug_rows). */
 /* Saturation audit of the fp16 activation storage: with MCEDM_DBG=4 in the environment the fused 16-bit convolution
  * epilogues (conv_rows_fused N=64, conv_flat_fused fast paths) count every accumulator / output value whose magnitude
  * exceeds 65504 (clamped by the saturating conversion) or is NaN; *host_out receives the count since the last reset. */

@@ -9,7 +9,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# MCEDM_LIB: an alternative build of the same library (A/B measurements of build-time knobs, scripts/build_alt.py)
+# MCEDM_LIB: another build of the same library, e.g. the parent commit's, for an A/B comparison
 LIB_PATH = os.environ.get("MCEDM_LIB") or os.path.join(_HERE, "lib", "libmcedm_b200.so")
 
 _vp = C.c_void_p

@@ -28,14 +28,13 @@
 //
 // H2 (single pass, fp16 operands): after the single pass the softmax warps themselves were the pacer (per element: FFMA,
 // MUFU.EX2, half of a pack, unpack + add for the row sum).  Now the exponent argument is rounded to fp16 PAIRS and one
-// `ex2.approx.f16x2` produces two weights already in operand format (no pack), and the row sums come from the tensor
-// core: l = P . 1 as eight extra N = 16 MMAs per key block against a constant all-ones K-major tile (exactly the sum of
-// the ROUNDED weights the P V product uses).  ~2.5 instructions per element instead of ~8, half the MUFU work.
+// `ex2.approx.f16x2` produces two weights already in operand format (no pack), and the row sums of those ROUNDED weights
+// (what the P V product sums) are three packed fp16 adds over 8 values, then fp32.
 //   warp 0 : TMA producer (Q once; K blocks in pass 1; K and V blocks in pass 2; 3-stage ring)
 //   warp 1 : MMA issuer (S double-buffered in TMEM so softmax of block j overlaps QK^T of block j+1)
-//   warps 2-9 : softmax / epilogue: two warps per TMEM lane quarter, each owning one 64-key half of every S block of
-//               its 32 query rows (TMEM lane == row: no shuffles); the halves' row maxima / row sums meet once per
-//               pass through shared memory.  (With 4 softmax warps = one per scheduler, the dependent
+//   warps 2.. : softmax / epilogue: KS warps per TMEM lane quarter (2, or 4 for H2), each owning 128 / KS keys of every
+//               S block of its 32 query rows (TMEM lane == row: no shuffles); the slices' row maxima / row sums meet
+//               once per pass through shared memory.  (With 4 softmax warps = one per scheduler, the dependent
 //               ld -> ex2 -> cvt -> st chain had nothing to overlap with and set the kernel's pace.)
 #include "ptx.cuh"
 #include "runtime.cuh"
@@ -60,17 +59,22 @@ __device__ __forceinline__ float ex2(float x) {
 // KS: softmax warps per TMEM lane quarter (each owns 128 / KS key columns of every S block).  2 for the two-pass /
 // fp32-exponential kernels; 4 for H2, whose per-warp chain (tcgen05.ld -> FFMA -> cvt -> MUFU -> st.shared) was latency-
 // bound at 10 resident warps (ncu: issue slots 29 % active, top stalls long scoreboard / wait / MIO throttle).
-template <bool SINGLE, bool H2 = false, int KS = 2, bool LMMA = false>
-__global__ void __launch_bounds__(64 + 128 * KS, 1)
+template <bool H2>
+constexpr int attn_threads() {
+  return 64 + 128 * (H2 ? 4 : 2);
+}
+
+template <bool SINGLE, bool H2>
+__global__ void __launch_bounds__(attn_threads<H2>(), 1)
 attn_kernel(const __grid_constant__ CUtensorMap tm_qkv, int L, __nv_bfloat16* __restrict__ out,
             float* __restrict__ lse_out, int fmt, unsigned int* err, unsigned int* __restrict__ flags, int n_tiles) {
+  constexpr int KS = H2 ? 4 : 2;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* q_smem = smem;                                  // 16 KB
   uint8_t* kv_smem = q_smem + kTile;                       // stages x (K 16 KB | V 16 KB)
   uint8_t* p_smem = kv_smem + kKvStages * 2 * kTile;       // 2 buffers x 32 KB (2 atoms of 64 keys)
-  uint8_t* ones_smem = p_smem + 2 * 2 * kTile;            // 2 KB: 16 rows x 64 fp16 ones (B operand of the row-sum MMAs)
-  uint64_t* bars = reinterpret_cast<uint64_t*>(ones_smem + 2048);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(p_smem + 2 * 2 * kTile);
   uint64_t* q_full = bars;            // 1
   uint64_t* o_full = bars + 1;        // 1
   uint64_t* s_full = bars + 2;        // 2
@@ -80,7 +84,7 @@ attn_kernel(const __grid_constant__ CUtensorMap tm_qkv, int L, __nv_bfloat16* __
   uint64_t* kv_full = bars + 10;      // stages
   uint64_t* kv_empty = bars + 10 + kKvStages;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 10 + 2 * kKvStages);
-  float* xch_m = reinterpret_cast<float*>(ones_smem + 2048 + 256);         // [KS][128 rows] partial row maxima
+  float* xch_m = reinterpret_cast<float*>(bars) + 64;                      // [KS][128 rows] partial row maxima
   float* xch_l = xch_m + 128 * KS;                                         // [KS][128 rows] partial row sums
 
   pdl_wait();       // (the flag words written below are read by the previous call's fallback launch)
@@ -135,18 +139,11 @@ attn_kernel(const __grid_constant__ CUtensorMap tm_qkv, int L, __nv_bfloat16* __
     }
     fence_barrier_init();
   }
-  if (H2 && warp >= 2 && warp < 10) {
-    // all-ones tile (uniform, so the 128-byte swizzle does not matter), made visible to the async proxy
-    reinterpret_cast<uint32_t*>(ones_smem)[threadIdx.x - 64] = 0x3C003C00u;
-    reinterpret_cast<uint32_t*>(ones_smem)[threadIdx.x - 64 + 256] = 0x3C003C00u;
-    fence_proxy_async_smem();
-  }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const uint32_t tmem_o = tmem_base + 256;
-  const uint32_t tmem_l = tmem_base + 320;      // H2: 16 columns, every one the row sum of the rounded weights
 
   if (warp == 0) {
     if (lane == 0) {
@@ -166,8 +163,6 @@ attn_kernel(const __grid_constant__ CUtensorMap tm_qkv, int L, __nv_bfloat16* __
     {
       const uint32_t idesc_s = umma_idesc_16(128, 128, 0, 0, fmt);
       const uint32_t idesc_o = umma_idesc_16(128, 64, 0, 1, fmt);    // B = V, MN-major
-      const uint32_t idesc_l = umma_idesc_16(128, 16, 0, 0, fmt);    // B = ones, K-major
-      const uint64_t od = umma_desc_k_sw128(smem_u32(ones_smem));
       mbar_wait(q_full, 0, err, 0x1200);
       tc_fence_after();
       const uint32_t q_base = smem_u32(q_smem);
@@ -203,12 +198,6 @@ attn_kernel(const __grid_constant__ CUtensorMap tm_qkv, int L, __nv_bfloat16* __
             for (int kk = 0; kk < 8; ++kk)
               umma_f16(tmem_o, pd + (uint64_t)(((kk >> 2) * kTile + (kk & 3) * 32) >> 4), vd + (uint64_t)((kk * 2048) >> 4),
                        idesc_o, (uint32_t)((jp | kk) != 0));
-            if constexpr (H2 && LMMA) {
-#pragma unroll
-              for (int kk = 0; kk < 8; ++kk)
-                umma_f16(tmem_l, pd + (uint64_t)(((kk >> 2) * kTile + (kk & 3) * 32) >> 4), od, idesc_l,
-                         (uint32_t)((jp | kk) != 0));
-            }
             umma_commit(&p_empty[pb]);
             umma_commit(&kv_empty[sp]);
           }
@@ -304,16 +293,14 @@ attn_kernel(const __grid_constant__ CUtensorMap tm_qkv, int L, __nv_bfloat16* __
               asm("max.NaN.f16x2 %0, %0, %1;" : "+r"(hmax) : "r"(hh));
               asm("ex2.approx.f16x2 %0, %1;" : "=r"(op[e]) : "r"(hh));
             }
-            if constexpr (!LMMA) {
-              // row sum of the ROUNDED weights: three packed fp16 adds over the 8 values, then fp32 (the fp16 partial of 8
-              // terms carries ~2^-11 relative error, random over the 128 partials of a row)
-              uint32_t s01, s23, s4;
-              asm("add.rn.f16x2 %0, %1, %2;" : "=r"(s01) : "r"(op[0]), "r"(op[1]));
-              asm("add.rn.f16x2 %0, %1, %2;" : "=r"(s23) : "r"(op[2]), "r"(op[3]));
-              asm("add.rn.f16x2 %0, %1, %2;" : "=r"(s4) : "r"(s01), "r"(s23));
-              const float2 sf = unpack_f16x2(s4);
-              l += sf.x + sf.y;
-            }
+            // row sum of the ROUNDED weights: three packed fp16 adds over the 8 values, then fp32 (the fp16 partial of 8
+            // terms carries ~2^-11 relative error, random over the 128 partials of a row)
+            uint32_t s01, s23, s4;
+            asm("add.rn.f16x2 %0, %1, %2;" : "=r"(s01) : "r"(op[0]), "r"(op[1]));
+            asm("add.rn.f16x2 %0, %1, %2;" : "=r"(s23) : "r"(op[2]), "r"(op[3]));
+            asm("add.rn.f16x2 %0, %1, %2;" : "=r"(s4) : "r"(s01), "r"(s23));
+            const float2 sf = unpack_f16x2(s4);
+            l += sf.x + sf.y;
             const int unit = ((c & 1) * 4 + u) ^ (row & 7);
             sts128(atom_row + unit * 16, o);
             continue;
@@ -359,12 +346,6 @@ attn_kernel(const __grid_constant__ CUtensorMap tm_qkv, int L, __nv_bfloat16* __
     for (int k = 1; k < KS; ++k) l += xch_l[k * 128 + row];
     mbar_wait(o_full, 0, err, 0x1900);
     tc_fence_after();
-    if constexpr (H2 && LMMA) {
-      uint32_t lv[16];
-      tmem_ld_x16(tmem_l + lane_addr, lv);
-      tmem_wait_ld();
-      l = __uint_as_float(lv[0]);
-    }
     const float inv_l = 1.0f / l;
     // saved for the backward: P[i][j] = exp2(S[i][j] * c1 - lse2[i])
     if (lse_out && hsel == 0) lse_out[(long long)b * L + q0 + row] = mc + log2f(l);
@@ -425,56 +406,38 @@ extern "C" int mcedm_attention(const void* qkv_bf16, int B, int L, void* out_bf1
   if (rc) return rc;
   unsigned int* err = watchdog_ptr();
   MCEDM_REQUIRE(err != nullptr, "attention: no watchdog word");
-  const int smem = 1024 + kTile + kKvStages * 2 * kTile + 4 * kTile + 2048 + 256 + 4096;
+  const int smem = 1024 + kTile + kKvStages * 2 * kTile + 4 * kTile + 256 + 4096;   // align | Q | K/V | P | barriers | row exchange
   static bool attr_set = false;
   if (!attr_set) {
-    MCEDM_CUDA(cudaFuncSetAttribute(attn_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    MCEDM_CUDA(cudaFuncSetAttribute(attn_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    MCEDM_CUDA((cudaFuncSetAttribute(attn_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)));
+    MCEDM_CUDA((cudaFuncSetAttribute(attn_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)));
     MCEDM_CUDA((cudaFuncSetAttribute(attn_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)));
-    MCEDM_CUDA((cudaFuncSetAttribute(attn_kernel<true, true, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)));
-    MCEDM_CUDA((cudaFuncSetAttribute(attn_kernel<true, true, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)));
     attr_set = true;
   }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const unsigned grid = (unsigned)(B * (L / 128));
   // inference (no log-sum-exp requested): single pass over the keys + a fallback launch whose CTAs return at once
-  // unless the single-pass CTA flagged an exponent beyond fp16's range.  MCEDM_ATTN_2PASS=1 forces the two-pass kernel.
-  static int force2 = -1, no_h2 = 0, ks4 = 1, lmma = 0;
-  if (force2 < 0) {
-    const char* e = getenv("MCEDM_ATTN_2PASS");
-    force2 = (e && atoi(e)) ? 1 : 0;
-    const char* h = getenv("MCEDM_ATTN_H2");
-    no_h2 = (h && !atoi(h)) ? 1 : 0;                   // MCEDM_ATTN_H2=0: fp32 exponentials in the single-pass kernel
-    const char* k4 = getenv("MCEDM_ATTN_KS");
-    ks4 = (k4 && atoi(k4) == 2) ? 0 : 1;               // MCEDM_ATTN_KS=2: 8 softmax warps instead of 16
-    const char* lm = getenv("MCEDM_ATTN_LMMA");
-    lmma = (lm && atoi(lm)) ? 1 : 0;                   // MCEDM_ATTN_LMMA=1 (with KS=2): row sums from P . 1 MMAs
-    if (lmma) ks4 = 0;
-  }
-  if (lse_out == nullptr && !force2) {
+  // unless the single-pass CTA flagged an exponent beyond fp16's range; training runs the two-pass kernel
+  auto* o = reinterpret_cast<__nv_bfloat16*>(out_bf16);
+  const int fmt = op_fmt ? 1 : 0;
+  if (lse_out == nullptr) {
     unsigned int* flags = attn_flags(grid);
     MCEDM_REQUIRE(flags != nullptr, "attention: cannot allocate the overflow flags");
-    if (op_fmt && !no_h2 && ks4)
-      MCEDM_CUDA(launch_pdl(attn_kernel<true, true, 4>, dim3(grid), dim3(576), (size_t)smem, st, tm, L, reinterpret_cast<__nv_bfloat16*>(out_bf16), nullptr, 1,
-                                                          err, flags, (int)grid));
-    else if (op_fmt && !no_h2 && lmma)
-      MCEDM_CUDA(launch_pdl(attn_kernel<true, true, 2, true>, dim3(grid), dim3(320), (size_t)smem, st, tm, L, reinterpret_cast<__nv_bfloat16*>(out_bf16), nullptr,
-                                                                1, err, flags, (int)grid));
-    else if (op_fmt && !no_h2)
-      MCEDM_CUDA(launch_pdl(attn_kernel<true, true>, dim3(grid), dim3(320), (size_t)smem, st, tm, L, reinterpret_cast<__nv_bfloat16*>(out_bf16), nullptr, 1, err,
-                                                       flags, (int)grid));
+    if (fmt)
+      MCEDM_CUDA(launch_pdl(attn_kernel<true, true>, dim3(grid), dim3(attn_threads<true>()), (size_t)smem, st, tm, L, o,
+                            nullptr, fmt, err, flags, (int)grid));
     else
-      MCEDM_CUDA(launch_pdl(attn_kernel<true>, dim3(grid), dim3(320), (size_t)smem, st, tm, L, reinterpret_cast<__nv_bfloat16*>(out_bf16), nullptr,
-                                                 op_fmt ? 1 : 0, err, flags, (int)grid));
+      MCEDM_CUDA(launch_pdl(attn_kernel<true, false>, dim3(grid), dim3(attn_threads<false>()), (size_t)smem, st, tm, L, o,
+                            nullptr, fmt, err, flags, (int)grid));
     MCEDM_CUDA(cudaGetLastError());
     const unsigned fb_grid = grid < (unsigned)num_sms() ? grid : (unsigned)num_sms();
-    MCEDM_CUDA(launch_pdl(attn_kernel<false>, dim3(fb_grid), dim3(320), (size_t)smem, st, tm, L, reinterpret_cast<__nv_bfloat16*>(out_bf16), nullptr,
-                                                   op_fmt ? 1 : 0, err, flags, (int)grid));
+    MCEDM_CUDA(launch_pdl(attn_kernel<false, false>, dim3(fb_grid), dim3(attn_threads<false>()), (size_t)smem, st, tm, L,
+                          o, nullptr, fmt, err, flags, (int)grid));
     MCEDM_CUDA(cudaGetLastError());
     return 0;
   }
-  MCEDM_CUDA(launch_pdl(attn_kernel<false>, dim3(grid), dim3(320), (size_t)smem, st, tm, L, reinterpret_cast<__nv_bfloat16*>(out_bf16), lse_out, op_fmt ? 1 : 0,
-                                              err, nullptr, (int)grid));
+  MCEDM_CUDA(launch_pdl(attn_kernel<false, false>, dim3(grid), dim3(attn_threads<false>()), (size_t)smem, st, tm, L, o,
+                        lse_out, fmt, err, nullptr, (int)grid));
   MCEDM_CUDA(cudaGetLastError());
   return 0;
 }

@@ -32,23 +32,6 @@
 #include <cuda_bf16.h>
 #include <cstdlib>
 
-#ifndef MCEDM_DUAL
-#define MCEDM_DUAL 1   // two MMA-issuing warps taking alternate tiles (fused kernel), see conv_rows.cu
-#endif
-#ifndef MCEDM_XF_H2
-#define MCEDM_XF_H2 0   // GroupNorm+SiLU transform in packed half arithmetic (see conv_rows.cu: +2 % speed, 2.5x the error: off)
-#endif
-
-#ifndef MCEDM_FLAT_WG
-#define MCEDM_FLAT_WG 1
-#endif
-#ifndef MCEDM_FLAT_XSETS
-#define MCEDM_FLAT_XSETS 1   // transform warp sets on alternate chunks (WG layout only)
-#endif
-#ifndef MCEDM_FLAT_LDG
-#define MCEDM_FLAT_LDG 1   // fused + transform: the transform warps fetch the raw chunk from global memory themselves
-#endif
-
 namespace mcedm {
 
 constexpr int kChunkBytes = 16 * 1024;
@@ -70,8 +53,8 @@ struct FlatParams {
   int out_f32;             // out is fp32 padded-flat [B*blk][N] (K-split partial) instead of 16-bit padded-flat
   int res_f32;             // res (mode 1 only) is fp32 padded-flat
   int res_pitch, res_blk;  // layout of the 16-bit residual tensor at ITS resolution: 0,0 dense NHWC, else padded-flat
-  int dbg;                 // bring-up switches (MCEDM_DBG): 1 = fp32 transform arithmetic
-  const void* src;         // the padded-flat source itself (the transform warps' direct loads, MCEDM_FLAT_LDG)
+  int dbg;                 // bring-up switches (MCEDM_DBG): 4 saturation audit, 16 TMA-loaded chunks instead of direct loads
+  const void* src;         // the padded-flat source itself (the transform warps' direct loads)
 };
 
 template <int N, bool FUSED>
@@ -81,7 +64,7 @@ struct FlatCfg {
   static constexpr int U = 8;
   static constexpr int W_SEG_BYTES = N * 128;
   static constexpr int EPI_WARPS = 4 * NCH;
-  static constexpr bool DUAL = FUSED && MCEDM_DUAL;
+  static constexpr bool DUAL = FUSED;   // two MMA-issuing warps taking alternate tiles, see conv_rows.cu
   // WG (fused): roles laid out on warpgroup boundaries so that setmaxnreg can move registers between them:
   //   warps 0-3 TMA | MMA | MMA 2 | idle,  warps 4-11 epilogue,  warps 12-19 transform (EIGHT warps: with both MMA warps
   //   issuing, the four transform warps were this kernel's pacer).  640 threads launch at 96 registers; the transform
@@ -91,14 +74,12 @@ struct FlatCfg {
   //   setmaxnreg instruction: each group has exactly one site (a dec per role branch of the first group - three
   //   different instructions - is undefined behaviour; it ran, and is the suspect of one launch failure in 8 x 99 x 8
   //   evaluations of an 8-GPU run).
-  static constexpr bool WG = FUSED && DUAL && MCEDM_FLAT_WG;
-  static constexpr int XF_WARPS = FUSED ? (WG ? 8 : 4) : 0;
-  static constexpr int THREADS = WG ? 640 : 64 + 32 * EPI_WARPS + 32 * XF_WARPS + (DUAL ? 32 : 0);
-  static constexpr int MMA2_WARP = WG ? 2 : (DUAL ? THREADS / 32 - 1 : -1);
-  static constexpr int XF_SETS = WG ? MCEDM_FLAT_XSETS : 1;
-  static constexpr int XF_SET_WARPS = FUSED ? XF_WARPS / XF_SETS : 1;
+  static constexpr bool WG = FUSED;
+  static constexpr int XF_WARPS = FUSED ? 8 : 0;
+  static constexpr int THREADS = WG ? 640 : 64 + 32 * EPI_WARPS;
+  static constexpr int MMA2_WARP = WG ? 2 : -1;
   static constexpr int EPI_W0 = WG ? 4 : 2;
-  static constexpr int XF_W0 = WG ? 12 : 2 + EPI_WARPS;
+  static constexpr int XF_W0 = 12;
   static constexpr int STAGE_BYTES = EPI_WARPS * 32 * CH * 4;   // (the 16-bit fast-path epilogue uses half of it)
   static constexpr int ACC_BUFS = 4;
   static constexpr int TMEM_COLS = (ACC_BUFS * N <= 256) ? 256 : 512;
@@ -209,8 +190,9 @@ conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
   const int n_tiles = (int)(t_end - t_begin);
   // LDG mode: no TMA for the activation chunks.  The kernel is bounded by shared-memory traffic (operand fetch of the MMAs
   // + everything the warps move); TMA write + transform read + transform write cost 48 KB per chunk, a direct global load
-  // into registers followed by ONE swizzled store costs 16.
-  const bool xf_ldg = Cfg::WG && MCEDM_FLAT_LDG && FUSED && p.coef != nullptr && !(p.dbg & 16);
+  // into registers followed by ONE swizzled store costs 16.  (MCEDM_DBG & 16 selects TMA-loaded chunks instead: the path
+  // that the direct loads are tested against.)
+  const bool xf_ldg = FUSED && p.coef != nullptr && !(p.dbg & 16);
 
   if (warp == 0 && lane == 0) {
     prefetch_tmap(&tm_w);
@@ -223,7 +205,7 @@ conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
     for (int i = 0; i < S; ++i) {
       mbar_init(&c_full[i], 1);
       mbar_init(&c_empty[i], 1);
-      mbar_init(&c_ready[i], FUSED ? Cfg::XF_SET_WARPS : 1);
+      mbar_init(&c_ready[i], FUSED ? Cfg::XF_WARPS : 1);
     }
     mbar_init(&turn[0], 1);
     mbar_init(&turn[1], 1);
@@ -267,7 +249,7 @@ conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
     // warp-uniform control flow, one elected lane issues (see conv_rows.cu)
     // DUAL (fused kernel): two warps take alternate tiles.  Tiles own separate accumulators, but the chunk ring is
     // released by commits that track only their own thread's MMAs, so the issue ORDER is handed over exactly as in
-    // conv_rows.cu (the pipe executes in issue order: when tile j is complete so is tile j - 1).  MCEDM_DBG & 8: single.
+    // conv_rows.cu (the pipe executes in issue order: when tile j is complete so is tile j - 1).
     // lean issue loop (see conv_rows.cu): wrap-around ring counters, one election per tile, immediate offsets
     {
       const uint32_t idesc = umma_idesc_16(128, N, 0, 0, fmt);
@@ -283,11 +265,10 @@ conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
       for (int t = 0; t < 9; ++t) tap_off[t] = ((t / 3 - 1) * p.P + (t % 3 - 1)) * 8;
       uint32_t slot = 0, wslot = 0, wph = 0;
       int waited = 0;
-      const bool dual = Cfg::DUAL && !(p.dbg & 8);
       const uint32_t my_par = (warp == 1) ? 0u : 1u;
       uint32_t my_n = 0;
-      for (int j = (!dual && warp != 1) ? n_tiles : 0; j < n_tiles; ++j) {
-        if (dual && ((uint32_t)j & 1u) != my_par) {              // the other warp's tile: only the ring position moves
+      for (int j = (!Cfg::DUAL && warp != 1) ? n_tiles : 0; j < n_tiles; ++j) {
+        if (Cfg::DUAL && ((uint32_t)j & 1u) != my_par) {              // the other warp's tile: only the ring position moves
           slot = (slot + 1 == (uint32_t)S) ? 0u : slot + 1;
           continue;
         }
@@ -311,7 +292,7 @@ conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
         uint32_t al[9];
 #pragma unroll
         for (int t = 0; t < 9; ++t) al[t] = centre + (uint32_t)tap_off[t];
-        if (dual) {
+        if (Cfg::DUAL) {
           if (my_par == 1u) mbar_wait(&turn[1], my_n & 1u, p.err, 0x3a01);
           else if (my_n > 0) mbar_wait(&turn[0], (my_n - 1u) & 1u, p.err, 0x3a00);
         }
@@ -325,7 +306,7 @@ conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
             umma_f16(d_tmem, ad + 4, bd + 4, idesc, 1u);
             umma_f16(d_tmem, ad + 6, bd + 6, idesc, 1u);
           }
-          if (dual) mbar_arrive(&turn[my_par ^ 1u]);      // tile j issued: the other warp may issue tile j + 1
+          if (Cfg::DUAL) mbar_arrive(&turn[my_par ^ 1u]);      // tile j issued: the other warp may issue tile j + 1
           umma_commit(&c_empty[slot]);        // chunk j has no further user
           if (j == n_tiles - 1) {
             umma_commit(&c_empty[s1]);
@@ -578,16 +559,13 @@ conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
     // thread t owns the logical 16-byte chunk jc = t & 7 (channels 8jc .. 8jc+7) of positions (t >> 3) + 16 i of every
     // 128-position chunk; physical 16-byte slot = jc ^ (position & 7) (SWIZZLE_128B, 1 KB-aligned chunk slots).
     if constexpr (Cfg::WG) setmaxnreg_dec<80>();      // (the ONE setmaxnreg instruction of the two transform warpgroups)
-    const int tx = (int)threadIdx.x - 32 * Cfg::XF_W0;
-    const int xset = tx / (32 * Cfg::XF_SET_WARPS);           // this thread's set: chunks k = xset (mod XF_SETS)
-    const int t = tx - xset * (32 * Cfg::XF_SET_WARPS);
+    const int t = (int)threadIdx.x - 32 * Cfg::XF_W0;
     const int jc = t & 7;
     const int prow = t >> 3;
-    constexpr int XF_ROWS = FUSED ? 4 * Cfg::XF_SET_WARPS : 16;   // positions covered per pass
+    constexpr int XF_ROWS = FUSED ? 4 * Cfg::XF_WARPS : 16;   // positions covered per pass
     constexpr int XF_IT = 128 / XF_ROWS;
     int cur_b = -1;
     float ca[8], cb[8];
-    uint32_t ca2[4], cb2[4];
     // LDG mode: chunk k+1 is in flight in registers while chunk k is transformed (a chunk period is ~1.3 us)
     const uint4* srcp = reinterpret_cast<const uint4*>(p.src);
     uint4 n0[XF_IT];
@@ -602,15 +580,11 @@ conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
         for (int i = 0; i < XF_IT; ++i) dst[i] = make_uint4(0u, 0u, 0u, 0u);
       }
     };
-    if (xf_ldg && Cfg::XF_SETS == 1) ldg_chunk(0, n0);
+    if (xf_ldg) ldg_chunk(0, n0);
     for (int k = 0; k < n_tiles + 2; ++k) {
-      if (Cfg::XF_SETS > 1 && (k % Cfg::XF_SETS) != xset) continue;
       const uint32_t slot = (uint32_t)k % (uint32_t)S, ph = ((uint32_t)k / (uint32_t)S) & 1u;
       uint4 v[XF_IT];
-      if (xf_ldg && Cfg::XF_SETS > 1) {
-        ldg_chunk(k, v);           // (the other set's chunk overlaps this load)
-        mbar_wait(&c_empty[slot], ph ^ 1u, p.err, 0x3100 + slot);
-      } else if (xf_ldg) {
+      if (xf_ldg) {
 #pragma unroll
         for (int i = 0; i < XF_IT; ++i) v[i] = n0[i];
         ldg_chunk(k + 1, n0);
@@ -645,11 +619,6 @@ conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
             ca[e] *= 0.5f;
             cb[e] *= 0.5f;
           }
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            ca2[e] = pack_f16x2(ca[2 * e], ca[2 * e + 1]);
-            cb2[e] = pack_f16x2(cb[2 * e], cb[2 * e + 1]);
-          }
         }
         const uint32_t base = smem_u32(ring) + slot * kChunkBytes;
         const bool mirror = slot < 2 && k >= S;
@@ -674,17 +643,10 @@ conv_flat_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
           const int pi = prow + XF_ROWS * i;
           // branch-free (lanes of a warp sit on different positions): padding positions hold zeros and get them back
           uint4 o;
-          if (MCEDM_XF_H2 && fmt == 1 && !(p.dbg & 1)) {        // MCEDM_DBG=1: fp32 transform (A/B switch)
-            o.x = silu_affine_h2(v[i].x, ca2[0], cb2[0]);
-            o.y = silu_affine_h2(v[i].y, ca2[1], cb2[1]);
-            o.z = silu_affine_h2(v[i].z, ca2[2], cb2[2]);
-            o.w = silu_affine_h2(v[i].w, ca2[3], cb2[3]);
-          } else {
-            o.x = flat_xf_pair(v[i].x, ca[0], cb[0], ca[1], cb[1], fmt);
-            o.y = flat_xf_pair(v[i].y, ca[2], cb[2], ca[3], cb[3], fmt);
-            o.z = flat_xf_pair(v[i].z, ca[4], cb[4], ca[5], cb[5], fmt);
-            o.w = flat_xf_pair(v[i].w, ca[6], cb[6], ca[7], cb[7], fmt);
-          }
+          o.x = flat_xf_pair(v[i].x, ca[0], cb[0], ca[1], cb[1], fmt);
+          o.y = flat_xf_pair(v[i].y, ca[2], cb[2], ca[3], cb[3], fmt);
+          o.z = flat_xf_pair(v[i].z, ca[4], cb[4], ca[5], cb[5], fmt);
+          o.w = flat_xf_pair(v[i].w, ca[6], cb[6], ca[7], cb[7], fmt);
           if (!ok[i]) o = v[i];
           const int off = pi * 128 + ((jc ^ (pi & 7)) << 4);
           sts128(base + off, o);

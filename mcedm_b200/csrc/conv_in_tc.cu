@@ -25,14 +25,11 @@ constexpr int kInTile = 16 * 1024;
 // hand-over ran back to back, so every input row exposed one full global-memory latency (1.1 us per row: 242 us per launch at
 // 256 samples; doubling the epilogue warps changed nothing).  Two sets of 4 builder warps now take alternate input rows and
 // each thread requests its NEXT row's values before it packs and stores the current one: four rows in flight per CTA.
-#ifndef MCEDM_IN_BSETS
-#define MCEDM_IN_BSETS 2
-#endif
 template <int CIN>
 struct InTcCfg {
   static constexpr int SETS = 1;                       // epilogue warp sets (alternate output rows): 2 measured slower (184 vs 169 us)
   static constexpr int EPI_WARPS = 8 * SETS;
-  static constexpr int BSETS = MCEDM_IN_BSETS;         // builder warp sets (alternate input rows)
+  static constexpr int BSETS = 2;                      // builder warp sets (alternate input rows)
   static constexpr int THREADS = 64 + 32 * EPI_WARPS + BSETS * 4 * 32;
   static constexpr int STAGE_BYTES = EPI_WARPS * 4096;
 };

@@ -40,29 +40,6 @@
 #include <cuda_bf16.h>
 #include <cstdlib>
 
-// 16 epilogue warps of 16 columns for the fused N = 64 kernel (tried twice: with the lean issue loop it gains 4 % without
-// the transform and loses with it: 22 warps at 80 registers starve the transform warps).  Kept as a build-time knob.
-#ifndef MCEDM_XF8
-#define MCEDM_XF8 0   // 8 transform warps for N = 64: +5 % without residual, -12 % with (96-register cap spills the epilogue)
-#endif
-#ifndef MCEDM_EPI16
-#define MCEDM_EPI16 0
-#endif
-#ifndef MCEDM_DUAL
-#define MCEDM_DUAL 1   // two MMA-issuing warps taking alternate input rows (stacked kernels), see the MMA issuer
-#endif
-#ifndef MCEDM_ROWS_WG
-#define MCEDM_ROWS_WG 1   // fused N = 64: roles on warpgroup boundaries + setmaxnreg, 8 transform warps (as conv_flat.cu)
-#endif
-#ifndef MCEDM_XF_SETS
-#define MCEDM_XF_SETS 1   // transform warp SETS taking alternate input rows in the N = 64 kernels (the N = 16 head: always 2)
-#endif
-#ifndef MCEDM_XF_H2
-#define MCEDM_XF_H2 0   // GroupNorm+SiLU transform in packed half arithmetic: 3 instructions per 2 elements instead of 9, but
-                        // measured +2 % only (the row is bounded by shared-memory bytes, not by the transform's ALU work) at
-                        // 2.5x the operand error -> off
-#endif
-
 namespace mcedm {
 
 constexpr int kHaloRows = 130;
@@ -90,14 +67,15 @@ struct RowsParams {
   int w_rows;            // rows per segment of the packed weight matrix (== n_total)
   const float* coef[2];  // FUSED: per halo source, fp32 [B][128] = (a | b) of y = silu(a*x + b); NULL = no transform
   int nchw_c;            // FUSED N = 16 head: > 0 -> out is fp32 NCHW [B, nchw_c, H, 128] (the network output F_x)
-  int dbg;               // bring-up instrumentation (MCEDM_DBG): 32 time every role's barrier waits, 64 time MMA issue / commits
+  int dbg;               // bring-up instrumentation (MCEDM_DBG): 2 drain-only epilogue, 4 saturation audit, 32 time every
+                         // role's barrier waits, 64 time MMA issue / commits
   int res_pitch, res_blk; // FUSED, res_mode 2: the half-resolution residual is padded-flat (0,0: dense NHWC)
   int row_align;          // CTA row ranges are multiples of this many rows (1, or 4: see r_begin)
 };
 
 template <int N, bool FUSED>
 struct RowsCfg {
-  static constexpr int CH = (N >= 32 && !(FUSED && N == 64 && MCEDM_EPI16)) ? 32 : 16;
+  static constexpr int CH = N >= 32 ? 32 : 16;
   static constexpr int NCH = N / CH;
   static constexpr int U = CH / 4;
   static constexpr int W_SEG_BYTES = N * 128;
@@ -107,23 +85,23 @@ struct RowsCfg {
   // WG (fused N = 64): warps 0-3 TMA | MMA | MMA 2 | idle, 4-11 epilogue, 12-19 transform; 640 threads launch at 96
   // registers and setmaxnreg re-balances them (first group stays at 96, epilogue 128, transform 64: releases = acquisitions).
   // EIGHT transform warps without the spills that the plain 608-thread layout (104 registers for everybody) had.
-  static constexpr bool WG = FUSED && N == 64 && MCEDM_DUAL && MCEDM_ROWS_WG && !MCEDM_EPI16;
-  static constexpr int XF_WARPS = FUSED ? ((N == 16 || WG || (N == 64 && MCEDM_XF8)) ? 8 : 4) : 0;
+  static constexpr bool WG = FUSED && N == 64;
+  static constexpr int XF_WARPS = FUSED ? (N == 16 || WG ? 8 : 4) : 0;
   // A row's transform is a latency chain (wait for the TMA, shared-memory load, MUFU, store, proxy fence, hand-over) that
   // takes ~1300 cycles however many warps share it (head kernel: the same with 8 warps as the N = 64 kernel with 4), and
   // with all transform warps on the same row nothing overlaps it.  XF_SETS sets take alternate rows instead: the head
   // (8 warps, the transform is its pacer) goes from 185 to 159 us per launch at 256 samples; the N = 64 kernels lose
   // (two sets of two warps: 313 vs 302 us, 423 vs 363 with the residual - each thread then carries 16 chunks per row).
-  static constexpr int XF_SETS = FUSED ? (N == 16 ? 2 : MCEDM_XF_SETS) : 1;
+  static constexpr int XF_SETS = FUSED && N == 16 ? 2 : 1;
   static constexpr int XF_SET_WARPS = FUSED ? XF_WARPS / XF_SETS : 1;
   // DUAL: a second MMA-issuing warp (the last warp of the CTA) for the stacked kernels
-  static constexpr bool DUAL = FUSED && (N == 64 || N == 16) && MCEDM_DUAL;
+  static constexpr bool DUAL = FUSED && (N == 64 || N == 16);
   static constexpr int THREADS = WG ? 640 : 64 + 32 * EPI_WARPS + 32 * XF_WARPS + (DUAL ? 32 : 0);
   static constexpr int MMA2_WARP = WG ? 2 : (DUAL ? THREADS / 32 - 1 : -1);
   static constexpr int EPI_W0 = WG ? 4 : 2;                  // first epilogue warp
   static constexpr int XF_W0 = WG ? 12 : 2 + EPI_WARPS;      // first transform warp
   // fused N = 64: the epilogue transposes through a 16-BIT staging tile (32 pixels x 64 B per warp), see the epilogue
-  static constexpr bool EPI_H16 = FUSED && N == 64 && !MCEDM_EPI16;
+  static constexpr bool EPI_H16 = FUSED && N == 64;
   static constexpr int STAGE_BYTES = EPI_H16 ? EPI_WARPS * 2048 : EPI_WARPS * 32 * CH * 4;
   // STACK (fused N = 64): the three vertical taps of a filter column are stacked into ONE N = 192 MMA per input row
   // (see the MMA issuer); eight 64-column accumulators then rotate through all 512 TMEM columns.
@@ -170,7 +148,7 @@ __device__ __forceinline__ uint32_t xf_pair(uint32_t v, float a0, float b0, floa
 
 // RM: residual mode folded at compile time (fused N = 64 instantiations; -1 = runtime p.res_mode)
 // INF: fp16 stores without saturation (the data-gradient convs of dynamic loss scaling, op_fmt MCEDM_FMT_F16_INF)
-template <int N, bool FUSED, int RM = -1, int EP = 0, bool INF = false>
+template <int N, bool FUSED, int RM = -1, bool INF = false>
 __global__ void __launch_bounds__(RowsCfg<N, FUSED>::THREADS, 1)
 conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_h0,
                  const __grid_constant__ CUtensorMap tm_h1, const __grid_constant__ CUtensorMap tm_c0,
@@ -335,12 +313,9 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
       // arrives on turn[other], which the other warp waits for before issuing step s + 1; while it issues, this warp
       // does its commits and the waits / arithmetic of step s + 2.  A commit tracks only its own thread's MMAs, but the
       // pipe executes in issue order, so when step s's MMAs are complete so are those of step s - 1.
-      // (MCEDM_DBG & 8: single issuer, the second warp idles: A/B switch.)
       // ---------------------------------------------------------------------------------------------------------
-      const bool dual = Cfg::DUAL && !(p.dbg & 8);
+      static_assert(Cfg::DUAL, "the stacked issue loop runs on two MMA warps");
       const uint32_t my_par = (warp == 1) ? 0u : 1u;
-      if (!dual && warp != 1) goto mma_done;
-      {
       uint32_t step = 0, my_n = 0;          // global step counter / steps issued by this warp
       long long r = r_begin;
       while (r < r_end) {
@@ -349,7 +324,7 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
         const int R = (int)((r_end - r) < (long long)(p.H - y0) ? (r_end - r) : (long long)(p.H - y0));
         for (int k = 0; k < R + 2; ++k, ++step) {
           const bool ctr_step = p.n_ctr > 0 && k >= 2;
-          if (dual && (step & 1u) != my_par) {       // the other warp's step: advance the ring counters only
+          if ((step & 1u) != my_par) {               // the other warp's step: advance the ring counters only
             if (++hs == ns) {
               hs = 0;
               hph ^= 1u;
@@ -397,12 +372,10 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
           const uint32_t d1 = tmem_base + ((blk0 + (uint32_t)split) & 7u) * (uint32_t)N;   // piece after the wrap
           const uint32_t wrow = w_lo + (uint32_t)kyA * (Cfg::W_SEG_BYTES >> 4);
           const bool fresh = kyA == 0;        // output row k starts here: its very first MMA must not accumulate
-          if (dual) {
-            // issue order: step s - 1 (other warp) must have been issued.  Warp 0's n-th step waits for the other's n-th
-            // arrival (none for n = 0), warp 1's n-th step for the (n + 1)-th.
-            if (my_par == 1u) mbar_wait(&turn[1], my_n & 1u, p.err, 0x2a01);
-            else if (my_n > 0) mbar_wait(&turn[0], (my_n - 1u) & 1u, p.err, 0x2a00);
-          }
+          // issue order: step s - 1 (other warp) must have been issued.  Warp 0's n-th step waits for the other's n-th
+          // arrival (none for n = 0), warp 1's n-th step for the (n + 1)-th.
+          if (my_par == 1u) mbar_wait(&turn[1], my_n & 1u, p.err, 0x2a01);
+          else if (my_n > 0) mbar_wait(&turn[0], (my_n - 1u) & 1u, p.err, 0x2a00);
           const long long dbg_c0 = (p.dbg & 64) ? clock64() : 0;
           if (nky == 3 && split == 3) {
             // interior row, contiguous window: N = 64 (fresh) + N = 128, then 11 x N = 192
@@ -441,7 +414,7 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
           }
           const long long dbg_c1 = (p.dbg & 64) ? clock64() : 0;
           if (elect_one()) {
-            if (dual && !(p.n_ctr > 0 && k >= 2)) mbar_arrive(&turn[my_par ^ 1u]);   // hand the issue order over
+            if (!ctr_now) mbar_arrive(&turn[my_par ^ 1u]);   // hand the issue order over
             umma_commit(&h_empty[hs]);                       // an input row is consumed entirely by its own step
             if (k >= 2) {
               const uint32_t td = t0 + (uint32_t)(k - 2);    // output row k-2 is complete after this step
@@ -454,7 +427,7 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
                   for (int ks = 0; ks < 4; ++ks) umma_f16(tmem_base + blk * (uint32_t)N, ad + 2 * ks, bd + 2 * ks, idesc1, 1u);
                   umma_commit(&c_empty[cidx[s]]);
                 }
-                if (dual) mbar_arrive(&turn[my_par ^ 1u]);   // (centre MMAs of this step issued: hand over now)
+                mbar_arrive(&turn[my_par ^ 1u]);   // (centre MMAs of this step issued: hand over now)
               }
               umma_commit(&acc_full[td & 7u]);
             }
@@ -482,12 +455,7 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
         t0 += (uint32_t)R;
         r += R;
       }
-      }
-    mma_done:
-      if (warp != 1) {
-        // (second issuer: no instrumentation)
-      } else
-      if (p.dbg & 64) {                                      // only the elected lane measured: take the warp maximum
+      if (warp == 1 && (p.dbg & 64)) {   // only the first issuer's elected lane measured: take the warp maximum
         for (int off = 16; off; off >>= 1) {
           const long long o1 = __shfl_xor_sync(0xffffffffu, dbg_w1, off), o2 = __shfl_xor_sync(0xffffffffu, dbg_w2, off);
           dbg_w1 = o1 > dbg_w1 ? o1 : dbg_w1;
@@ -617,129 +585,7 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
     const int q = warp & 3;                 // TMEM lane quarter
     const int ew = warp - Cfg::EPI_W0;      // 0 .. EPI_WARPS-1
     const int ch = ew >> 2;                 // column chunk drained by this warp
-    if constexpr (Cfg::EPI_H16 && EP == 1) {
-      // ---------------------------------------------------------------------------------------------------------
-      // Register-direct epilogue (no staging tile).  tcgen05.ld 32x32b hands every thread ONE pixel and 32 consecutive
-      // channels = 64 contiguous bytes of the NHWC output row: bias and residual (two 256-bit loads, requested one tile
-      // ahead) are added in fp32, the result is rounded once and leaves as two 256-bit stores (full 32-byte sectors).
-      // Nothing of the epilogue touches shared memory any more (the 16-bit staging tile cost 16 KB written + 16 KB read
-      // per row of a kernel that is bounded by shared-memory bytes, plus two warp barriers per tile).  GroupNorm sums:
-      // a thread keeps (sum, sum of squares) of its pixel's 8 four-channel groups across the 4 rows of a block, then
-      // ONE transposing butterfly (8+4+2+1+1 shuffles for the 16 values) leaves value i on lanes 2i, 2i+1 - exactly
-      // the order of the record, which 16 lanes write as one 64-byte row.
-      // ---------------------------------------------------------------------------------------------------------
-      const int NT = p.n_total;
-      const int cg = p.n_off + ch * 32;              // first of this thread's 32 channels inside the out / res rows
-      const uint16_t* res16 = reinterpret_cast<const uint16_t*>(p.res);
-      uint16_t* out16p = reinterpret_cast<uint16_t*>(p.out);
-      // bias of the 32 channels: broadcast reads from a 256-byte table in the (otherwise unused) staging area
-      const uint32_t bias_s = smem_u32(stage_smem) + ew * 2048;
-      if (lane < 8) {
-        float4 bv = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (p.bias) bv = __ldg(reinterpret_cast<const float4*>(p.bias + cg) + lane);
-        sts128(bias_s + lane * 16, make_uint4(__float_as_uint(bv.x), __float_as_uint(bv.y), __float_as_uint(bv.z),
-                                              __float_as_uint(bv.w)));
-      }
-      __syncwarp();
-      uint32_t rn[16];                               // residual of the NEXT tile (requested one tile ahead)
-      auto load_res = [&](long long r) {
-        if (res_mode == 1) {
-          const uint16_t* a = res16 + (r * 128 + q * 32 + lane) * NT + cg;
-          ldg256(a, rn);
-          ldg256(a + 16, rn + 8);
-        } else if (res_mode == 2) {
-          const int bimg = (int)(r / p.H);
-          const int y = (int)(r - (long long)bimg * p.H);
-          const long long rrow = (p.res_pitch > 0)
-                                     ? ((long long)bimg * p.res_blk + (long long)((y >> 1) + 1) * p.res_pitch) * NT + cg
-                                     : ((long long)bimg * (p.H >> 1) + (y >> 1)) * 64 * NT + cg;
-          const uint16_t* a = res16 + rrow + ((q * 32 + lane) >> 1) * NT;
-          ldg256(a, rn);
-          ldg256(a + 16, rn + 8);
-        }
-      };
-      if (r_begin < r_end) load_res(r_begin);
-      float gs[16];                                  // gs[2g] = sum, gs[2g+1] = sum of squares of group g (4 channels)
-#pragma unroll
-      for (int i = 0; i < 16; ++i) gs[i] = 0.f;
-      long long dbg_w3 = 0;
-      const long long dbg_t0 = clock64();
-      uint32_t tcount = 0;
-      for (long long r = r_begin; r < r_end; ++r, ++tcount) {
-        const uint32_t buf = tcount % Cfg::ACC_BUFS, aph = (tcount / Cfg::ACC_BUFS) & 1u;
-        uint32_t rh[16];
-        if (res_mode != 0) {
-#pragma unroll
-          for (int i = 0; i < 16; ++i) rh[i] = rn[i];
-          if (r + 1 < r_end) load_res(r + 1);
-        }
-        timed_wait(&acc_full[buf], aph, p.err, 0x2700 + buf, dbg_w3, (p.dbg & 32) != 0);
-        tc_fence_after();
-        uint32_t v[32];
-        const uint32_t acc_col = ((8u - buf) & 7u) * (uint32_t)N;          // STACK: descending tile order
-        tmem_ld_x32(tmem_base + ((uint32_t)(q * 32) << 16) + acc_col + ch * 32, v);
-        tmem_wait_ld();
-        tc_fence_before();
-        mbar_arrive_warp(&acc_empty[buf]);
-        if (p.dbg & 2) continue;                  // bring-up: drain-only epilogue
-        uint32_t o[16];
-#pragma unroll
-        for (int c = 0; c < 8; ++c) {             // group c: channels 4c .. 4c+3
-          const float4 bz = lds128f(bias_s + c * 16);
-          float a0 = __uint_as_float(v[4 * c + 0]) + bz.x, a1 = __uint_as_float(v[4 * c + 1]) + bz.y;
-          float a2 = __uint_as_float(v[4 * c + 2]) + bz.z, a3 = __uint_as_float(v[4 * c + 3]) + bz.w;
-          if (res_mode != 0) {
-            const float2 r0 = unpack_f16x2(rh[2 * c]), r1 = unpack_f16x2(rh[2 * c + 1]);
-            a0 += r0.x; a1 += r0.y; a2 += r1.x; a3 += r1.y;
-          }
-          gs[2 * c] += (a0 + a1) + (a2 + a3);
-          gs[2 * c + 1] += (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3);
-          if (p.dbg & 4) {
-            const float aa[4] = {a0, a1, a2, a3};
-            sat_audit(p.err, aa);
-          }
-          o[2 * c] = pack_f16x2_g<INF>(a0, a1);
-          o[2 * c + 1] = pack_f16x2_g<INF>(a2, a3);
-        }
-        uint16_t* dst = out16p + (r * 128 + q * 32 + lane) * NT + cg;
-        stg256(dst, o);
-        stg256(dst + 16, o + 8);
-        if ((r & 3) == 3) {
-          // end of a 4-row block (ranges are block-aligned and H % 4 == 0, so blocks never straddle images or CTAs)
-          if (p.stats) {
-            float b8[8], c4[4], d2[2], e1;
-            const bool h16 = (lane & 16) != 0, h8 = (lane & 8) != 0, h4 = (lane & 4) != 0, h2 = (lane & 2) != 0;
-#pragma unroll
-            for (int k = 0; k < 8; ++k) {
-              const float mine = h16 ? gs[8 + k] : gs[k], theirs = h16 ? gs[k] : gs[8 + k];
-              b8[k] = mine + __shfl_xor_sync(0xffffffffu, theirs, 16);
-            }
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const float mine = h8 ? b8[4 + k] : b8[k], theirs = h8 ? b8[k] : b8[4 + k];
-              c4[k] = mine + __shfl_xor_sync(0xffffffffu, theirs, 8);
-            }
-#pragma unroll
-            for (int k = 0; k < 2; ++k) {
-              const float mine = h4 ? c4[2 + k] : c4[k], theirs = h4 ? c4[k] : c4[2 + k];
-              d2[k] = mine + __shfl_xor_sync(0xffffffffu, theirs, 4);
-            }
-            {
-              const float mine = h2 ? d2[1] : d2[0], theirs = h2 ? d2[0] : d2[1];
-              e1 = mine + __shfl_xor_sync(0xffffffffu, theirs, 2);
-            }
-            e1 += __shfl_xor_sync(0xffffffffu, e1, 1);
-            if (!(lane & 1)) p.stats[(((r >> 2) * 4 + q) * (NT / 4) + (cg >> 2)) * 2 + (lane >> 1)] = e1;
-          }
-#pragma unroll
-          for (int i = 0; i < 16; ++i) gs[i] = 0.f;
-        }
-      }
-      if ((p.dbg & 32) && warp == Cfg::EPI_W0 && lane == 0) {
-        g_rows_dbg[blockIdx.x][3] = dbg_w3;
-        g_rows_dbg[blockIdx.x][5] = clock64() - dbg_t0;
-      }
-    } else if constexpr (Cfg::EPI_H16) {
+    if constexpr (Cfg::EPI_H16) {
       // ---------------------------------------------------------------------------------------------------------
       // 16-bit staging.  (Also measured and dropped: the 8 warps as two SETS of 4 on alternate tiles, each warp draining
       // both 32-column halves of its lane quarter, so that consecutive tiles' latency chains overlap: 317 vs 301 us.)  The kernel is bounded by shared-memory BYTES per row (MMA operand fetch 120 KB + TMA 17 KB +
@@ -1027,7 +873,6 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
       const int y0 = (int)(r - (long long)b * p.H);
       const int R = (int)((r_end - r) < (long long)(p.H - y0) ? (r_end - r) : (long long)(p.H - y0));
       float ca[2][8], cb[2][8];
-      uint32_t ca2[2][4], cb2[2][4];          // the same, pre-halved and packed fp16 (MCEDM_XF_H2)
 #pragma unroll
       for (int s = 0; s < 2; ++s) {
         if (s < n_halo && p.coef[0] != nullptr) {
@@ -1041,11 +886,6 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
           for (int e = 0; e < 8; ++e) {
             ca[s][e] *= 0.5f;
             cb[s][e] *= 0.5f;
-          }
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            ca2[s][e] = pack_f16x2(ca[s][2 * e], ca[s][2 * e + 1]);
-            cb2[s][e] = pack_f16x2(cb[s][2 * e], cb[s][2 * e + 1]);
           }
         }
       }
@@ -1071,17 +911,10 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
               for (int i = 0; i < XF_SUB; ++i) {
                 const int px = 1 + prow + XF_ROWS * (i0 + i);
                 uint4 o;
-                if (MCEDM_XF_H2 && fmt == 1 && !(p.dbg & 1)) {      // MCEDM_DBG=1: fp32 transform (A/B switch)
-                  o.x = silu_affine_h2(v[i].x, ca2[s][0], cb2[s][0]);
-                  o.y = silu_affine_h2(v[i].y, ca2[s][1], cb2[s][1]);
-                  o.z = silu_affine_h2(v[i].z, ca2[s][2], cb2[s][2]);
-                  o.w = silu_affine_h2(v[i].w, ca2[s][3], cb2[s][3]);
-                } else {
-                  o.x = xf_pair(v[i].x, ca[s][0], cb[s][0], ca[s][1], cb[s][1], fmt);
-                  o.y = xf_pair(v[i].y, ca[s][2], cb[s][2], ca[s][3], cb[s][3], fmt);
-                  o.z = xf_pair(v[i].z, ca[s][4], cb[s][4], ca[s][5], cb[s][5], fmt);
-                  o.w = xf_pair(v[i].w, ca[s][6], cb[s][6], ca[s][7], cb[s][7], fmt);
-                }
+                o.x = xf_pair(v[i].x, ca[s][0], cb[s][0], ca[s][1], cb[s][1], fmt);
+                o.y = xf_pair(v[i].y, ca[s][2], cb[s][2], ca[s][3], cb[s][3], fmt);
+                o.z = xf_pair(v[i].z, ca[s][4], cb[s][4], ca[s][5], cb[s][5], fmt);
+                o.w = xf_pair(v[i].w, ca[s][6], cb[s][6], ca[s][7], cb[s][7], fmt);
                 sts128(base + px * 128 + ((j ^ (px & 7)) << 4), o);
               }
               }
@@ -1104,7 +937,7 @@ conv_rows_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant
   }
 }
 
-template <int N, bool FUSED, int RM = -1, int EP = 0, bool INF = false>
+template <int N, bool FUSED, int RM = -1, bool INF = false>
 static int launch_rows(const CUtensorMap& tm_w, const CUtensorMap* tm_h, const CUtensorMap* tm_c, RowsParams p,
                        cudaStream_t stream) {
   using Cfg = RowsCfg<N, FUSED>;
@@ -1112,17 +945,15 @@ static int launch_rows(const CUtensorMap& tm_w, const CUtensorMap* tm_h, const C
   const int fixed = 1024 + n_seg * Cfg::W_SEG_BYTES + Cfg::STAGE_BYTES + 512;
   const int slot_bytes = p.n_halo * kHaloBytes;
   // centre ring: 2 x n_ctr tiles if the halo ring keeps its preferred depth, else n_ctr + 1 (still one tile of
-  // look-ahead), else n_ctr (MCEDM_CSLOTS overrides, bring-up)
+  // look-ahead), else n_ctr
   const int min_pref = FUSED ? 5 : 4, min_ok = FUSED ? 4 : 3;
   int slots = 0;
   p.n_cslots = 0;
   const int cand[3] = {2 * p.n_ctr, p.n_ctr + 1, p.n_ctr};
-  int forced = 0;
-  if (const char* e = getenv("MCEDM_CSLOTS")) forced = atoi(e);
   for (int i = 0; i < 3; ++i) {
-    const int nc = forced >= p.n_ctr && p.n_ctr > 0 ? forced : cand[i];
+    const int nc = cand[i];
     const int sl = (232448 - fixed - nc * kCtrBytes) / slot_bytes;
-    if (sl >= (i == 0 ? min_pref : min_ok) || i == 2 || forced) {
+    if (sl >= (i == 0 ? min_pref : min_ok) || i == 2) {
       p.n_cslots = nc;
       slots = sl;
       break;
@@ -1136,12 +967,12 @@ static int launch_rows(const CUtensorMap& tm_w, const CUtensorMap* tm_h, const C
   const int smem = fixed + slots * slot_bytes + p.n_cslots * kCtrBytes;
   static bool attr_set = false;
   if (!attr_set) {
-    MCEDM_CUDA(cudaFuncSetAttribute(conv_rows_kernel<N, FUSED, RM, EP, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
+    MCEDM_CUDA(cudaFuncSetAttribute(conv_rows_kernel<N, FUSED, RM, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
     attr_set = true;
   }
   const long long units = p.total_rows / p.row_align;
   long long grid = units < num_sms() ? units : num_sms();
-  MCEDM_CUDA(launch_pdl(conv_rows_kernel<N, FUSED, RM, EP, INF>, dim3((unsigned)grid), dim3(Cfg::THREADS), (size_t)smem, stream, tm_w,
+  MCEDM_CUDA(launch_pdl(conv_rows_kernel<N, FUSED, RM, INF>, dim3((unsigned)grid), dim3(Cfg::THREADS), (size_t)smem, stream, tm_w,
                         tm_h[0], tm_h[1], tm_c[0], tm_c[1], p));
   return 0;
 }
@@ -1223,7 +1054,7 @@ extern "C" int mcedm_conv_rows_fused(const void* const* halo_src, const float* c
   p.w_rows = n_total;
   p.res_pitch = res_pitch;
   p.res_blk = res_blk;
-  p.row_align = (N == 64 && !MCEDM_EPI16) ? 4 : 1;     // GroupNorm records per 4-row block (see the epilogue)
+  p.row_align = N == 64 ? 4 : 1;     // GroupNorm records per 4-row block (see the epilogue)
   if (const char* e = getenv("MCEDM_DBG")) p.dbg = atoi(e);
   for (int i = 0; i < n_halo && i < 2; ++i) {
     p.coef[i] = halo_coef ? halo_coef[i] : nullptr;      // all NULL: the sources are already-normalised operands
@@ -1239,19 +1070,14 @@ extern "C" int mcedm_conv_rows_fused(const void* const* halo_src, const float* c
   MCEDM_REQUIRE(N == 32 || n_halo == 1, "conv_rows_fused: N = 16 / 64 take one halo source (K-split 128-channel convs)");
   if (op_fmt == MCEDM_FMT_F16_INF) {
     // the data gradient of a 3x3 conv (no transform, no residual) is the one gradient this kernel writes
-    MCEDM_REQUIRE(N == 64 && res_mode == 0 && p.coef[0] == nullptr && !(p.dbg & 128),
+    MCEDM_REQUIRE(N == 64 && res_mode == 0 && p.coef[0] == nullptr,
                   "conv_rows_fused: op_fmt MCEDM_FMT_F16_INF is the N = 64 data-gradient launch (no coefficients, no residual)");
-    return launch_rows<64, true, 0, 0, true>(tm_w, tm_h, tm_c, p, st);
+    return launch_rows<64, true, 0, true>(tm_w, tm_h, tm_c, p, st);
   }
   switch (N) {
     case 16: return launch_rows<16, true>(tm_w, tm_h, tm_c, p, st);
     case 32: return launch_rows<32, true>(tm_w, tm_h, tm_c, p, st);
     case 64:
-      if ((p.dbg & 128) && !MCEDM_EPI16) {       // MCEDM_DBG=128: register-direct epilogue (A/B: measured 14 % SLOWER, see below)
-        if (res_mode == 0) return launch_rows<64, true, 0, 1>(tm_w, tm_h, tm_c, p, st);
-        if (res_mode == 1) return launch_rows<64, true, 1, 1>(tm_w, tm_h, tm_c, p, st);
-        return launch_rows<64, true, 2, 1>(tm_w, tm_h, tm_c, p, st);
-      }
       if (res_mode == 0) return launch_rows<64, true, 0>(tm_w, tm_h, tm_c, p, st);
       if (res_mode == 1) return launch_rows<64, true, 1>(tm_w, tm_h, tm_c, p, st);
       return launch_rows<64, true, 2>(tm_w, tm_h, tm_c, p, st);

@@ -313,18 +313,6 @@ __device__ __forceinline__ float2 unpack_f16x2(uint32_t v) {
       : "=f"(lo), "=f"(hi) : "r"(v));
   return make_float2(lo, hi);
 }
-// silu(a*x + b) on TWO fp16 values with packed half arithmetic: h = a/2 * x + b/2 (HFMA2), t = tanh(h) (one MUFU for
-// the pair), y = h*t + h (HFMA2) - 3 instructions per pair instead of 9 (unpack x2, FFMA x2, MUFU x2, FFMA x2, pack).
-// The transform warps of the fused convs share four schedulers with the epilogue and MMA warps, so their instruction
-// count is what bounds a row.  a2 / b2 = the PRE-HALVED coefficients of the two channels, packed fp16.  Accuracy: the
-// operand is rounded to fp16 anyway; the extra error is the fp16 rounding of (a/2, b/2) and of h (2^-11 relative each).
-__device__ __forceinline__ uint32_t silu_affine_h2(uint32_t x2, uint32_t a2, uint32_t b2) {
-  uint32_t h, t, y;
-  asm("fma.rn.f16x2 %0, %1, %2, %3;" : "=r"(h) : "r"(x2), "r"(a2), "r"(b2));
-  asm("tanh.approx.f16x2 %0, %1;" : "=r"(t) : "r"(h));
-  asm("fma.rn.f16x2 %0, %1, %2, %1;" : "=r"(y) : "r"(h), "r"(t));
-  return y;
-}
 // Saturation audit of the fp16 activation storage (MCEDM_DBG & 4): counts values whose magnitude exceeds the largest
 // finite fp16 (65504; the packing conversions clamp them, `satfinite`) into word 8 of the watchdog buffer, so that a
 // residual stream drifting out of fp16's range is REPORTED (mcedm_saturation_count) instead of silently clipped.
